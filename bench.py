@@ -3,7 +3,7 @@
 random valid-action policy, 262,144 envs per GPU per launch), with roofline, CPU baseline and
 the end-to-end numbers through the drop-in API.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 One "step" = ONE launch of the fused K1 kernel over ONE batch of `--envs` environments
@@ -13,10 +13,13 @@ packed protocol (129 algorithmic bytes per env-step).  To keep every launch HBM-
 bench rotates over `--batches` independent env batches whose combined footprint exceeds the
 126 MB L2 (stated in config.l2).  The batches are independent, so consecutive launches
 alternate over `--streams` CUDA streams (default 2): launch k+1 fills the SMs that the few
-long warps of launch k (trio searches) leave idle.  The timed region is a block of exactly K
-launches bracketed by barrier + synchronize; the block is repeated until >= --min-seconds of
-device time have been measured and the MEDIAN block is reported (spread in `timing`).  Weak
+long warps of launch k (trio searches) leave idle.  The timed region is one block of exactly K
+launches bracketed by barrier + synchronize, right after the W warm-up launches.  Weak
 scaling: every rank owns its own batches; there is no data-path collective.
+
+--dump-outputs DIR writes what the last timed launch returned to its caller (rank 0) as float
+.npy files, so that two builds can be compared output for output: every input is derived from
+the fixed seed, so the same arguments give the same arrays.
 
 CPU arm (--impl reference, and the cpu_baseline keys): the REAL reference
 (VectorizedBlockBlastEnv(64, seed=42) + sample_valid_actions loop, scripts/benchmark.py:101-144;
@@ -74,7 +77,10 @@ def load_peaks():
 
 
 class ClockSampler:
-    """nvidia-smi clocks / throttle reasons sampled during the timed region."""
+    """nvidia-smi clocks / throttle reasons, sampled every 100 ms from before the preroll until 0.25 s
+    after the timed block (the timed block alone can be shorter than one period: ~40 ms at --steps 1000)."""
+    WINDOW = ("every 100 ms from before the preroll to 0.25 s after the timed block: preroll, warm-up, "
+              "timed block, then idle")
     Q = ("clocks.sm,clocks.max.sm,power.draw,clocks_event_reasons.hw_slowdown,"
          "clocks_event_reasons.hw_thermal_slowdown,clocks_event_reasons.sw_thermal_slowdown,"
          "clocks_event_reasons.sw_power_cap")
@@ -98,7 +104,7 @@ class ClockSampler:
 
     def stop(self):
         if not self.proc:
-            return {"sm_mhz": None, "sm_max_mhz": None, "reasons": ["nvidia-smi unavailable"]}
+            return {"sm_mhz": None, "sm_max_mhz": None, "reasons": ["nvidia-smi unavailable"], "window": self.WINDOW}
         time.sleep(0.25)
         self.proc.terminate()
         try:
@@ -117,7 +123,7 @@ class ClockSampler:
                 continue
         sm.sort()
         return {"sm_mhz": sm[len(sm) // 2] if sm else None, "sm_max_mhz": max(mx) if mx else None,
-                "reasons": sorted(reasons), "samples": len(sm)}
+                "reasons": sorted(reasons), "samples": len(sm), "window": self.WINDOW}
 
 
 # ----------------------------------------------------------------------------- CPU arms
@@ -478,6 +484,28 @@ def _spread(xs, per):
             "max": xs[-1] / per}
 
 
+DUMP_MAX_ROWS = 65536          # 788 B per dumped env: at most 52 MB in all
+
+
+def dump_step_outputs(out_dir, o, env_offset, seed):
+    """Write one bb_env_step_random launch's results as its caller receives them, for at most
+    DUMP_MAX_ROWS envs of the batch (a fixed seeded sample of a larger one): env_id (global env id),
+    actions, rewards, terminated, and action_mask [rows, 192] (action = piece slot * 64 + cell)."""
+    import numpy as np
+    n = o["actions"].numel()
+    rows = np.arange(n) if n <= DUMP_MAX_ROWS else np.sort(np.random.default_rng(seed).choice(n, DUMP_MAX_ROWS, replace=False))
+    mask = np.ascontiguousarray(o["mask"].cpu().numpy()[:, rows])
+    dense = np.unpackbits(mask.view(np.uint8).reshape(3, len(rows), 8), axis=2, bitorder="little")
+    arrays = {"env_id": (env_offset + rows).astype(np.float64),
+              "actions": o["actions"].cpu().numpy()[rows].astype(np.float32),
+              "rewards": o["rewards"].cpu().numpy()[rows],
+              "terminated": o["term"].cpu().numpy()[rows].astype(np.float32),
+              "action_mask": dense.transpose(1, 0, 2).reshape(len(rows), 192).astype(np.float32)}
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 # ----------------------------------------------------------------------------- GPU arm
 def main():
     ap = argparse.ArgumentParser()
@@ -489,7 +517,7 @@ def main():
     ap.add_argument("--batches", type=int, default=8, help="independent env batches rotated per GPU (L2-cold launches)")
     ap.add_argument("--streams", type=int, default=2, help="CUDA streams the independent batches alternate over")
     ap.add_argument("--preroll", type=int, default=64, help="untimed random steps to reach the steady-state mix")
-    ap.add_argument("--min-seconds", type=float, default=0.5, help="repeat the K-step block until this much device time is measured")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed launch's outputs (rank 0) to DIR/<name>.npy (bench_outputs/ is git-ignored)")
     ap.add_argument("--e2e-steps", type=int, default=0, help="steps per e2e block; 0 = min(steps, 100)")
     ap.add_argument("--e2e-min-seconds", type=float, default=2.0)
     ap.add_argument("--cpu-seconds", type=float, default=8.0)
@@ -554,6 +582,12 @@ def main():
                          term=torch.zeros(n, dtype=torch.uint8, device=dev),
                          mask=torch.zeros((3, n), dtype=torch.int64, device=dev)))
     stats = torch.zeros(8, dtype=torch.int64, device=dev)
+    # the sampler's start-up wait comes before the preroll, so the GPU does not idle between the
+    # preroll, the warm-up and the timed block
+    sampler = ClockSampler(local_rank)
+    if rank == 0:
+        sampler.start()
+        time.sleep(0.3)
     for e, o in zip(envs, outs):
         e.step_random(args.preroll, None, None, None, o["mask"])          # desynchronise episodes (all envs start in lockstep)
     torch.cuda.synchronize()
@@ -591,12 +625,9 @@ def main():
         barrier()
         return ev0.elapsed_time(ev1)
 
-    block(0, W, sptr)                                         # warm-up
+    block(0, W, sptr)                                         # warm-up, directly before the timed block
     stats.zero_()
-    sampler = ClockSampler(local_rank)
-    if rank == 0:
-        sampler.start()
-        time.sleep(0.3)
+
     def agree(count):
         """the same block count on every rank (each block contains barriers): max over ranks"""
         t = torch.tensor([int(count)], dtype=torch.int64, device=dev)
@@ -605,28 +636,23 @@ def main():
         return int(t.item())
 
     t_wall0 = time.perf_counter()
-    times, k0, launched = [], W, 0
-    n_blocks = 5
-    while len(times) < n_blocks:
-        times.append(block(k0, K, sptr))
-        k0 += K
-        launched += K
-        if len(times) == 5:               # size the run from the first blocks: >= min_seconds of device time in total
-            n_blocks = agree(min(2000, max(5, int(args.min_seconds * 1e3 / _median(times)) + 1)))
+    ms = block(W, K, sptr)                                    # the timed steps: exactly K launches
     wall = time.perf_counter() - t_wall0
     clocks = sampler.stop() if rank == 0 else None
     s = stats.cpu().tolist()
-    assert s[0] == n * launched, "kernel did not process the expected number of env-steps"
-    ms = _median(times)
+    assert s[0] == n * K, "kernel did not process the expected number of env-steps"
+    if args.dump_outputs and rank == 0:
+        last = (W + K - 1) % M
+        dump_step_outputs(args.dump_outputs, outs[last], (rank * M + last) * n, seed)
     tms = torch.tensor([ms], dtype=torch.float64, device=dev)
     if world > 1:
         dist.all_reduce(tms, op=dist.ReduceOp.MAX)
     ms_max = float(tms.item())
     value = world * n * K / (ms_max * 1e-3)
 
-    # the same K-launch blocks serialised on ONE stream (launch k+1 waits for the last warp of launch k)
-    t1s = [block(k0 + i * K, K, sptr[:1]) for i in range(max(5, min(len(times), 100)))]
-    ms_single = _median(t1s)
+    # K-launch blocks serialised on ONE stream (launch k+1 waits for the last warp of launch k), beside
+    # the value: median of 5..100 blocks, about 0.5 s of device time (ms_max is the same on every rank)
+    ms_single = _median([block(W + K * (i + 1), K, sptr[:1]) for i in range(max(5, min(100, int(500.0 / ms_max) + 1)))])
 
     # L2-warm variant (single batch, state+outputs 21 MB stay in L2): reported beside, not as value
     o0 = outs[0]
@@ -736,10 +762,10 @@ def main():
                        "protocol": "packed: state 48 B R+W, action 4 B, reward 4 B, terminated 1 B, mask 24 B R+W",
                        "parallelism": "env shards per GPU, no data-path collective; launches of independent batches "
                                       "alternate over %d streams" % S},
-            "timing": {"block_steps": K, "what": "device ms per step, one entry per timed block of K launches "
-                       "(barrier + synchronize on both sides); value = median block", **_spread(times, K),
-                       "timed_device_s": sum(times) * 1e-3, "launches_timed": launched},
-            "gpu_launches": launched,
+            "timing": {"block_steps": K, "what": "device ms per step of the one timed block of K launches "
+                       "(barrier + synchronize on both sides)", **_spread([ms], K),
+                       "timed_device_s": ms * 1e-3, "launches_timed": K},
+            "gpu_launches": K,
             "roofline": {"bound": "hbm", "achieved": achieved, "peak": peak, "unit": "GB/s",
                          "frac": achieved / peak, "traffic": NCU_DRAM_BYTES_PER_LAUNCH,
                          "traffic_source": TRAFFIC_SOURCE,

@@ -44,17 +44,24 @@ def test_piece_table_matches_oracle_table(libpath):
     assert [r["n"] for r in table].count(4) == 19 and [r["n"] for r in table].count(3) == 8
 
 
-@pytest.mark.reference
-def test_committed_tables_equal_fresh_derivation_from_reference():
+def test_committed_tables_equal_fresh_derivation_from_reference(tmp_path):
+    """The three generated tables against a fresh derivation from the reference's PIECE_LIST as stored in
+    tests/golden/reference_pieces.json (written by tools/gen_piece_tables.py --golden)."""
     import importlib.util
     spec = importlib.util.spec_from_file_location("gen", os.path.join(ROOT, "tools", "gen_piece_tables.py"))
     gen = importlib.util.module_from_spec(spec)
     spec.loader.exec_module(gen)
-    rows = gen.derive()
+    rows = gen.derive(json.load(open(os.path.join(ROOT, "tests", "golden", "reference_pieces.json"))))
     table = json.load(open(os.path.join(ROOT, "oracle", "piece_table.json")))
+    assert len(rows) == len(table) == 37
     for r, t in zip(rows, table):
         assert r["name"] == t["name"] and r["mask"] == int(t["mask"], 16) and r["inb"] == int(t["inb"], 16)
         assert [list(c) for c in r["cells"]] == t["cells"]
+    for write, committed in ((gen.write_json, os.path.join("oracle", "piece_table.json")),
+                             (gen.write_oracle_header, os.path.join("oracle", "bb_piece_cells.h")),
+                             (gen.write_cuda_inc, os.path.join(gen.PKG, "csrc", "bb_piece_table.inc"))):
+        write(rows, str(tmp_path / "out"))
+        assert (tmp_path / "out").read_text() == open(os.path.join(ROOT, committed)).read(), committed
 
 
 def test_philox_known_answers():

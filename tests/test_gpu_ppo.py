@@ -255,17 +255,29 @@ def test_evaluation_episodes_replay_through_the_oracle(torch):
     assert res["mean_score"] == float(res["scores"].mean()) and res["max_length"] == int(res["lengths"].max())
 
 
-@pytest.mark.reference_copy
+class _ReferenceAgentOnCPU:
+    """The reference's PPOAgent as far as loading a checkpoint goes (src/agents/ppo.py:246, :252, :433-439):
+    a BlockBlastNetwork on the CPU (test_network_is_state_dict_compatible_with_reference pins the module against
+    the reference's recorded outputs), a plain Adam(lr, eps=1e-5) over its parameters, and load = torch.load with
+    its defaults, network.load_state_dict(ck['network_state_dict']) and optimizer.load_state_dict(ck['optimizer_state_dict'])."""
+
+    def __init__(self, torch):
+        from bbgpu.network import BlockBlastNetwork
+        from bbgpu.ppo import PPOConfig
+        self.torch = torch
+        self.network = BlockBlastNetwork()
+        self.optimizer = torch.optim.Adam(self.network.parameters(), lr=PPOConfig().learning_rate, eps=1e-5)
+
+    def load(self, path):
+        ck = self.torch.load(path, map_location="cpu")
+        self.network.load_state_dict(ck["network_state_dict"])
+        self.optimizer.load_state_dict(ck["optimizer_state_dict"])
+
+
 def test_checkpoint_loads_in_the_references_own_agent(torch, tmp_path):
-    """PPOAgent.save -> the REFERENCE's PPOAgent.load (src/agents/ppo.py:433-439) on the CPU: same
-    parameters, the optimizer state accepted, and the reference network then computes the logits and values
-    our network computes on the same observation (fp32)."""
-    import sys
-    from conftest import reference_paths
-    for pth in reference_paths():
-        if pth not in sys.path:
-            sys.path.insert(0, pth)
-    from agents.ppo import PPOAgent as RefAgent, PPOConfig as RefConfig
+    """PPOAgent.save -> the reference's PPOAgent.load (src/agents/ppo.py:433-439) on the CPU: same
+    parameters, the optimizer state accepted, and the loaded network then computes the logits and values
+    our network computes on the same observation (fp32) and keeps training from the loaded state."""
     from bbgpu.ppo import PPOAgent
     from bbgpu.vec_env import VectorizedBlockBlastEnv
     torch.manual_seed(2)
@@ -278,7 +290,7 @@ def test_checkpoint_loads_in_the_references_own_agent(torch, tmp_path):
     mine.update(buf, lv)                                   # so that the optimizer has state to save
     path = str(tmp_path / "ck.pt")
     mine.save(path)
-    theirs = RefAgent(config=RefConfig(), device=torch.device("cpu"))
+    theirs = _ReferenceAgentOnCPU(torch)
     theirs.load(path)
     sd_m, sd_t = mine.network.state_dict(), theirs.network.state_dict()
     assert set(sd_m) == set(sd_t)
@@ -287,14 +299,15 @@ def test_checkpoint_loads_in_the_references_own_agent(torch, tmp_path):
     assert len(theirs.optimizer.state_dict()["state"]) == len(mine.optimizer.state_dict()["state"])
     nv = VectorizedBlockBlastEnv(16, seed=8)
     obs, _ = nv.reset()
-    mine.eval(); theirs.eval()
+    mine.eval(); theirs.network.eval()
     with torch.no_grad():
         lg_t, v_t = theirs.network(torch.from_numpy(obs["board"]), torch.from_numpy(obs["pieces"]))
         lg_m, v_m = mine.network(torch.from_numpy(obs["board"]).cuda(), torch.from_numpy(obs["pieces"]).cuda())
     assert torch.allclose(lg_t, lg_m.cpu(), atol=2e-3, rtol=2e-3) and torch.allclose(v_t, v_m.cpu(), atol=2e-3, rtol=2e-3)
     theirs.optimizer.zero_grad()                           # and it can keep training from the loaded state
+    m = torch.from_numpy(obs["action_mask"]).float()
     a, lp, ent, val = theirs.network.get_action_and_value(torch.from_numpy(obs["board"]), torch.from_numpy(obs["pieces"]),
-                                                          torch.from_numpy(obs["action_mask"]).float())
+                                                          m, action=lg_t.masked_fill(m == 0, float("-inf")).argmax(1))
     (-(lp.mean()) + val.pow(2).mean()).backward()
     theirs.optimizer.step()
     nv.close(); venv.close()

@@ -1,5 +1,6 @@
 """CPU-only tests of the host-side PPO plumbing: network layout, mask packing, env sharding,
 and the multi-rank logic (flat gradient bucket, scalar all-reduce) on a world_size-2 gloo group."""
+import copy
 import os
 import socket
 import sys
@@ -29,31 +30,38 @@ def test_network_layout_matches_reference_spec():
     assert torch.isinf(logits[:, 5]).all() and torch.isfinite(logits[:, 6]).all()
 
 
-@pytest.mark.reference
 def test_network_is_state_dict_compatible_with_reference():
-    sys.path.insert(0, os.path.join(ROOT, "tests", "golden", "_gym_stub"))
-    sys.path.insert(0, "/root/reference/src")
-    sys.dont_write_bytecode = True
-    from models.network import BlockBlastNetwork as Ref
+    """Against what the reference's own network computed (tests/golden/policy_golden.npz, make_golden.py
+    record_policy): its BlockBlastNetwork() after torch.manual_seed(0), eval mode, on the observations of its
+    VectorizedBlockBlastEnv(64, seed=5) after 7 sample_valid_actions steps under numpy seed 11, which the oracle
+    rebuilds.  Equal logits from the same seed mean that every parameter up to the policy head is created in the
+    reference's order, with its shape and its initialisation, so the state_dicts load into each other."""
+    from oracle import bb_oracle as O
     from bbgpu.network import BlockBlastNetwork
-    ref, net = Ref(), BlockBlastNetwork()
-    assert list(ref.state_dict().keys()) == list(net.state_dict().keys())
-    net.load_state_dict(ref.state_dict())
-    ref.eval(); net.eval()
-    b, p = torch.rand(6, 8, 8).round(), torch.rand(6, 3, 8, 8).round()
-    m = (torch.rand(6, 192) < 0.4).float()
-    m[:, 0] = 1
+    g = np.load(os.path.join(ROOT, "tests", "golden", "policy_golden.npz"))
+    vec = O.VecEnv([O.Env(seed=5 + i, rng_factory=O.numpy_rng_factory) for i in range(64)])
+    obs, _ = vec.reset()
+    rs = np.random.RandomState(11)
+    for _ in range(7):
+        obs, *_ = vec.step(vec.sample_valid_actions(rs))
+    assert np.array_equal(obs["action_mask"].astype(np.uint8), g["mask"])
+    torch.manual_seed(0)
+    net = BlockBlastNetwork()
+    net.eval()
+    b, p, m = torch.from_numpy(obs["board"]), torch.from_numpy(obs["pieces"]), torch.from_numpy(g["mask"]).float()
     with torch.no_grad():
-        lr, vr = ref.forward(b, p, m)
-        ln, vn = net.forward(b, p, m)
-        assert torch.allclose(vr, vn, atol=1e-5)
-        assert torch.equal(torch.isinf(lr), torch.isinf(ln))
-        assert torch.allclose(lr[torch.isfinite(lr)], ln[torch.isfinite(ln)], atol=1e-5)
-        # differentiable evaluation path == the reference's get_action_and_value for given actions
-        a = torch.multinomial(m, 1).squeeze(1)
-        _, lp_r, en_r, _ = ref.get_action_and_value(b, p, m, action=a)
-        _, lp_n, en_n, _ = net.evaluate_actions(torch.cat([b.unsqueeze(1), p], 1), m, a)
-        assert torch.allclose(lp_r, lp_n, atol=1e-6) and torch.allclose(en_r, en_n, atol=1e-6)
+        raw, _ = net.forward(b, p, None)
+        np.testing.assert_allclose(raw.numpy() * 3.0, g["logits"], rtol=1e-5, atol=1e-5)   # recorded: raw x 3
+        lm, _ = net.forward(b, p, m)
+        assert torch.equal(torch.isinf(lm), m == 0) and torch.equal(lm[m == 1], raw[m == 1])
+        assert np.array_equal(lm.argmax(1).numpy(), g["argmax"])
+        # differentiable evaluation path == the reference's get_action_and_value for the recorded actions, on the
+        # recorded (x 3) logits: scale the policy head's output layer by 3
+        net.policy_head[2].weight.mul_(3.0)
+        net.policy_head[2].bias.mul_(3.0)
+        _, lp, en, _ = net.evaluate_actions(torch.cat([b.unsqueeze(1), p], 1), m, torch.from_numpy(g["actions"]))
+    np.testing.assert_allclose(lp.numpy(), g["log_prob"], rtol=1e-5, atol=1e-5)
+    np.testing.assert_allclose(en.numpy(), g["entropy"], rtol=1e-5, atol=1e-5)
 
 
 def test_mask_plane_packing():
@@ -108,14 +116,19 @@ def _gloo_worker(rank, world, port, out):
     # backward is still running, the rest afterwards; two consecutive steps give the plain mean both times
     lin2 = torch.nn.Sequential(torch.nn.Linear(5, 3), torch.nn.Linear(3, 2))
     dist.broadcast_module(lin2)
+    # the local gradients come from a plain copy: the bucket's early slice may already be mid-reduction
+    # (in place, on gloo's thread) when backward returns
+    plain = copy.deepcopy(lin2)
     b2 = dist.FlatGradBucket(lin2.parameters(), early_from=2)
     early = []
     for step in range(2):
         b2.zero()
         (lin2(x * (step + 1)).sum() * (rank + 2)).backward()
-        loc2 = b2.flat.clone()
         fired = b2._work is not None
         b2.all_reduce_mean()
+        plain.zero_grad()
+        (plain(x * (step + 1)).sum() * (rank + 2)).backward()
+        loc2 = torch.cat([p.grad.flatten() for p in plain.parameters()])
         early.append((fired, loc2.tolist(), b2.flat.tolist()))
     out.put((rank, w0.tolist(), local.tolist(), bucket.flat.tolist(), tot, mx, dist.shard(9), early))
     torch.distributed.barrier()
