@@ -66,6 +66,7 @@ def lib():
     L.bb_env_rollout_random.argtypes = [vp, i32, vp, vp, vp, vp, vp, vp]
     L.bb_env_observe.argtypes = [vp, vp, vp, vp, vp]
     L.bb_env_sample_valid_actions.argtypes = [vp, u64, vp, vp, vp]
+    L.bb_env_expand.argtypes = [vp, u64, i32, i64, vp, vp, vp, vp, vp, vp, vp, vp, vp]
     L.bb_env_get_state.argtypes = [vp, vp, vp]
     L.bb_env_set_state.argtypes = [vp, vp, vp]
     L.bb_env_step_host.argtypes = [vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp]
@@ -191,6 +192,33 @@ class EnvHandle:
 
     def observe(self, board_out=None, pieces_out=None, mask_out=None):
         check(lib().bb_env_observe(self.h, ptr(board_out), ptr(pieces_out), ptr(mask_out), current_stream()))
+
+    def expand(self, call_counter, samples=1):
+        """One-ply successors of every env's current state (bb_env_expand; no state changes).
+        Two calls: a size query, then the fill with the same ``call_counter`` (the item count is read
+        back, which synchronises the stream).  Returns CUDA tensors: ``offsets`` int64 [n+1] (items of
+        env i are offsets[i]:offsets[i+1]), ``action`` int32, ``reward`` f32, ``terminated`` u8,
+        ``info`` int32 (the u32 info word), ``board`` int64, ``pieces`` int32 — all [items] — and
+        ``mask`` int64 [3, items]."""
+        import torch
+        dev = self.device
+        offsets = torch.empty(self.n + 1, dtype=torch.int64, device=dev)
+        L = lib()
+        check(L.bb_env_expand(self.h, int(call_counter), int(samples), 0, ptr(offsets), None, None, None, None, None,
+                              None, None, current_stream()))
+        cap = int(offsets[self.n].item())
+        out = {"offsets": offsets,
+               "action": torch.empty(cap, dtype=torch.int32, device=dev),
+               "reward": torch.empty(cap, dtype=torch.float32, device=dev),
+               "terminated": torch.empty(cap, dtype=torch.uint8, device=dev),
+               "info": torch.empty(cap, dtype=torch.int32, device=dev),
+               "board": torch.empty(cap, dtype=torch.int64, device=dev),
+               "pieces": torch.empty(cap, dtype=torch.int32, device=dev),
+               "mask": torch.empty((3, cap), dtype=torch.int64, device=dev)}
+        check(L.bb_env_expand(self.h, int(call_counter), int(samples), cap, ptr(offsets), ptr(out["action"]),
+                              ptr(out["reward"]), ptr(out["terminated"]), ptr(out["info"]), ptr(out["board"]),
+                              ptr(out["pieces"]), ptr(out["mask"]), current_stream()))
+        return out
 
     def get_state(self):
         rec = np.zeros(self.n, STATE_DTYPE)

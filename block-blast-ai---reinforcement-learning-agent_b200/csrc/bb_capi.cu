@@ -38,6 +38,7 @@ struct bb_env {
     uint8_t* d_block;      // the eight result arrays above live in this one allocation (bb_env_host_layout)
     uint8_t* d_dense;      // lazily allocated reference-layout result block (bb_env_host_dense_layout)
     uint8_t* d_trios;      // injected candidate trios (bb_env_set_trios), owned
+    int64_t* d_expand_scratch;   // block totals of bb_env_expand's offset scan, sized by n_envs at create
 };
 
 static const double BB_DEFAULT_CFG[7] = {1.0, 0.01, -1.0, -0.05, 0.02, 0.5, 0.001};
@@ -93,6 +94,10 @@ int bb_env_create(bb_env** out, int64_t n_envs, uint64_t seed, int64_t global_en
         bb_env_destroy(e);
         return fail(-2, "bb_env_create: cudaMemset state", err);
     }
+    if ((err = cudaMalloc(&e->d_expand_scratch, (size_t)bb_expand_scratch_count(n_envs) * sizeof(int64_t))) != cudaSuccess) {
+        bb_env_destroy(e);
+        return fail(-2, "bb_env_create: cudaMalloc expand scratch", err);
+    }
     // the first reset (the reference constructs each GameEngine with a dealt trio)
     err = bb_launch_reset(e->arr, nullptr, nullptr, 0);
     if (err == cudaSuccess) err = cudaDeviceSynchronize();
@@ -108,6 +113,7 @@ int bb_env_destroy(bb_env* e) {
     if (!e) return 0;
     cudaFree(e->arr.s0); cudaFree(e->arr.s1); cudaFree(e->arr.s2);
     cudaFree(e->d_actions); cudaFree(e->d_block); cudaFree(e->d_dense); cudaFree(e->d_trios);
+    cudaFree(e->d_expand_scratch);
     delete e;
     return 0;
 }
@@ -205,6 +211,21 @@ int bb_env_sample_valid_actions(bb_env* e, uint64_t call_counter, int32_t* actio
         BB_CUDA(cudaMemcpyAsync(h_actions_out, d, e->arr.n * sizeof(int32_t), cudaMemcpyDeviceToHost, s), "D2H actions");
         BB_CUDA(cudaStreamSynchronize(s), "bb_env_sample_valid_actions sync");
     }
+    return 0;
+}
+
+int bb_env_expand(bb_env* e, uint64_t call_counter, int32_t samples, int64_t capacity, int64_t* offsets,
+                  int32_t* action_out, float* reward_out, uint8_t* terminated_out, uint32_t* info_out,
+                  uint64_t* board_out, uint32_t* pieces_out, uint64_t* mask_out, void* stream) {
+    if (!e) return fail(-1, "bb_env_expand: env is NULL");
+    if (!offsets) return fail(-1, "bb_env_expand: offsets is NULL (it is always written)");
+    if (samples < 1 || samples > 64) return fail(-1, "bb_env_expand: samples must be in [1, 64]");
+    if (call_counter >= (1ull << 25)) return fail(-1, "bb_env_expand: call_counter must be < 2^25");
+    if (capacity < 0) return fail(-1, "bb_env_expand: negative capacity");
+    BB_DEVICE(e, "bb_env_expand");
+    BB_CUDA(bb_launch_expand(e->arr, e->cfg, (uint32_t)call_counter, samples, capacity, offsets, e->d_expand_scratch,
+                             action_out, reward_out, terminated_out, info_out, board_out, pieces_out, mask_out,
+                             (cudaStream_t)stream), "bb_env_expand launch");
     return 0;
 }
 

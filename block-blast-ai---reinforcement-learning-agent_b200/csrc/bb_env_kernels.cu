@@ -153,8 +153,11 @@ __device__ __forceinline__ bool bb_warp_solve(bool hard, const BBItem& item, uin
     return solved;
 }
 
+// Src: where candidates come from (bb_candidate overloads in bb_rules.cuh) — BBTrioSrc for K1 (the env's
+// own Philox stream or the injected table), BBLookaheadSrc for bb_env_expand.
+template <class Src>
 __device__ __forceinline__ uint32_t bb_warp_deal(bool pending, uint64_t board, const BBTables* T,
-                                                 const BBTrioSrc& src, uint64_t env_id, uint32_t& pieces,
+                                                 const Src& src, uint64_t env_id, uint32_t& pieces,
                                                  uint32_t& draw_ctr, BBProf& pf) {
     const unsigned FULL = 0xffffffffu;
     const int lane = threadIdx.x & 31;
@@ -424,9 +427,153 @@ bb_sample_valid_kernel(BBEnvArrays E, uint64_t call_counter, int32_t* __restrict
 }
 
 // ---------------------------------------------------------------------------------------
+// bb_env_expand: one-ply successors of every env's current state (bb_expand_* in bb_rules.cuh).
+// Phase 1 counts the items of each env and scans the counts into offsets[n+1] (three launches: a
+// block-local scan, a one-block scan of the block totals, the add); phase 2 runs one lane per item.
+// Nothing of the env state is written.
+// ---------------------------------------------------------------------------------------
+__device__ __forceinline__ int64_t bb_warp_incl_scan(int64_t v) {
+    const int lane = threadIdx.x & 31;
+#pragma unroll
+    for (int o = 1; o < 32; o <<= 1) {
+        const int64_t u = __shfl_up_sync(0xffffffffu, v, o);
+        if (lane >= o) v += u;
+    }
+    return v;
+}
+
+// inclusive scan over the block (blockDim.x = BB_STEP_THREADS); *total = the block's sum
+__device__ __forceinline__ int64_t bb_block_incl_scan(int64_t v, int64_t* total) {
+    __shared__ int64_t warp_sums[BB_STEP_THREADS / 32];
+    const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
+    v = bb_warp_incl_scan(v);
+    if (lane == 31) warp_sums[w] = v;
+    __syncthreads();
+    if (w == 0) {
+        int64_t t = lane < BB_STEP_THREADS / 32 ? warp_sums[lane] : 0;
+        t = bb_warp_incl_scan(t);
+        if (lane < BB_STEP_THREADS / 32) warp_sums[lane] = t;
+    }
+    __syncthreads();
+    if (w > 0) v += warp_sums[w - 1];
+    *total = warp_sums[BB_STEP_THREADS / 32 - 1];
+    __syncthreads();
+    return v;
+}
+
+// offsets[i] = exclusive scan of env i's item count within its block; block_sums[b] = block total
+__global__ void __launch_bounds__(BB_STEP_THREADS)
+bb_expand_count_kernel(BBEnvArrays E, int samples, int64_t* __restrict__ offsets, int64_t* __restrict__ block_sums) {
+    const BBTables& T = g_bb_tables;
+    const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    int64_t c = 0;
+    if (i < E.n) {
+        BBState s;
+        bb_load_state(E, i, s);
+        uint64_t m[3];
+        bb_action_mask(s, &T, m);
+        c = bb_expand_count(s, m, samples);
+    }
+    int64_t total;
+    const int64_t incl = bb_block_incl_scan(c, &total);
+    if (i < E.n) offsets[i] = incl - c;
+    if (threadIdx.x == 0) block_sums[blockIdx.x] = total;
+}
+
+// one block: block_sums[0..nb) -> exclusive scan in place; offsets[n] = grand total
+__global__ void __launch_bounds__(BB_STEP_THREADS)
+bb_expand_scan_blocks_kernel(int64_t* __restrict__ block_sums, int64_t nb, int64_t* __restrict__ offsets_end) {
+    int64_t carry = 0;
+    for (int64_t base = 0; base < nb; base += BB_STEP_THREADS) {
+        const int64_t j = base + threadIdx.x;
+        const int64_t v = j < nb ? block_sums[j] : 0;
+        int64_t total;
+        const int64_t incl = bb_block_incl_scan(v, &total);
+        if (j < nb) block_sums[j] = carry + incl - v;
+        carry += total;
+    }
+    if (threadIdx.x == 0) *offsets_end = carry;
+}
+
+__global__ void __launch_bounds__(BB_STEP_THREADS)
+bb_expand_add_kernel(int64_t n, const int64_t* __restrict__ block_sums, int64_t* __restrict__ offsets) {
+    const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i < n) offsets[i] += block_sums[blockIdx.x];
+}
+
+// Phase 2: lane = item.  Items of one env are adjacent, so the deals of a state with one piece left
+// (all of its items) share warps — the many-pending case bb_warp_deal spreads over the lanes.
+__global__ void __launch_bounds__(BB_STEP_THREADS, BB_STEP_MIN_BLOCKS)
+bb_expand_kernel(BBEnvArrays E, BBRewardCfg cfg, uint32_t call_counter, int samples, int64_t capacity,
+                 const int64_t* __restrict__ offsets, int32_t* __restrict__ action_out, float* __restrict__ reward_out,
+                 uint8_t* __restrict__ terminated_out, uint32_t* __restrict__ info_out,
+                 uint64_t* __restrict__ board_out, uint32_t* __restrict__ pieces_out, uint64_t* __restrict__ mask_out) {
+    const BBTables& T = g_bb_tables;
+    const int64_t item = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    const int64_t n = E.n;
+    const bool live = item < capacity && item < offsets[n];
+    BBState s;
+    s.board = 0; s.pieces = 0; s.aux = 0; s.draw_ctr = 0; s.policy_ctr = 0;
+    s.score = s.streak = s.moves = s.lines_total = s.max_streak = s.blocks_total = 0;
+    BBStepOut o;
+    BBMove mv;
+    mv.ok = false; mv.needs_deal = false; mv.n = 0; mv.lines = 0; mv.gain = 0;
+    int action = 0, k = 0;
+    uint64_t env_id = 0;
+    if (live) {
+        int64_t lo = 0, hi = n;                       // offsets[lo] <= item < offsets[hi]
+        while (hi - lo > 1) {
+            const int64_t mid = (lo + hi) >> 1;
+            if (offsets[mid] <= item) lo = mid; else hi = mid;
+        }
+        env_id = (uint64_t)(E.env_offset + lo);
+        bb_load_state(E, lo, s);
+        uint64_t m[3];
+        bb_action_mask(s, &T, m);
+        action = bb_expand_item(s, m, samples, (int)(item - offsets[lo]), &k);
+        mv = bb_env_pre(s, action, &T, o);
+    }
+    BBLookaheadSrc src;
+    src.seed = E.seed; src.call_counter = call_counter;
+    uint32_t draw = (uint32_t)k << 8;                 // LOOKAHEAD candidate index k << 8 | d (bb_rules.cuh)
+    BBProf pf;
+    const uint32_t draws = bb_warp_deal(live && mv.ok && mv.needs_deal, s.board, &T, src, env_id, s.pieces, draw, pf);
+    if (!live) return;
+    bb_env_post(s, mv, draws, &T, cfg, BBTrioSrc(E.seed), env_id, BB_FLAG_NO_AUTO_RESET, o);
+    if (action_out) action_out[item] = action;
+    if (reward_out) reward_out[item] = o.reward;
+    if (terminated_out) terminated_out[item] = (uint8_t)o.terminated;
+    if (info_out) info_out[item] = o.info;
+    if (board_out) board_out[item] = s.board;
+    if (pieces_out) pieces_out[item] = s.pieces;
+    if (mask_out) {
+        mask_out[item] = o.mask[0];
+        mask_out[capacity + item] = o.mask[1];
+        mask_out[2 * capacity + item] = o.mask[2];
+    }
+}
+
+// ---------------------------------------------------------------------------------------
 // launchers
 // ---------------------------------------------------------------------------------------
 static inline unsigned bb_grid(int64_t n) { return (unsigned)((n + BB_STEP_THREADS - 1) / BB_STEP_THREADS); }
+
+int64_t bb_expand_scratch_count(int64_t n) { return (int64_t)bb_grid(n); }
+
+cudaError_t bb_launch_expand(const BBEnvArrays& E, const BBRewardCfg& cfg, uint32_t call_counter, int samples,
+                             int64_t capacity, int64_t* offsets, int64_t* scratch, int32_t* action_out, float* reward_out,
+                             uint8_t* terminated_out, uint32_t* info_out, uint64_t* board_out, uint32_t* pieces_out,
+                             uint64_t* mask_out, cudaStream_t stream) {
+    const unsigned nb = bb_grid(E.n);
+    bb_expand_count_kernel<<<nb, BB_STEP_THREADS, 0, stream>>>(E, samples, offsets, scratch);
+    bb_expand_scan_blocks_kernel<<<1, BB_STEP_THREADS, 0, stream>>>(scratch, (int64_t)nb, offsets + E.n);
+    bb_expand_add_kernel<<<nb, BB_STEP_THREADS, 0, stream>>>(E.n, scratch, offsets);
+    if (capacity > 0)
+        bb_expand_kernel<<<bb_grid(capacity), BB_STEP_THREADS, 0, stream>>>(
+            E, cfg, call_counter, samples, capacity, offsets, action_out, reward_out, terminated_out, info_out, board_out,
+            pieces_out, mask_out);
+    return cudaGetLastError();
+}
 
 cudaError_t bb_launch_step(const BBEnvArrays& E, const BBRewardCfg& cfg, const int32_t* actions,
                            float* rewards, uint8_t* terminated, uint64_t* mask_out, uint64_t* board_out,

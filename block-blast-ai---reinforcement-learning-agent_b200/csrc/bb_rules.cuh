@@ -365,6 +365,24 @@ BB_HD uint32_t bb_candidate(const BBTrioSrc& src, uint64_t env_id, uint32_t draw
     return bb_draw_trio(src.seed, env_id, draw);
 }
 
+// LOOKAHEAD stream (bb_env_expand): the trio dealt to a SUCCESSOR state that placed the env's last
+// unused piece.  Independent of the env's own TRIO stream, so a planner never reads the deck it
+// will be dealt from.  Sample k of call `call_counter`, candidate d (0..99) of that deal:
+//   counter = (env_id lo, env_id hi, call_counter << 7 | d, 4 | k << 8)   (call_counter < 2^25, k < 64)
+// The deal loops pass `draw` = k << 8 | d (the k of the item travels with the draw counter, which the
+// warp deal shuffles from the owner lane), so the source itself holds only what the warp shares.
+#define BB_STREAM_LOOKAHEAD 4u
+struct BBLookaheadSrc {
+    uint64_t seed;
+    uint32_t call_counter;
+};
+
+BB_HD uint32_t bb_candidate(const BBLookaheadSrc& src, uint64_t env_id, uint32_t draw) {
+    const BBPhilox4 r = bb_philox((uint32_t)env_id, (uint32_t)(env_id >> 32), (src.call_counter << 7) | (draw & 0xFFu),
+                                  BB_STREAM_LOOKAHEAD | (draw >> 8 << 8), (uint32_t)src.seed, (uint32_t)(src.seed >> 32));
+    return bb_mulhi(r.x, 37u) | (bb_mulhi(r.y, 37u) << 8) | (bb_mulhi(r.z, 37u) << 16);
+}
+
 // ---------------------------------------------------------------------------------------
 // trio solvability (engine.py:174-238).  The reference enumerates piece orders and anchors
 // depth-first with line clears after every simulated placement and returns a boolean, so any
@@ -654,8 +672,10 @@ BB_HD float bb_reward(const BBRewardCfg& c, int n_blocks, int lines, bool game_o
 }
 
 // draw until a solvable trio appears, at most 100 candidates (engine.py:155-172) — the
-// sequential form; the step kernel runs the same loop warp-cooperatively (bb_warp_deal)
-BB_HD uint32_t bb_deal(uint64_t board, const BBTables* T, const BBTrioSrc& src, uint64_t env_id, uint32_t* draw_ctr) {
+// sequential form; the step kernel runs the same loop warp-cooperatively (bb_warp_deal).
+// Src: BBTrioSrc (the env's own stream / injected table) or BBLookaheadSrc (bb_env_expand).
+template <class Src>
+BB_HD uint32_t bb_deal(uint64_t board, const BBTables* T, const Src& src, uint64_t env_id, uint32_t* draw_ctr) {
     uint32_t trio = 0;
     for (int attempt = 0; attempt < 100; ++attempt) {
         trio = bb_candidate(src, env_id, *draw_ctr);
@@ -805,14 +825,39 @@ BB_HD void bb_env_apply(BBState& s, int action, const BBTables* T, const BBRewar
 }
 
 // k-th valid action (piece-major, then bit order = np.where(mask)[0] order,
-// block_blast_env.py:313-323) for the fused random-valid policy.
-BB_HD int bb_pick_action(const uint64_t m[3], uint32_t word) {
-    const int n0 = bb_popc(m[0]), n1 = bb_popc(m[1]), n2 = bb_popc(m[2]);
-    const int total = n0 + n1 + n2;
-    if (total == 0) return 0;
-    int k = (int)bb_mulhi(word, (uint32_t)total);
+// block_blast_env.py:313-323); k < number of valid actions
+BB_HD int bb_kth_action(const uint64_t m[3], int k) {
+    const int n0 = bb_popc(m[0]), n1 = bb_popc(m[1]);
     int p = 0;
     uint64_t w = m[0];
     if (k >= n0) { k -= n0; p = 1; w = m[1]; if (k >= n1) { k -= n1; p = 2; w = m[2]; } }
     return p * 64 + bb_select(w, k);
+}
+
+// the fused random-valid policy: k = mulhi(word, n_valid); 0 when nothing is valid
+BB_HD int bb_pick_action(const uint64_t m[3], uint32_t word) {
+    const int total = bb_popc(m[0]) + bb_popc(m[1]) + bb_popc(m[2]);
+    if (total == 0) return 0;
+    return bb_kth_action(m, (int)bb_mulhi(word, (uint32_t)total));
+}
+
+// ---------------------------------------------------------------------------------------
+// bb_env_expand: the one-ply successors of a state.  Items of an env, in order: its valid actions
+// in np.where(mask) order; when exactly one piece is left unused, every valid action places it and
+// deals, and gives `samples` items (k = 0..samples-1) instead of one.  m = bb_action_mask(s), so a
+// game-over state has no items.
+// ---------------------------------------------------------------------------------------
+BB_HD bool bb_expand_deals(const BBState& s) { return bb_popc32(BB_USED(s)) == 2; }
+
+BB_HD int bb_expand_count(const BBState& s, const uint64_t m[3], int samples) {
+    const int n = bb_popc(m[0]) + bb_popc(m[1]) + bb_popc(m[2]);
+    return bb_expand_deals(s) ? n * samples : n;
+}
+
+// item j (0 <= j < bb_expand_count) -> action; *k = its sample index (0 for a non-deal item)
+BB_HD int bb_expand_item(const BBState& s, const uint64_t m[3], int samples, int j, int* k) {
+    int a = j;
+    *k = 0;
+    if (bb_expand_deals(s)) { a = j / samples; *k = j - a * samples; }
+    return bb_kth_action(m, a);
 }

@@ -6,6 +6,11 @@ stays GAME_OVER and its further steps are no-ops), so the returned statistics ar
 like the reference's: scores, lengths, lines cleared, max combo.
 
     python -m bbgpu.evaluate --checkpoint checkpoints/best.pt --episodes 1000
+
+``--lookahead K`` (K >= 1) replaces the argmax policy by a one-ply value look-ahead: every legal move
+of every env is expanded on the GPU (``bb_env_expand``; a move that places the last piece is dealt K
+sampled trios from the look-ahead stream, never the env's own), the successors are scored by the value
+head, and each env plays the move with the highest mean ``reward + gamma * (1 - terminated) * V``.
 """
 import argparse
 import json
@@ -18,9 +23,33 @@ from .ppo import PPOAgent
 
 
 @torch.no_grad()
+def lookahead_actions(agent, h, n, call_counter, samples, chunk=65536):
+    """One-ply value look-ahead for the ``n`` envs of handle ``h``: int32 [n] actions maximising the mean
+    over an action's expansion items of  q = reward + gamma * (1 - terminated) * V(successor)  (lowest
+    action index on ties; action 0 for an env without a legal move).  Also returns the expansion and the
+    per-(env, action) table q [n, 192] (-inf where an action is not legal)."""
+    ex = h.expand(call_counter, samples)
+    dev = ex["offsets"].device
+    items = ex["action"].numel()
+    q = torch.full((n * 192,), float("-inf"), dtype=torch.float32, device=dev)
+    if items:
+        v = agent.values({"board": ex["board"], "pieces": ex["pieces"], "mask": ex["mask"]}, chunk=chunk).reshape(-1)
+        q_item = ex["reward"] + float(agent.config.gamma) * (1.0 - ex["terminated"].float()) * v.float()
+        env = torch.repeat_interleave(torch.arange(n, device=dev), ex["offsets"].diff(), output_size=items)
+        key = env * 192 + ex["action"].long()
+        sums = torch.zeros(n * 192, dtype=torch.float32, device=dev).index_add_(0, key, q_item)
+        cnt = torch.zeros(n * 192, dtype=torch.float32, device=dev).index_add_(0, key, torch.ones_like(q_item))
+        q = torch.where(cnt > 0, sums / cnt.clamp(min=1.0), q)
+    q = q.view(n, 192)
+    return q.argmax(dim=1).to(torch.int32), ex, q
+
+
+@torch.no_grad()
 def evaluate(agent, num_episodes=100, seed=0, deterministic=True, max_steps=10000, reward_config=None,
-             return_actions=False):
-    """``return_actions``: also return ``actions`` int32 [steps, n] (the action every env was given at every
+             return_actions=False, lookahead=0):
+    """``lookahead``: 0 = the agent's own policy (argmax when ``deterministic``); K >= 1 = one-ply value
+    look-ahead with K sampled trios per dealing move (``lookahead_actions``, expansion call counter = the
+    step number).  ``return_actions``: also return ``actions`` int32 [steps, n] (the action every env was given at every
     step; entries after an env's game over are ignored by the env) and ``rewards_per_episode`` — enough to
     replay every episode through another implementation of the rules (tests do, through the oracle)."""
     dev = agent.device
@@ -38,8 +67,11 @@ def evaluate(agent, num_episodes=100, seed=0, deterministic=True, max_steps=1000
     steps = 0
     log = []
     while steps < max_steps and not bool(done.all()):
-        h.observe(board, pieces, mask)
-        act, _, _ = agent.act({"board": board, "pieces": pieces, "mask": mask}, deterministic=deterministic)
+        if lookahead:
+            act, _, _ = lookahead_actions(agent, h, n, steps, int(lookahead))
+        else:
+            h.observe(board, pieces, mask)
+            act, _, _ = agent.act({"board": board, "pieces": pieces, "mask": mask}, deterministic=deterministic)
         if return_actions:
             log.append(act.clone())
         h.step(act, rewards, term, None, None, None, None)
@@ -69,10 +101,12 @@ def main():
     ap.add_argument("--episodes", type=int, default=100)
     ap.add_argument("--seed", type=int, default=0)
     ap.add_argument("--stochastic", action="store_true")
+    ap.add_argument("--lookahead", type=int, default=0,
+                    help="K >= 1: one-ply value look-ahead with K sampled trios per dealing move (0 = policy argmax)")
     a = ap.parse_args()
     agent = PPOAgent()
     agent.load(a.checkpoint)
-    res = evaluate(agent, a.episodes, a.seed, deterministic=not a.stochastic)
+    res = evaluate(agent, a.episodes, a.seed, deterministic=not a.stochastic, lookahead=a.lookahead)
     print(json.dumps({k: v for k, v in res.items() if not isinstance(v, np.ndarray)}, indent=1))
 
 

@@ -18,6 +18,16 @@ Philox4x32-10 (Salmon et al., SC'11), one block per event:
                       (row & 0xffffffff, row >> 32, call_counter, 2); word 0 -> u in [0,1);
                       the action is the inverse CDF of u * sum(p) taken over the kernel's lane
                       order of the 192 actions (``sample_order()``), a fixed permutation
+    stream 3  SAMPLE_VALID  bb_env_sample_valid_actions: index = the caller's call counter;
+                      word 0 picks the k-th valid action as in stream 1
+    stream 4  LOOKAHEAD  the trios dealt to SUCCESSOR states in bb_env_expand, deliberately
+                      NOT the env's own TRIO stream (a planner must not see the trio the env
+                      will really be dealt).  Counter = (env_id lo, env_id hi,
+                      call_counter << 7 | d, 4 | k << 8): call_counter < 2^25 is the caller's
+                      expansion counter, k < 64 the sample index, d < 100 the candidate
+                      index within the deal; words 0..2 -> piece ids as in stream 0.  The
+                      stream does not depend on the action (common random numbers: every
+                      deal of an env with the same k sees the same candidate sequence).
 
 Everything here is numpy on the host; it is documentation-by-code of the device streams and
 the generator of candidate-trio fixtures.  It launches nothing and is not a fallback for any
@@ -34,6 +44,8 @@ MASK32 = np.uint64(0xFFFFFFFF)
 STREAM_TRIO = 0
 STREAM_POLICY = 1
 STREAM_SAMPLE = 2
+STREAM_SAMPLE_VALID = 3
+STREAM_LOOKAHEAD = 4
 
 
 def philox4x32_10(c0, c1, c2, c3, k0, k1):
@@ -66,6 +78,17 @@ def candidate_trios(seed, env_ids, n_draws, first_draw=0):
     w = philox4x32_10(env_ids & MASK32, env_ids >> np.uint64(32), d, STREAM_TRIO,
                       seed & 0xFFFFFFFF, (seed >> 32) & 0xFFFFFFFF)
     return np.stack([mulhi32(w[k], 37) for k in range(3)], axis=-1).astype(np.uint8)
+
+
+def lookahead_trios(seed, env_ids, call_counter, k, n_draws):
+    """uint8 [len(env_ids), n_draws, 3]: LOOKAHEAD candidates d = 0..n_draws-1 (n_draws <= 100) of
+    sample k in expansion call ``call_counter`` for global env ids ``env_ids``."""
+    assert 0 <= call_counter < 2 ** 25 and 0 <= k < 64 and 0 < n_draws <= 100
+    env_ids = np.asarray(env_ids, dtype=np.uint64).reshape(-1, 1)
+    d = np.arange(n_draws, dtype=np.uint64).reshape(1, -1)
+    w = philox4x32_10(env_ids & MASK32, env_ids >> np.uint64(32), (np.uint64(call_counter) << np.uint64(7)) | d,
+                      STREAM_LOOKAHEAD | (k << 8), seed & 0xFFFFFFFF, (seed >> 32) & 0xFFFFFFFF)
+    return np.stack([mulhi32(w[j], 37) for j in range(3)], axis=-1).astype(np.uint8)
 
 
 def policy_words(seed, env_ids, steps):

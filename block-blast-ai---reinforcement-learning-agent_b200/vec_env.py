@@ -399,6 +399,21 @@ class VectorizedBlockBlastEnv:
         self._handle.sample_valid_actions(self._sample_ctr, self._d_actions, None)
         return self._d_actions.clone()
 
+    def expand(self, samples=1):
+        """One-ply look-ahead of every env's current state (bb_env_expand, ``capi.EnvHandle.expand``):
+        one item per valid action (np.where(mask) order), ``samples`` items for an action that places
+        the last unused piece (its new trio drawn from the LOOKAHEAD stream, not the env's own).
+        Keys: offsets [N+1], action, reward, terminated, info, board, pieces [items], mask [3, items].
+        No env state changes; every call advances this env's own expansion counter.  CUDA tensors in
+        "torch" / "packed" mode, numpy copies in "numpy" mode."""
+        self._expand_ctr = getattr(self, "_expand_ctr", 0) + 1
+        out = self._handle.expand(self._expand_ctr, samples)
+        if self.output == "numpy":
+            out = {k: v.cpu().numpy() for k, v in out.items()}
+            for k, dt in (("info", np.uint32), ("board", np.uint64), ("pieces", np.uint32), ("mask", np.uint64)):
+                out[k] = out[k].view(dt)
+        return out
+
     def close(self):
         self._handle.close()
 

@@ -144,6 +144,37 @@ int bb_env_rollout_random(bb_env* env, int32_t n_steps, int32_t* actions_out, fl
 int bb_env_sample_valid_actions(bb_env* env, uint64_t call_counter, int32_t* actions_out,
                                 int32_t* h_actions_out, void* stream);
 
+/* One-ply look-ahead: every legal successor of every env's CURRENT state, without changing any
+ * state (no counter moves either).  What a planner would otherwise get from GameEngine.make_move
+ * (engine.py:390-454) on a copy of the engine per legal action, with _generate_new_pieces
+ * (engine.py:155-172) and BlockBlastEnv._calculate_reward (block_blast_env.py:148-193).
+ * Items of env i, in order: its valid actions in np.where(mask) order (piece 0's bits, then 1's,
+ * then 2's: the order bb_env_sample_valid_actions indexes).  An action that does not use the last
+ * unused piece gives ONE item: exactly what bb_env_step with that action returns for env i created
+ * with BB_ENV_NO_AUTO_RESET.  When exactly one piece is left, every valid action deals a new trio and
+ * gives `samples` items k = 0..samples-1 (k ascending): the same step, but the trio is dealt from the
+ * LOOKAHEAD stream, NOT the env's own candidate stream (which would reveal the trio the env will
+ * really be dealt): Philox key seed, counter (global env id lo, hi, call_counter << 7 | d,
+ * 4 | k << 8), d = candidate 0..99 of the deal, piece ids mulhi(word, 37) of words 0..2, first solvable
+ * candidate kept (the 100th when none is).  It does not depend on the action, so all deal items of
+ * an env with the same k see the same candidates.  Game-over envs have no items.
+ *   call_counter  < 2^25; samples 1..64; capacity >= 0 = room of the item arrays
+ *   offsets        device i64[n+1]   exclusive scan of the item counts; offsets[n] = total.
+ *                                    ALWAYS written completely (capacity 0 = size query)
+ *   action_out     device i32[cap]   (every item array may be NULL; items >= capacity are dropped)
+ *   reward_out     device f32[cap]   bit-exact bb_env_step reward
+ *   terminated_out device u8[cap]
+ *   info_out       device u32[cap]   bb_env_step's info word; candidates drawn = LOOKAHEAD draws
+ *   board_out      device u64[cap]   successor board
+ *   pieces_out     device u32[cap]   successor pieces word
+ *   mask_out       device u64[3*cap] successor action mask, plane-major with plane stride `capacity`
+ *                                    (all zero when terminated)
+ * The same call_counter gives the same items, so a size query followed by a fill call is consistent. */
+int bb_env_expand(bb_env* env, uint64_t call_counter, int32_t samples, int64_t capacity,
+                  int64_t* offsets, int32_t* action_out, float* reward_out, uint8_t* terminated_out,
+                  uint32_t* info_out, uint64_t* board_out, uint32_t* pieces_out, uint64_t* mask_out,
+                  void* stream);
+
 /* Packed observation of the current states (engine.get_observation, engine.py:478-507):
  * board_out device u64[n], pieces_out device u32[n], mask_out device u64[3*n]; any NULL. */
 int bb_env_observe(bb_env* env, uint64_t* board_out, uint32_t* pieces_out, uint64_t* mask_out,
