@@ -359,14 +359,16 @@ bb_masked_sample_kernel(const void* __restrict__ logits, const uint64_t* __restr
     const bool any_valid = m > 0.5f * K3_MASKED;
     const float nm2 = any_valid ? -m * K3_LOG2E : 0.f;
     // z[i] becomes the lane's running sum of e (its local CDF); sz2 = sum e_i d_i log2e
-    float run = 0.f, sz2 = 0.f, best = -1.f;
+    float run = 0.f, sz2 = 0.f, best = K3_MASKED;
     int bi = 0;
 #pragma unroll
     for (int i = 0; i < 48; ++i) {
+        // argmax on the masked logit, not on e: two logits a few ulps apart can give equal e (or e in the
+        // wrong order, ex2.approx is accurate to 2^-22 only)
+        if (MODE == 1) { if (z[i] > best) { best = z[i]; bi = i; } }   // first maximum = lowest action index of the lane
         const float d2 = fmaf(z[i], K3_LOG2E, nm2);               // (z - m) log2e <= 0
         const float e = k3_ex2(d2);                               // exactly 0 for masked actions
         if (ENT) sz2 = fmaf(e, d2, sz2);
-        if (MODE == 1) { if (e > best) { best = e; bi = i; } }     // first maximum = lowest action index of the lane
         run += e;
         z[i] = run;
     }
@@ -377,7 +379,7 @@ bb_masked_sample_kernel(const void* __restrict__ logits, const uint64_t* __restr
     if (MODE == 2) {
         act = action[row];
     } else if (MODE == 1) {
-        // argmax of probs, lowest action index on ties (torch.argmax)
+        // argmax of the masked logits (= of probs), lowest action index on ties (torch.argmax)
         int idx = 16 * (bi >> 2) + 4 * l + (bi & 3);
 #pragma unroll
         for (int d = 1; d < 4; d <<= 1) {
@@ -403,8 +405,12 @@ bb_masked_sample_kernel(const void* __restrict__ logits, const uint64_t* __restr
         // rounding can leave t >= total: fall back to the last lane with mass
         const int L = hit ? (__ffs((int)hit) - 1) : (nz ? (31 - __clz((int)nz)) : 0);
         // inside the lane: the pick is the number of CDF entries <= the local threshold (masked entries
-        // repeat the previous value, so they are skipped together with it), at most its last valid one
-        const float tl = t - (incl - lane_tot);
+        // repeat the previous value, so they are skipped together with it), at most its last valid one.
+        // incl - lane_tot is the lane's exclusive prefix as a difference of rounded float sums: it can exceed
+        // the true prefix (small mass in a lower lane, a + b rounded up), and a t in that gap would give a
+        // negative threshold, cnt = 0 and the lane's first action whether or not it is valid.  With tl >= 0
+        // the first entry whose CDF exceeds tl has e > 0, and masked entries have e == 0 exactly.
+        const float tl = fmaxf(t - (incl - lane_tot), 0.f);
         int cnt = 0;
 #pragma unroll
         for (int i = 0; i < 48; ++i) cnt += (z[i] <= tl) ? 1 : 0;
