@@ -49,7 +49,9 @@ __device__ __forceinline__ uint4 bn_pack(const BF8& r) {
 // the rows t / G, t / G + R, ... of its block's share; the block folds its row lanes in shared
 // memory and writes ONE partial per channel to part[block][2][C] (no atomics: the finalize
 // kernel adds the partials in a fixed order, so results are bit-reproducible).
-//   MODE 0: sum x, sum x^2                                  (forward statistics)
+//   MODE 0: sum (x - K), sum (x - K)^2, K = x[row 0]        (forward statistics; shifted by a value of the
+//           channel so that q/M - (s/M)^2 does not cancel: with K = 0 the fp32 rounding left in sum x^2,
+//           ~u x^2, is of the order of eps for |x| >~ 3 and a constant channel got var ~ 3e-5 instead of 0)
 //   MODE 1: sum g, sum g * xhat, g = dy * [y > 0]           (backward reductions)
 //   MODE 2: the same with the ReLU mask recomputed from x, [x * scale + shift > 0] with the forward's own
 //           scale / shift expressions — layers without a residual input do not need y read back at all
@@ -64,6 +66,11 @@ bb_bn_reduce_kernel(const uint4* __restrict__ x, const uint4* __restrict__ y, co
     float a[8], b[8], mu[8], rs[8], sc[8], sf[8];
 #pragma unroll
     for (int k = 0; k < 8; ++k) { a[k] = 0.f; b[k] = 0.f; mu[k] = 0.f; rs[k] = 1.f; }
+    if (MODE == 0 && r0 < R) {                         // the shift K = row 0 (x - K is exact in fp32 for bf16
+        const BF8 k0 = bn_unpack(__ldg(x + g));        // values within a factor 2^15 of each other in magnitude)
+#pragma unroll
+        for (int k = 0; k < 8; ++k) mu[k] = k0.v[k];
+    }
     if (MODE >= 1) {
 #pragma unroll
         for (int k = 0; k < 8; ++k) { mu[k] = mean[g * 8 + k]; rs[k] = rstd[g * 8 + k]; }
@@ -94,7 +101,7 @@ bb_bn_reduce_kernel(const uint4* __restrict__ x, const uint4* __restrict__ y, co
                 const BF8 xv = bn_unpack(xq[u]);
                 if (MODE == 0) {
 #pragma unroll
-                    for (int k = 0; k < 8; ++k) { a[k] += xv.v[k]; b[k] = fmaf(xv.v[k], xv.v[k], b[k]); }
+                    for (int k = 0; k < 8; ++k) { const float d = xv.v[k] - mu[k]; a[k] += d; b[k] = fmaf(d, d, b[k]); }
                 } else if (MODE == 1) {
                     const BF8 yv = bn_unpack(yq[u]);
                     const BF8 dv = bn_unpack(dq[u]);
@@ -147,18 +154,20 @@ __device__ __forceinline__ void bn_sum_partials(const float* __restrict__ part, 
 }
 
 // forward finalize: mean / rstd of the batch, running statistics (momentum update with the
-// unbiased variance, as torch.nn.BatchNorm2d), and the affine pair y = x * scale + shift
+// unbiased variance, as torch.nn.BatchNorm2d), and the affine pair y = x * scale + shift.
+// The partials are shifted sums of x - K (K = x[row 0][c], see MODE 0): mu = K + s/M, var = q/M - (s/M)^2.
 __global__ void bb_bn_finalize_fwd_kernel(const float* __restrict__ part, int nblocks, int64_t M, int C, float eps,
                                           float momentum, const float* __restrict__ gamma, const float* __restrict__ beta,
                                           const float* __restrict__ pre_bias, float* __restrict__ running_mean, float* __restrict__ running_var,
                                           float* __restrict__ save_mean, float* __restrict__ save_rstd,
-                                          float* __restrict__ scale, float* __restrict__ shift) {
+                                          float* __restrict__ scale, float* __restrict__ shift, const __nv_bfloat16* __restrict__ x) {
     const int c = blockIdx.x;                     // one block per channel
     double s, q;
     bn_sum_partials(part, nblocks, C, c, s, q);
     if (threadIdx.x != 0) return;
-    const double mu = s / (double)M;
-    double var = q / (double)M - mu * mu;
+    const double d = s / (double)M;
+    const double mu = (double)__bfloat162float(x[c]) + d;
+    double var = q / (double)M - d * d;
     var = var > 0.0 ? var : 0.0;
     const float rstd = (float)(1.0 / sqrt(var + (double)eps));
     save_mean[c] = (float)mu;
@@ -318,7 +327,8 @@ cudaError_t bb_launch_bn_relu_fwd(const void* x, const void* skip, const float* 
         bb_bn_reduce_kernel<0><<<g, BN_THREADS, (size_t)R * 2 * C * sizeof(float), stream>>>(
             (const uint4*)x, nullptr, nullptr, nullptr, nullptr, part, M, C);
         bb_bn_finalize_fwd_kernel<<<C, BN_FIN_THREADS, 0, stream>>>(part, g, M, C, eps, momentum, gamma, beta, pre_bias,
-                                                                      running_mean, running_var, save_mean, save_rstd, scale, shift);
+                                                                      running_mean, running_var, save_mean, save_rstd, scale, shift,
+                                                                      (const __nv_bfloat16*)x);
     } else {
         bb_bn_affine_eval_kernel<<<(C + 127) / 128, 128, 0, stream>>>(gamma, beta, pre_bias, running_mean, running_var, eps, C, scale, shift);
     }
