@@ -9,7 +9,8 @@ by either side load in the other (``network_state_dict``, src/agents/ppo.py:425-
 The CNN body stays PyTorch (north_star).  What is replaced is the categorical head:
 ``get_action_and_value`` without gradients (rollout / evaluation) runs the fused K3 kernel
 (-inf masking + softmax + sample/argmax + log-prob + masked entropy, network.py:172-262);
-with gradients (PPO update) the same maths is expressed in torch ops so autograd applies.
+with gradients (given actions) the same maths is expressed in torch ops so autograd applies.
+The PPO update runs the whole loss tail after the CNN as one kernel (``PPOLossTail``).
 """
 import torch
 import torch.nn as nn
@@ -134,36 +135,6 @@ def _pack_mask_planes(mask_dense):
     shifts = (8 * torch.arange(8, device=mask_dense.device, dtype=torch.int64)).view(1, 1, 8)
     hi_fix = rows << shifts                                          # row 7 lands in the sign bit: two's complement is fine
     return hi_fix.sum(-1).t().contiguous()                           # wraps modulo 2**64
-
-
-class MaskedHead(torch.autograd.Function):
-    """log_prob[action] and masked entropy from raw logits + packed mask planes, forward = K3
-    (evaluate mode), backward = bb_masked_head_backward: one kernel each way instead of the
-    dozen elementwise ops of network.py:210-262 under autograd."""
-
-    @staticmethod
-    def forward(ctx, logits, planes, action):
-        lg = logits.detach()
-        if lg.dtype not in (torch.float32, torch.bfloat16):
-            lg = lg.float()
-        lg = lg.contiguous()
-        n = lg.shape[0]
-        act = action.to(torch.int32).contiguous()
-        logp = torch.empty(n, dtype=torch.float32, device=lg.device)
-        ent = torch.empty(n, dtype=torch.float32, device=lg.device)
-        capi.masked_sample(lg, planes, planes.stride(0), 0, 0, 2, act, logp, ent)
-        ctx.save_for_backward(lg, planes, act)
-        ctx.in_dtype = logits.dtype
-        return logp, ent
-
-    @staticmethod
-    def backward(ctx, g_logp, g_ent):
-        lg, planes, act = ctx.saved_tensors
-        grad = torch.empty_like(lg)
-        g1 = g_logp.float().contiguous()
-        g2 = g_ent.float().contiguous() if g_ent is not None else None
-        capi.masked_head_backward(lg, planes, planes.stride(0), act, g1, g2, grad)
-        return grad.to(ctx.in_dtype), None, None
 
 
 class PPOLossTail(torch.autograd.Function):
@@ -349,13 +320,6 @@ class BlockBlastNetwork(nn.Module):
         planes = _pack_mask_planes(action_mask)
         act, logp, ent = self.head_from_logits(logits, planes, action, deterministic)
         return act.long(), logp, ent, value
-
-    def evaluate_actions_fused(self, x_nchw, mask_planes, action):
-        """Same as evaluate_actions with the categorical head fused (MaskedHead); takes the packed
-        mask planes int64 [3,B] instead of the dense mask."""
-        logits, value = self.trunk(x_nchw)
-        logp, ent = MaskedHead.apply(logits, mask_planes, action)
-        return action, logp, ent, value
 
     def evaluate_actions(self, x_nchw, action_mask, action):
         """Differentiable log-prob / masked entropy of given actions (PPO update,

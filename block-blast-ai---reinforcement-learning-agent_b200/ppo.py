@@ -13,8 +13,6 @@ from typing import Tuple
 
 import numpy as np
 import torch
-import torch.nn as nn
-import torch.nn.functional as F
 
 from . import capi, dist
 from .network import BlockBlastNetwork, PPOLossTail, _pack_mask_planes
@@ -37,7 +35,6 @@ class PPOConfig:
     fc_hidden: Tuple[int, ...] = (512, 256)
     precision: str = "fp32"          # "fp32" (reference numerics) | "bf16" (autocast, channels_last)
     fused_bn: bool = True            # bf16 only: BatchNorm + ReLU (+ residual add) as bb_bn_relu_* kernels around cuDNN's convs
-    fused_head: bool = True          # PPO update: the loss tail after the CNN as one kernel (bb_ppo_loss) instead of torch ops
 
     def to_dict(self):
         return {f.name: getattr(self, f.name) for f in fields(self)}
@@ -195,6 +192,11 @@ class PPOAgent:
         self.optimizer.step()
         sums += torch.stack([means[0], means[1], means[2], loss.detach().double(), means[3], means[4]])
 
+    def _minibatch(self, buffer, idx, mean_std, out, sums):
+        """gather (bb_gather_minibatch) of samples ``idx``, then one optimiser step on them."""
+        g = buffer.gather(idx, mean_std, out=out)
+        self._fused_step(g["obs"], g["mask"], g["actions"], g["logp"], g["adv"], g["ret"], sums)
+
     def _graph_step(self, buffer):
         """The minibatch step as a replayable CUDA graph: gather (bb_gather_minibatch) of the static
         index tensor, CNN forward / backward, loss tail, gradient all-reduce, clip, Adam — ~250
@@ -208,72 +210,41 @@ class PPOAgent:
               "ms": torch.zeros(2, dtype=torch.float32, device=dev),
               "sums": torch.zeros(6, dtype=torch.float64, device=dev)}
         st["out"] = buffer.gather(st["idx"], st["ms"])
-
-        def body():
-            g = buffer.gather(st["idx"], st["ms"], out=st["out"])
-            self._fused_step(g["obs"], g["mask"], g["actions"], g["logp"], g["adv"], g["ret"], st["sums"])
-
         graph = torch.cuda.CUDAGraph()
         with torch.cuda.graph(graph):
-            body()
+            self._minibatch(buffer, st["idx"], st["ms"], st["out"], st["sums"])
         st["graph"] = graph
         self._graph = st
         return st
 
     def update(self, buffer, last_values, use_graph=False):
-        """ppo.py:330-423.  Returns the reference's metric dict.  ``use_graph``: replay the minibatch
-        step as a CUDA graph (fused path, full minibatches; the first update always runs eagerly so
-        that cuDNN autotuning and the optimiser state exist before the capture)."""
+        """ppo.py:330-423.  Returns the reference's metric dict.  Every minibatch is ``_minibatch``;
+        with ``use_graph`` and full minibatches it is replayed as a captured CUDA graph (the first
+        update always runs eagerly so that cuDNN autotuning and the optimiser state exist before the
+        capture)."""
         cfg = self.config
         buffer.compute_returns_and_advantages(last_values, cfg.gamma, cfg.gae_lambda)
-        sums = torch.zeros(6, dtype=torch.float64, device=self.device)
-        n_updates = 0
         self.bucket.rebind()
-        fused = cfg.fused_head and buffer.piece_planes is None
-        total = buffer.buffer_size * buffer.num_envs
+        total, b = buffer.buffer_size * buffer.num_envs, cfg.batch_size
         self._updates_done = getattr(self, "_updates_done", 0) + 1
-        if use_graph and fused and total % cfg.batch_size == 0 and self._updates_done > 1:
-            st = self._graph_step(buffer)
-            mean, std = buffer.advantage_mean_std()
-            st["ms"].copy_(torch.stack([mean, std]).float())
-            st["sums"].zero_()
-            for _ in range(cfg.num_epochs):
-                perm = torch.randperm(total, device=self.device)
-                for start in range(0, total, cfg.batch_size):
-                    st["idx"].copy_(perm[start:start + cfg.batch_size])
-                    st["graph"].replay()
-                    n_updates += 1
-            s = (st["sums"] / max(n_updates, 1)).cpu().tolist()
-            return {"policy_loss": s[0], "value_loss": s[1], "entropy": s[2], "total_loss": s[3],
-                    "approx_kl": s[4], "clip_fraction": s[5]}
+        graph = use_graph and total % b == 0 and self._updates_done > 1
+        st = self._graph_step(buffer) if graph else None
+        mean, std = buffer.advantage_mean_std()
+        ms = torch.stack([mean, std]).float()
+        if graph:
+            st["ms"].copy_(ms)
+            sums = st["sums"].zero_()
+        else:
+            sums = torch.zeros(6, dtype=torch.float64, device=self.device)
+        n_updates = 0
         for _ in range(cfg.num_epochs):
-            for obs, mask, actions, old_logp, adv, ret in buffer.iter_minibatches(cfg.batch_size, packed_mask=fused):
-                if fused:           # mask = int64 planes [3,B]: trunk in torch, everything after it in one kernel
-                    self._fused_step(obs, mask, actions, old_logp, adv, ret, sums)
-                    n_updates += 1
-                    continue
-                if cfg.precision == "bf16":
-                    obs = obs.contiguous(memory_format=torch.channels_last)
-                with self._autocast():
-                    _, new_logp, entropy, values = self.network.evaluate_actions(obs, mask, actions)
-                values = values.float()
-                ratio = torch.exp(new_logp - old_logp)
-                surr1 = ratio * adv
-                surr2 = torch.clamp(ratio, 1 - cfg.clip_epsilon, 1 + cfg.clip_epsilon) * adv
-                policy_loss = -torch.min(surr1, surr2).mean()
-                value_loss = F.mse_loss(values, ret)
-                entropy_loss = -entropy.mean()
-                loss = policy_loss + cfg.value_coef * value_loss + cfg.entropy_coef * entropy_loss
-                self.bucket.zero()
-                loss.backward()
-                self.bucket.all_reduce_mean()                      # C1: one flat NCCL all-reduce
-                self.bucket.clip_grad_norm_(cfg.max_grad_norm)
-                self.optimizer.step()
-                with torch.no_grad():
-                    approx_kl = ((ratio - 1) - torch.log(ratio)).mean()
-                    clip_frac = ((ratio - 1).abs() > cfg.clip_epsilon).float().mean()
-                    sums += torch.stack([policy_loss.detach(), value_loss.detach(), entropy.mean().detach(),
-                                         loss.detach(), approx_kl, clip_frac]).double()
+            perm = torch.randperm(total, device=self.device)
+            for start in range(0, total, b):
+                if graph:
+                    st["idx"].copy_(perm[start:start + b])
+                    st["graph"].replay()
+                else:
+                    self._minibatch(buffer, perm[start:start + b], ms, None, sums)
                 n_updates += 1
         s = (sums / max(n_updates, 1)).cpu().tolist()
         return {"policy_loss": s[0], "value_loss": s[1], "entropy": s[2], "total_loss": s[3],
@@ -289,7 +260,7 @@ class PPOAgent:
         fused / foreach / capturable flags of ours.  ``b200_state`` (ignored by the reference)
         carries the sampling-noise position for --resume."""
         cfgd = {k: (list(v) if isinstance(v, tuple) else v) for k, v in self.config.to_dict().items()
-                if k not in ("precision", "fused_head", "fused_bn")}
+                if k not in ("precision", "fused_bn")}
         opt = self.optimizer.state_dict()
         opt = {"state": {k: {n: (v.detach().cpu().float().reshape(()) if n == "step" and torch.is_tensor(v) else v)
                              for n, v in st.items()} for k, st in opt["state"].items()},
@@ -312,7 +283,7 @@ class PPOAgent:
         if "config" in ck:
             cfg = {k: (tuple(v) if isinstance(v, list) else v) for k, v in ck["config"].items()}
             self.config = PPOConfig.from_dict({**cfg, "precision": self.config.precision,
-                                               "fused_head": self.config.fused_head, "fused_bn": self.config.fused_bn})
+                                               "fused_bn": self.config.fused_bn})
         if "b200_state" in ck:
             self.network.sample_calls = ck["b200_state"].get("sample_calls", 0)
         self.bucket.rebind()

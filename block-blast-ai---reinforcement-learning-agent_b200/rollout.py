@@ -23,13 +23,24 @@ def _to_dev(x, device, dtype):
 
 def pack_dense_obs(board, pieces_planes, action_mask, device):
     """Reference-layout observation (board (N,8,8), pieces (N,3,8,8), action_mask (N,192)) ->
-    packed (board int64[N], piece planes int64[3,N] , mask planes int64[3,N]).  Only used when
-    a caller hands dense arrays to ``add`` (compatibility path)."""
+    the packed protocol the env writes: board int64[N], pieces word int32[N] (piece ids in bytes
+    0-2, used flags in bits 24-26), mask planes int64[3,N].  Each piece plane is looked up in the
+    library's piece table; an all-zero plane is a used slot.  Raises ValueError for a plane that
+    is not one of the 37 pieces drawn at the origin."""
     w = (2 ** torch.arange(64, device=device, dtype=torch.int64))          # bit weights (wraps at 2**63)
     b = (_to_dev(board, device, torch.float32).reshape(-1, 64) != 0).to(torch.int64)
     p = (_to_dev(pieces_planes, device, torch.float32).reshape(-1, 3, 64) != 0).to(torch.int64)
     m = (_to_dev(action_mask, device, torch.float32).reshape(-1, 3, 64) != 0).to(torch.int64)
-    return (b * w).sum(-1), (p * w).sum(-1).t().contiguous(), (m * w).sum(-1).t().contiguous()
+    planes = (p * w).sum(-1)                                                # [N,3]
+    table = torch.as_tensor(capi.piece_table()[0].view(np.int64), device=device)
+    hit = planes.unsqueeze(-1) == table                                     # [N,3,37]; the 37 masks are distinct
+    used = planes == 0
+    if bool((~used & ~hit.any(-1)).any()):
+        raise ValueError("RolloutBuffer.add: a piece plane is neither empty nor a piece at the origin")
+    ids = (hit.to(torch.int64) * torch.arange(37, device=device)).sum(-1)   # 0 for a used slot
+    k = torch.arange(3, device=device)
+    word = ((ids << (8 * k)) | (used.to(torch.int64) << (24 + k))).sum(-1).to(torch.int32)
+    return (b * w).sum(-1), word, (m * w).sum(-1).t().contiguous()
 
 
 class RolloutBuffer:
@@ -47,9 +58,7 @@ class RolloutBuffer:
         # one after the last step.  On the device-resident path the step kernel writes row t+1 itself
         # (obs_row), so collecting a rollout copies nothing.
         self.boards = torch.zeros((T + 1, N), dtype=torch.int64, device=dev)
-        # piece planes are stored as the packed pieces word when available, else as planes
         self.pieces = torch.zeros((T + 1, N), dtype=torch.int32, device=dev)
-        self.piece_planes = None                      # int64 [T,3,N], allocated by the dense path only
         self.action_masks = torch.zeros((T + 1, 3, N), dtype=torch.int64, device=dev)
         self.terminated = torch.zeros((T, N), dtype=torch.uint8, device=dev)   # raw done flags of the step kernel
         self.actions = torch.zeros((T, N), dtype=torch.int32, device=dev)
@@ -65,42 +74,18 @@ class RolloutBuffer:
     # ------------------------------------------------------------------ filling
     def add(self, board, pieces, action_mask, action, log_prob, reward, done, value):
         """ppo.py:116-139.  Accepts either packed tensors (board int64[N], pieces int32[N],
-        action_mask int64[3,N]) or the reference's dense arrays."""
+        action_mask int64[3,N]) or the reference's dense arrays, which are packed on the way in."""
         t, dev = self.ptr, self.device
-        if isinstance(board, torch.Tensor) and board.dtype == torch.int64 and board.dim() == 1:
-            self.boards[t].copy_(board, non_blocking=True)
-            self.pieces[t].copy_(pieces, non_blocking=True)
-            self.action_masks[t].copy_(action_mask, non_blocking=True)
-        else:
-            b, pp, m = pack_dense_obs(board, pieces, action_mask, dev)
-            if self.piece_planes is None:
-                self.piece_planes = torch.zeros((self.buffer_size, 3, self.num_envs), dtype=torch.int64, device=dev)
-            self.boards[t], self.piece_planes[t], self.action_masks[t] = b, pp, m
+        if not (isinstance(board, torch.Tensor) and board.dtype == torch.int64 and board.dim() == 1):
+            board, pieces, action_mask = pack_dense_obs(board, pieces, action_mask, dev)
+        self.boards[t].copy_(board, non_blocking=True)
+        self.pieces[t].copy_(pieces, non_blocking=True)
+        self.action_masks[t].copy_(action_mask, non_blocking=True)
         self.actions[t] = _to_dev(action, dev, torch.int32)
         self.log_probs[t] = _to_dev(log_prob, dev, torch.float32)
         self.rewards[t] = _to_dev(reward, dev, torch.float32)
         self.dones[t] = _to_dev(done, dev, torch.float32)
         self.values[t] = _to_dev(value, dev, torch.float32)
-        self.ptr += 1
-        if self.ptr >= self.buffer_size:
-            self.full = True
-
-    def add_obs(self, obs, action, log_prob, value):
-        """Fast path, first half: store the packed observation the action was chosen on (the env
-        overwrites its observation tensors in place on the next step) plus action/log-prob/value."""
-        t = self.ptr
-        self.boards[t].copy_(obs["board"], non_blocking=True)
-        self.pieces[t].copy_(obs["pieces"], non_blocking=True)
-        self.action_masks[t].copy_(obs["mask"], non_blocking=True)
-        self.actions[t].copy_(action, non_blocking=True)
-        self.log_probs[t].copy_(log_prob, non_blocking=True)
-        self.values[t].copy_(value, non_blocking=True)
-
-    def add_outcome(self, reward, done):
-        """Fast path, second half: reward and done flag of the step just taken."""
-        t = self.ptr
-        self.rewards[t].copy_(reward, non_blocking=True)
-        self.dones[t].copy_(done, non_blocking=True)
         self.ptr += 1
         if self.ptr >= self.buffer_size:
             self.full = True
@@ -116,7 +101,7 @@ class RolloutBuffer:
             self.action_masks[0].copy_(obs["mask"], non_blocking=True)
 
     def finish_direct(self):
-        """After a rollout written in place (train.collect_rollout): done flags u8 -> f32, buffer full."""
+        """After a rollout written in place (train.RolloutRunner): done flags u8 -> f32, buffer full."""
         self.dones.copy_(self.terminated)
         self.ptr, self.full = self.buffer_size, True
 
@@ -144,39 +129,11 @@ class RolloutBuffer:
         return mean.float(), var.sqrt().float()
 
     # ------------------------------------------------------------------ minibatches
-    def _expand(self, idx, packed_mask=False):
-        """Gather samples idx (flat over T*N) and expand them to (B,4,8,8) f32 + (B,192) f32
-        (or, with packed_mask, the int64 [3,B] mask planes the fused head consumes)."""
-        n = idx.numel()
-        T, N = self.buffer_size, self.num_envs
-        boards = self.boards.view(-1)[idx]
-        t_i, n_i = idx // N, idx % N
-        masks = self.action_masks[t_i, :, n_i].t().contiguous()            # [3,B]
-        obs = torch.empty((n, 4, 8, 8), dtype=torch.float32, device=self.device)
-        if packed_mask and self.piece_planes is None:
-            capi.unpack_obs(boards, self.pieces.view(-1)[idx], masks, n, obs=obs, mask_dense=None, n=n)
-            return obs, masks
-        dense = torch.empty((n, 192), dtype=torch.float32, device=self.device)
-        if self.piece_planes is None:
-            pieces = self.pieces.view(-1)[idx]
-            capi.unpack_obs(boards, pieces, masks, n, obs=obs, mask_dense=dense, n=n)
-        else:
-            # dense-path buffers carry piece planes, not ids: expand the three planes like boards
-            pl = self.piece_planes[t_i, :, n_i].t().contiguous()           # [3,B]
-            zero = torch.full((n,), 0x07000000, dtype=torch.int32, device=self.device)   # all "used": planes stay 0
-            capi.unpack_obs(boards, zero, masks, n, obs=obs, mask_dense=dense, n=n)
-            tmp = torch.empty((n, 4, 8, 8), dtype=torch.float32, device=self.device)
-            for k in range(3):
-                capi.unpack_obs(pl[k].contiguous(), zero, masks, n, obs=tmp, mask_dense=None, n=n)
-                obs[:, 1 + k] = tmp[:, 0]
-        return obs, dense
-
     def gather(self, idx, mean_std, obs_dtype=torch.float32, out=None):
         """Minibatch ``idx`` (int64 flat sample indices) of the packed buffer in ONE library call
         (bb_gather_minibatch): obs planes (B,4,8,8), mask planes int64 [3,B], actions int32, old
         log-probs, advantages normalised with ``mean_std`` (float32 [2] device tensor), returns.
         ``out``: a dict of preallocated outputs to fill (static buffers of a captured CUDA graph)."""
-        assert self.piece_planes is None, "gather() needs the packed pieces words"
         b, dev = idx.numel(), self.device
         if out is None:
             out = dict(obs=torch.empty((b, 4, 8, 8), dtype=obs_dtype, device=dev),
@@ -190,27 +147,17 @@ class RolloutBuffer:
                               out["actions"], out["logp"], out["adv"], out["ret"])
         return out
 
-    def iter_minibatches(self, batch_size, generator=None, packed_mask=False):
-        """Fast path: yields (obs_nchw f32 (B,4,8,8), mask f32 (B,192) [or int64 planes [3,B] with
-        packed_mask], actions i64, old_log_probs, normalised advantages, returns), all CUDA tensors."""
+    def get_samples(self, batch_size):
+        """ppo.py:171-213: yields (boards (B,8,8), pieces (B,3,8,8), action_masks (B,192) f32,
+        actions int64, old_log_probs, advantages, returns) in the reference's layouts (CUDA
+        tensors), one ``gather`` per minibatch of a random permutation."""
         total = self.buffer_size * self.num_envs
         mean, std = self.advantage_mean_std()
-        perm = torch.randperm(total, device=self.device, generator=generator)
-        if packed_mask and self.piece_planes is None:
-            ms = torch.stack([mean, std]).float()
-            for start in range(0, total, batch_size):
-                g = self.gather(perm[start:start + batch_size], ms)
-                yield g["obs"], g["mask"], g["actions"], g["logp"], g["adv"], g["ret"]
-            return
-        adv = (self.advantages.view(-1) - mean) / (std + 1e-8)
+        ms = torch.stack([mean, std])
+        perm = torch.randperm(total, device=self.device)
         for start in range(0, total, batch_size):
-            idx = perm[start:start + batch_size]
-            obs, dense = self._expand(idx, packed_mask and self.piece_planes is None)
-            yield (obs, dense, self.actions.view(-1)[idx].long(), self.log_probs.view(-1)[idx], adv[idx],
-                   self.returns.view(-1)[idx])
-
-    def get_samples(self, batch_size):
-        """ppo.py:171-213: yields (boards, pieces, action_masks, actions, old_log_probs,
-        advantages, returns) in the reference's layouts (CUDA tensors)."""
-        for obs, dense, act, lp, adv, ret in self.iter_minibatches(batch_size):
-            yield obs[:, 0], obs[:, 1:], dense, act, lp, adv, ret
+            g = self.gather(perm[start:start + batch_size], ms)
+            b = g["actions"].numel()
+            dense = torch.empty((b, 192), dtype=torch.float32, device=self.device)
+            capi.unpack_obs(None, None, g["mask"], b, mask_dense=dense, n=b)
+            yield g["obs"][:, 0], g["obs"][:, 1:], dense, g["actions"].long(), g["logp"], g["adv"], g["ret"]

@@ -37,25 +37,6 @@ def set_seed(seed):
     torch.cuda.manual_seed_all(seed)
 
 
-def collect_rollout(vec_env, agent, buffer, obs, ep):
-    """scripts/train.py:173-203: one rollout of buffer.buffer_size steps, all on the device.
-    ``ep`` accumulates episode statistics as device scalars [count, sum score, max score, sum len].
-    Generic form over the public step() API; the training loop itself uses RolloutRunner."""
-    buffer.reset()
-    for _ in range(buffer.buffer_size):
-        actions, log_probs, values = agent.act(obs)
-        buffer.add_obs(obs, actions, log_probs, values)
-        obs, rewards, terminated, truncated, infos = vec_env.step(actions)
-        buffer.add_outcome(rewards, terminated.float())
-        t = terminated
-        sc = torch.where(t, infos["ep_score"], torch.zeros_like(infos["ep_score"]))
-        ep[0] += t.sum()
-        ep[1] += sc.sum()
-        ep[2] = torch.maximum(ep[2], sc.max())
-        ep[3] += torch.where(t, infos["ep_len"], torch.zeros_like(infos["ep_len"])).sum()
-    return obs
-
-
 class RolloutRunner:
     """The collect phase of scripts/train.py:173-207 with every result written in place: K2 -> CNN ->
     K3 put action / log-prob / value straight into row t of the RolloutBuffer, K1 puts reward, done flag

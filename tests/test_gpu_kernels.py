@@ -199,10 +199,11 @@ def test_sampling_is_valid_reproducible_and_distributed_like_softmax(torch):
 
 
 @pytest.mark.parametrize("dtype", ["float32", "bfloat16"])
-def test_fused_head_backward_matches_torch_autograd(torch, dtype):
-    """MaskedHead (K3 forward + bb_masked_head_backward) against autograd through the torch
-    restatement of network.py:210-262 (which tests/test_ppo_host.py pins to the reference)."""
-    from bbgpu.network import BlockBlastNetwork, MaskedHead, _pack_mask_planes
+def test_masked_head_backward_kernel_matches_torch_autograd(torch, dtype):
+    """K3 in evaluate mode (log-prob, entropy) and bb_masked_head_backward against autograd through
+    the torch restatement of network.py:210-262 (which tests/test_ppo_host.py pins to the reference)."""
+    from bbgpu import capi
+    from bbgpu.network import _pack_mask_planes
     torch.manual_seed(3)
     n = 4096
     dt = getattr(torch, dtype)
@@ -226,15 +227,17 @@ def test_fused_head_backward_matches_torch_autograd(torch, dtype):
     a = base.clone().requires_grad_(True)
     lp_r, en_r = ref(a)
     (w1 * lp_r + w2 * en_r).sum().backward()
-    b = base.clone().requires_grad_(True)
-    lp_f, en_f = MaskedHead.apply(b, planes, act)
-    (w1 * lp_f + w2 * en_f).sum().backward()
+    act32 = act.to(torch.int32)
+    lp_f, en_f = torch.empty(n, device="cuda"), torch.empty(n, device="cuda")
+    capi.masked_sample(base, planes, planes.stride(0), 0, 0, 2, act32, lp_f, en_f)
+    grad = torch.empty_like(base)                                # d(w1 . logp + w2 . entropy) / d logits
+    capi.masked_head_backward(base, planes, planes.stride(0), act32, w1, w2, grad)
     torch.testing.assert_close(lp_f, lp_r, rtol=1e-5, atol=2e-6)
     torch.testing.assert_close(en_f, en_r, rtol=1e-5, atol=2e-6)
     tol = dict(rtol=2e-2, atol=2e-2) if dtype == "bfloat16" else dict(rtol=1e-4, atol=1e-5)
-    torch.testing.assert_close(b.grad.float(), a.grad.float(), **tol)
-    assert (b.grad[~dense] == 0).all() and b.grad.dtype == dt
-    assert float(b.grad[0].abs().sum()) == 0.0                   # clamped at 1 - eps, like torch
+    torch.testing.assert_close(grad.float(), a.grad.float(), **tol)
+    assert (grad[~dense] == 0).all() and grad.dtype == dt
+    assert float(grad[0].abs().sum()) == 0.0                     # clamped at 1 - eps, like torch
 
 
 @pytest.mark.gpu

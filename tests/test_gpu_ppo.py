@@ -77,7 +77,7 @@ def test_single_env_matches_python_oracle_episode(torch):
     env.close()
 
 
-def test_rollout_buffer_gae_and_samples(torch):
+def test_rollout_buffer_gae_and_gathered_samples(torch):
     from bbgpu.rollout import RolloutBuffer
     from bbgpu.vec_env import VectorizedBlockBlastEnv
     from oracle import bb_oracle as O
@@ -91,10 +91,10 @@ def test_rollout_buffer_gae_and_samples(torch):
         act = venv.sample_valid_actions()
         lp = torch.from_numpy(rs.randn(N).astype(np.float32)).cuda()
         val = torch.from_numpy(rs.randn(N).astype(np.float32)).cuda()
-        kept.append((obs["board"].cpu().numpy().copy(), obs["pieces"].cpu().numpy().copy(), obs["mask"].cpu().numpy().copy()))
-        buf.add_obs(obs, act, lp, val)
+        row = tuple(obs[k].clone() for k in ("board", "pieces", "mask"))     # the env overwrites obs in place
+        kept.append(tuple(x.cpu().numpy() for x in row))
         obs, rew, term, trunc, infos = venv.step(act)
-        buf.add_outcome(rew, term.float())
+        buf.add(*row, act, lp, rew, term.float(), val)
     assert buf.full
     last = torch.from_numpy(rs.randn(N).astype(np.float32)).cuda()
     buf.compute_returns_and_advantages(last, 0.99, 0.95)
@@ -113,33 +113,36 @@ def test_rollout_buffer_gae_and_samples(torch):
     mean, std = buf.advantage_mean_std()
     got = ((buf.advantages.view(-1) - mean) / (std + 1e-8)).cpu().numpy()
     np.testing.assert_allclose(got, norm, rtol=1e-4, atol=1e-5)
-    idx = torch.arange(T * N, device="cuda")
-    x, dense = buf._expand(idx)
-    x, dense = x.cpu().numpy(), dense.cpu().numpy()
+    ms = torch.stack([mean, std])
+    g = buf.gather(torch.arange(T * N, device="cuda"), ms)
+    x, planes = g["obs"].cpu().numpy(), g["mask"].cpu().numpy()
+    dense = VE.expand_mask(planes.view(np.uint64)).astype(np.float32)
     for t in (0, T // 2, T - 1):
         b, p, m = kept[t]
         sl = slice(t * N, (t + 1) * N)
         assert np.array_equal(x[sl, 0], VE.expand_board(b.view(np.uint64)))
         assert np.array_equal(x[sl, 1:], VE.expand_pieces(p.view(np.uint32)))
         assert np.array_equal(dense[sl], VE.expand_mask(m.view(np.uint64)).astype(np.float32))
-    # the reference-layout add() path stores the same content
+    # the reference-layout add() path stores the same content (the pieces word of a used slot
+    # carries another id byte, so it is compared through its expansion)
     buf2 = RolloutBuffer(2, N)
     b, p, m = kept[0]
     z = np.zeros(N, np.float32)
     for _ in range(2):
         buf2.add(VE.expand_board(b.view(np.uint64)), VE.expand_pieces(p.view(np.uint32)), VE.expand_mask(m.view(np.uint64)),
                  np.zeros(N, np.int64), z, z, z, z)
-    x2, d2 = buf2._expand(torch.arange(N, device="cuda"))
-    assert np.array_equal(x2.cpu().numpy(), x[:N]) and np.array_equal(d2.cpu().numpy(), dense[:N])
+    g2 = buf2.gather(torch.arange(N, device="cuda"), ms)
+    assert np.array_equal(g2["obs"].cpu().numpy(), x[:N]) and np.array_equal(g2["mask"].cpu().numpy(), planes[:, :N])
     venv.close()
 
 
-def test_ppo_update_metrics_match_independent_computation(torch):
+def test_ppo_update_metrics_on_runner_rollout_match_independent_computation(torch):
     """One epoch, one minibatch = the whole buffer, eval mode (no dropout / batch-stat noise):
     the metrics of PPOAgent.update must equal ppo.py:372-406 evaluated with the oracle's
     masked log-prob / entropy on the same logits."""
     from bbgpu.ppo import PPOAgent, PPOConfig
     from bbgpu.rollout import RolloutBuffer
+    from bbgpu.train import RolloutRunner
     from bbgpu.vec_env import VectorizedBlockBlastEnv
     from bbgpu import vec_env as VE
     from oracle import bb_oracle as O
@@ -148,24 +151,19 @@ def test_ppo_update_metrics_match_independent_computation(torch):
     agent = PPOAgent(PPOConfig(num_epochs=1, batch_size=T * N, learning_rate=1e-3))
     agent.eval()
     venv = VectorizedBlockBlastEnv(N, seed=9, output="packed")
-    obs, _ = venv.reset()
+    venv.reset()
     buf = RolloutBuffer(T, N)
-    for t in range(T):
-        act, lp, val = agent.act(obs)
-        buf.add_obs(obs, act, lp, val)
-        obs, rew, term, _, _ = venv.step(act)
-        assert (rew > -5).all()                       # K3 only samples valid actions
-        buf.add_outcome(rew, term.float())
-    last = agent.values(obs)
+    last = RolloutRunner(venv, agent, buf, use_graph=False).run()
+    assert (buf.rewards > -5).all()                   # K3 only samples valid actions
     # independent expectation, before the update changes the weights
-    idx = torch.arange(T * N, device="cuda")
-    x, dense = buf._expand(idx)
+    g = buf.gather(torch.arange(T * N, device="cuda"), None)
+    dense = VE.expand_mask(g["mask"].cpu().numpy().view(np.uint64)).astype(np.float32)
     with torch.no_grad():
-        logits, values = agent.network.trunk(x)
+        logits, values = agent.network.trunk(g["obs"])
     adv, ret = O.gae(buf.rewards.cpu().numpy(), buf.values.cpu().numpy(), buf.dones.cpu().numpy(), last.cpu().numpy(), 0.99, 0.95)
     a_n = O.normalize_advantages(adv)
     acts = buf.actions.view(-1).cpu().numpy()
-    _, new_lp, ent = O.masked_policy_terms(logits.cpu().numpy(), dense.cpu().numpy(), acts)
+    _, new_lp, ent = O.masked_policy_terms(logits.cpu().numpy(), dense, acts)
     old_lp = buf.log_probs.view(-1).cpu().numpy()
     np.testing.assert_allclose(new_lp, old_lp, rtol=1e-4, atol=1e-5)     # K3's log-prob == oracle's on the same weights
     ratio = np.exp(new_lp - old_lp)
@@ -509,3 +507,89 @@ def test_gather_minibatch_equals_fancy_indexing(torch, obs_dtype):
     capi.unpack_obs(buf.boards[t_i, n_i].contiguous(), buf.pieces[t_i, n_i].contiguous(), out["mask"], B, obs=ref, n=B)
     assert torch.equal(out["obs"], ref) and out["obs"].dtype == dt
     assert float(out["obs"][:, 0].float().sum()) == float(sum(bin(int(x) & (2 ** 64 - 1)).count("1") for x in buf.boards[t_i, n_i].tolist()))
+
+
+def test_dense_add_stores_the_packed_rows(torch):
+    """RolloutBuffer.add with the reference's dense arrays packs them into the rows the env writes:
+    gather gives the same minibatch as from a buffer filled with those packed rows, PPOAgent.update
+    runs on it (three minibatches, the last one short), and a piece plane that is not a piece at the
+    origin is rejected."""
+    from bbgpu import vec_env as VE
+    from bbgpu.ppo import PPOAgent, PPOConfig
+    from bbgpu.rollout import RolloutBuffer
+    from bbgpu.vec_env import VectorizedBlockBlastEnv
+    T, N = 4, 64
+    venv = VectorizedBlockBlastEnv(N, seed=3, output="packed")
+    obs, _ = venv.reset()
+    dense_buf, packed_buf = RolloutBuffer(T, N), RolloutBuffer(T, N)
+    rs = np.random.RandomState(2)
+    for t in range(T):
+        act = venv.sample_valid_actions()
+        lp, val = (torch.from_numpy(rs.randn(N).astype(np.float32)).cuda() for _ in range(2))
+        row = tuple(obs[k].clone() for k in ("board", "pieces", "mask"))
+        obs, rew, term, _, _ = venv.step(act)
+        packed_buf.add(*row, act, lp, rew, term.float(), val)
+        b, p, m = (x.cpu().numpy() for x in row)
+        dense_buf.add(VE.expand_board(b.view(np.uint64)), VE.expand_pieces(p.view(np.uint32)),
+                      VE.expand_mask(m.view(np.uint64)), act.cpu().numpy(), lp.cpu().numpy(), rew.cpu().numpy(),
+                      term.float().cpu().numpy(), val.cpu().numpy())
+    assert ((packed_buf.pieces[:T] >> 24) & 7).any()           # used slots (all-zero planes) are covered
+    last = torch.from_numpy(rs.randn(N).astype(np.float32)).cuda()
+    for buf in (dense_buf, packed_buf):
+        buf.compute_returns_and_advantages(last, 0.99, 0.95)
+    ms = torch.stack(packed_buf.advantage_mean_std())
+    idx = torch.randperm(T * N, device="cuda")
+    gd, gp = dense_buf.gather(idx, ms), packed_buf.gather(idx, ms)
+    for k in gp:
+        assert torch.equal(gd[k], gp[k]), k
+    agent = PPOAgent(PPOConfig(num_epochs=1, batch_size=100))
+    metrics = agent.update(dense_buf, last)
+    assert all(np.isfinite(v) for v in metrics.values())
+    bad = VE.expand_pieces(p.view(np.uint32)).copy()
+    bad[5, 1] = 0
+    bad[5, 1, 7, 7] = 1                                         # one cell, but not at the origin
+    with pytest.raises(ValueError):
+        RolloutBuffer(1, N).add(VE.expand_board(b.view(np.uint64)), bad, VE.expand_mask(m.view(np.uint64)),
+                                np.zeros(N, np.int64), *(np.zeros(N, np.float32),) * 4)
+    venv.close()
+
+
+def test_get_samples_equals_the_torch_formula_bitwise(torch):
+    """get_samples (gather + one dense-mask expansion per minibatch) yields, bit for bit, what the
+    torch statement of ppo.py:171-213 yields on the same permutation: float32 advantages
+    (a - mean) / (std + 1e-8), fancy-indexed scalars, K2-expanded planes and dense mask."""
+    from bbgpu import capi
+    from bbgpu.rollout import RolloutBuffer
+    T, N, B = 6, 37, 64                                          # 222 samples: the last minibatch is short
+    g = torch.Generator(device="cuda").manual_seed(5)
+    buf = RolloutBuffer(T, N)
+    buf.boards[:T] = torch.randint(-2 ** 62, 2 ** 62, (T, N), device="cuda", generator=g)
+    buf.pieces[:T] = (torch.randint(0, 37, (T, N), device="cuda", generator=g) | (torch.randint(0, 37, (T, N), device="cuda", generator=g) << 8)
+                      | (torch.randint(0, 37, (T, N), device="cuda", generator=g) << 16) | (torch.randint(0, 8, (T, N), device="cuda", generator=g) << 24)).int()
+    buf.action_masks[:T] = torch.randint(-2 ** 62, 2 ** 62, (T, 3, N), device="cuda", generator=g)
+    buf.actions.copy_(torch.randint(0, 192, (T, N), device="cuda", generator=g))
+    for t in (buf.log_probs, buf.rewards, buf.values):
+        t.copy_(torch.randn(T, N, device="cuda", generator=g))
+    buf.dones.copy_((torch.rand(T, N, device="cuda", generator=g) < 0.1).float())
+    buf.compute_returns_and_advantages(torch.randn(N, device="cuda", generator=g), 0.99, 0.95)
+    torch.manual_seed(8)
+    got = list(buf.get_samples(B))
+    torch.manual_seed(8)
+    perm = torch.randperm(T * N, device="cuda")
+    mean, std = buf.advantage_mean_std()
+    adv = (buf.advantages.view(-1) - mean) / (std + 1e-8)
+    assert len(got) == 4
+    for i, start in enumerate(range(0, T * N, B)):
+        idx = perm[start:start + B]
+        n = idx.numel()
+        masks = buf.action_masks[idx // N, :, idx % N].t().contiguous()
+        obs = torch.empty((n, 4, 8, 8), dtype=torch.float32, device="cuda")
+        dense = torch.empty((n, 192), dtype=torch.float32, device="cuda")
+        capi.unpack_obs(buf.boards.view(-1)[idx], buf.pieces.view(-1)[idx], masks, n, obs=obs, mask_dense=dense, n=n)
+        want = (obs[:, 0], obs[:, 1:], dense, buf.actions.view(-1)[idx].long(), buf.log_probs.view(-1)[idx], adv[idx],
+                buf.returns.view(-1)[idx])
+        for k, (w, h) in enumerate(zip(want, got[i])):
+            assert h.dtype == w.dtype and h.shape == w.shape, (i, k)
+            if w.dtype == torch.float32:
+                w, h = w.view(torch.int32), h.view(torch.int32)
+            assert torch.equal(h, w), (i, k)
