@@ -12,7 +12,7 @@ PKG_DIR = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(PKG_DIR, "csrc")
 LIB = os.path.join(PKG_DIR, "libbbgpu.so")
 SOURCES = ["bb_env_kernels.cu", "bb_policy_kernels.cu", "bb_gae_kernels.cu", "bb_bn_kernels.cu", "bb_capi.cu"]
-HEADERS = ["bb_rules.cuh", "bb_kernels.h", "bb_piece_table.inc", os.path.join("..", "..", "include", "bbgpu.h")]
+HEADERS = ["bb_rules.cuh", "bb_kernels.h", "bb_piece_table.inc", "bb_sym_table.inc", os.path.join("..", "..", "include", "bbgpu.h")]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
               "--fmad=true", "-Xcompiler", "-fPIC", "-Xptxas", "-v", "-Xptxas", "-warn-spills"]
 

@@ -77,6 +77,9 @@ def lib():
     L.bb_unpack_obs.argtypes = [vp, vp, vp, i64, vp, C.c_int, vp, C.c_int, i64, vp]
     L.bb_unpack_obs_reference_layout.argtypes = [vp, vp, vp, i64, vp, vp, vp, i64, vp]
     L.bb_gather_minibatch.argtypes = [vp, i64, i64, vp, vp, vp, vp, vp, vp, vp, vp, vp, C.c_int, vp, vp, vp, vp, vp, vp]
+    L.bb_unpack_obs_sym.argtypes = [vp, vp, vp, vp, C.c_int, i64, vp]
+    L.bb_sym_logits_mean.argtypes = [vp, C.c_int, vp, vp, i64, vp]
+    L.bb_sym_logits_mean_backward.argtypes = [vp, vp, vp, C.c_int, i64, vp]
     L.bb_masked_sample.argtypes = [vp, C.c_int, vp, i64, u64, u64, C.c_int, vp, vp, vp, i64, i64, vp, vp]
     L.bb_masked_head_backward.argtypes = [vp, C.c_int, vp, i64, vp, vp, vp, vp, i64, vp]
     L.bb_ppo_loss.argtypes = [vp, C.c_int, vp, i64, vp, vp, vp, vp, vp, C.c_double, C.c_double, C.c_double, vp, vp, vp, i64, vp]
@@ -312,11 +315,38 @@ def unpack_obs_reference_layout(board, pieces, mask, mask_stride, board_f32, pie
                                                ptr(pieces_f32), ptr(action_mask_i8), n, current_stream()))
 
 
+def unpack_obs_sym(board, pieces, obs, index=None, n=None):
+    """K7a (bb_unpack_obs_sym): obs [8n,4,8,8] f32 / bf16, row g*n + i = view g of packed row i (or index[i])."""
+    import torch
+    n = int((index.numel() if index is not None else board.numel()) if n is None else n)
+    assert obs.is_contiguous() and obs.shape[0] == 8 * n
+    dt = BB_BF16 if obs.dtype == torch.bfloat16 else BB_F32
+    check(lib().bb_unpack_obs_sym(ptr(board), ptr(pieces), ptr(index), ptr(obs), dt, n, current_stream()))
+
+
+def sym_logits_mean(logits, pieces, out):
+    """K7b forward (bb_sym_logits_mean): logits [8n,192] f32 / bf16, pieces int32 [n] -> out f32 [n,192]."""
+    import torch
+    n = pieces.numel()
+    assert logits.is_contiguous() and logits.shape == (8 * n, 192) and out.dtype == torch.float32 and out.is_contiguous()
+    dt = BB_BF16 if logits.dtype == torch.bfloat16 else BB_F32
+    check(lib().bb_sym_logits_mean(ptr(logits), dt, ptr(pieces), ptr(out), n, current_stream()))
+
+
+def sym_logits_mean_backward(grad_out, pieces, grad_logits):
+    """K7b backward (bb_sym_logits_mean_backward): grad_out f32 [n,192] -> grad_logits [8n,192] f32 / bf16."""
+    import torch
+    n = pieces.numel()
+    assert grad_out.is_contiguous() and grad_out.dtype == torch.float32 and grad_logits.shape == (8 * n, 192)
+    dt = BB_BF16 if grad_logits.dtype == torch.bfloat16 else BB_F32
+    check(lib().bb_sym_logits_mean_backward(ptr(grad_out), ptr(pieces), ptr(grad_logits), dt, n, current_stream()))
+
+
 def gather_minibatch(index, n_envs, board, pieces, mask, action, logp, adv, ret, adv_mean_std, obs, mask_out,
                      action_out, logp_out, adv_out, ret_out):
-    """RolloutBuffer.get_samples' gathers + K2 in one call (bb_gather_minibatch)."""
+    """RolloutBuffer.get_samples' gathers + K2 in one call (bb_gather_minibatch); obs None: no planes."""
     import torch
-    dt = BB_BF16 if obs.dtype == torch.bfloat16 else BB_F32
+    dt = BB_BF16 if obs is not None and obs.dtype == torch.bfloat16 else BB_F32
     check(lib().bb_gather_minibatch(ptr(index), int(index.numel()), int(n_envs), ptr(board), ptr(pieces), ptr(mask),
                                     ptr(action), ptr(logp), ptr(adv), ptr(ret), ptr(adv_mean_std), ptr(obs), dt,
                                     ptr(mask_out), ptr(action_out), ptr(logp_out), ptr(adv_out), ptr(ret_out),

@@ -467,14 +467,50 @@ int bb_gather_minibatch(const int64_t* index, int64_t batch, int64_t n_envs, con
                         const float* adv_mean_std, void* obs_nchw, int obs_dtype, uint64_t* mask_out, int32_t* action_out,
                         float* logp_out, float* adv_out, float* ret_out, void* stream) {
     if (batch < 0 || n_envs <= 0) return fail(-1, "bb_gather_minibatch: bad size");
-    if (obs_dtype != BB_F32 && obs_dtype != BB_BF16) return fail(-1, "bb_gather_minibatch: obs_dtype must be BB_F32 or BB_BF16");
+    if (obs_nchw && obs_dtype != BB_F32 && obs_dtype != BB_BF16)
+        return fail(-1, "bb_gather_minibatch: obs_dtype must be BB_F32 or BB_BF16");
     if (batch == 0) return 0;
-    if (!index || !board || !pieces || !mask || !action || !logp || !adv || !ret || !obs_nchw || !mask_out || !action_out ||
+    // obs_nchw == NULL: no observation planes (the symmetric update expands eight views with bb_unpack_obs_sym)
+    if (!index || !board || !pieces || !mask || !action || !logp || !adv || !ret || !mask_out || !action_out ||
         !logp_out || !adv_out || !ret_out)
         return fail(-1, "bb_gather_minibatch: NULL array");
     BB_CUDA(bb_launch_gather_minibatch(index, batch, n_envs, board, pieces, mask, action, logp, adv, ret, adv_mean_std,
                                        obs_nchw, obs_dtype, mask_out, action_out, logp_out, adv_out, ret_out,
                                        (cudaStream_t)stream), "bb_gather_minibatch launch");
+    return 0;
+}
+
+int bb_unpack_obs_sym(const uint64_t* board, const uint32_t* pieces, const int64_t* index, void* obs_nchw, int obs_dtype,
+                      int64_t n, void* stream) {
+    if (n < 0) return fail(-1, "bb_unpack_obs_sym: negative n");
+    if (obs_dtype != BB_F32 && obs_dtype != BB_BF16) return fail(-1, "bb_unpack_obs_sym: obs_dtype must be BB_F32 or BB_BF16");
+    if (n == 0) return 0;
+    if (!board || !pieces || !obs_nchw) return fail(-1, "bb_unpack_obs_sym: board/pieces/obs_nchw are required");
+    BB_CUDA(bb_launch_unpack_obs_sym(board, pieces, index, obs_nchw, obs_dtype, n, (cudaStream_t)stream),
+            "bb_unpack_obs_sym launch");
+    return 0;
+}
+
+int bb_sym_logits_mean(const void* logits, int logits_dtype, const uint32_t* pieces, float* out, int64_t n, void* stream) {
+    if (n < 0) return fail(-1, "bb_sym_logits_mean: negative n");
+    if (logits_dtype != BB_F32 && logits_dtype != BB_BF16) return fail(-1, "bb_sym_logits_mean: logits_dtype must be BB_F32 or BB_BF16");
+    if (n == 0) return 0;
+    if (!logits || !pieces || !out) return fail(-1, "bb_sym_logits_mean: NULL array");
+    if ((uintptr_t)logits & 15) return fail(-1, "bb_sym_logits_mean: logits must be 16-byte aligned");
+    BB_CUDA(bb_launch_sym_logits_mean(logits, logits_dtype, pieces, out, n, (cudaStream_t)stream), "bb_sym_logits_mean launch");
+    return 0;
+}
+
+int bb_sym_logits_mean_backward(const float* grad_out, const uint32_t* pieces, void* grad_logits, int logits_dtype, int64_t n,
+                                void* stream) {
+    if (n < 0) return fail(-1, "bb_sym_logits_mean_backward: negative n");
+    if (logits_dtype != BB_F32 && logits_dtype != BB_BF16)
+        return fail(-1, "bb_sym_logits_mean_backward: logits_dtype must be BB_F32 or BB_BF16");
+    if (n == 0) return 0;
+    if (!grad_out || !pieces || !grad_logits) return fail(-1, "bb_sym_logits_mean_backward: NULL array");
+    if ((uintptr_t)grad_logits & 15) return fail(-1, "bb_sym_logits_mean_backward: grad_logits must be 16-byte aligned");
+    BB_CUDA(bb_launch_sym_logits_mean_bwd(grad_out, pieces, grad_logits, logits_dtype, n, (cudaStream_t)stream),
+            "bb_sym_logits_mean_backward launch");
     return 0;
 }
 

@@ -61,6 +61,13 @@ cudaError_t bb_launch_gather_minibatch(const int64_t* index, int64_t B, int64_t 
                                        const float* logp, const float* adv, const float* ret, const float* mean_std,
                                        void* obs, int obs_dtype, uint64_t* mask_out, int32_t* action_out, float* logp_out,
                                        float* adv_out, float* ret_out, cudaStream_t stream);
+// K7a (eight views of each row, view-major; index: optional row gather) and K7b (view average of the logits)
+cudaError_t bb_launch_unpack_obs_sym(const uint64_t* board, const uint32_t* pieces, const int64_t* index, void* obs,
+                                     int obs_dtype, int64_t n, cudaStream_t stream);
+cudaError_t bb_launch_sym_logits_mean(const void* logits, int dtype, const uint32_t* pieces, float* out, int64_t n,
+                                      cudaStream_t stream);
+cudaError_t bb_launch_sym_logits_mean_bwd(const float* dout, const uint32_t* pieces, void* dlogits, int dtype, int64_t n,
+                                          cudaStream_t stream);
 cudaError_t bb_launch_masked_sample(const void* logits, int logits_dtype, const uint64_t* mask,
                                     int64_t mask_stride, uint64_t seed, uint64_t call_counter, int mode,
                                     int32_t* action, float* logp, float* entropy, int64_t n, cudaStream_t stream,

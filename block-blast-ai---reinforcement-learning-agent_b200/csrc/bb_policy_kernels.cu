@@ -15,20 +15,32 @@
 #include "bb_kernels.h"
 
 __constant__ uint64_t c_piece_cells[BB_NUM_PIECES + 3] = BB_PIECE_MASKS;
+__constant__ uint64_t c_piece_inb[BB_NUM_PIECES + 3] = BB_PIECE_INB;
+__device__ const BBSymTables g_bb_sym = {BB_SYM_PERM, BB_SYM_SHIFT};
 
 // ------------------------------------------------------------------------------------ K2
 // One item = 16 output bytes, so consecutive lanes always store consecutive 16-byte pieces
 // (full 32-byte sectors per instruction): bf16 item = (env, channel, row) -> 8 values,
 // f32 item = (env, channel, row, half) -> 4 values.
-template <bool BF16>
+// SYM (K7a): output row g*n + i is view g (bb_sym_board / BB_SYM_PERM, bb_rules.cuh) of input row i, so each
+// view is a contiguous block of n rows; `perm` = the [8][40] piece permutation in shared memory.
+template <bool BF16, bool SYM = false>
 __device__ __forceinline__ uint64_t bb_obs_plane(const uint64_t* __restrict__ board, const uint32_t* __restrict__ pieces,
-                                                 const uint64_t* cells, int64_t t, const int64_t* __restrict__ index = nullptr) {
+                                                 const uint64_t* cells, int64_t t, const int64_t* __restrict__ index = nullptr,
+                                                 int64_t n = 0, const uint8_t* perm = nullptr) {
     int64_t env = t >> (BF16 ? 5 : 6);
+    int g = 0;
+    if (SYM) {
+#pragma unroll
+        for (int k = 1; k < BB_SYM_N; ++k) g += env >= k * n ? 1 : 0;
+        env -= g * n;
+    }
     if (index) env = __ldg(index + env);          // minibatch gather: output row -> rollout-buffer sample
     const int ch = (int)(t >> (BF16 ? 3 : 4)) & 3;
-    if (ch == 0) return __ldg(board + env);
+    if (ch == 0) return SYM ? bb_sym_board(g, __ldg(board + env)) : __ldg(board + env);
     const uint32_t pw = __ldg(pieces + env);
-    const uint32_t id = (pw >> (8 * (ch - 1))) & 0xFFu;
+    uint32_t id = (pw >> (8 * (ch - 1))) & 0xFFu;
+    if (SYM && id < BB_NUM_PIECES) id = perm[g * BB_TABLE_N + id];
     const bool used = (pw >> (24 + ch - 1)) & 1u;
     return used ? 0ull : cells[id < BB_NUM_PIECES ? id : BB_NUM_PIECES];
 }
@@ -68,27 +80,34 @@ __device__ __forceinline__ void bb_unpack_obs_item(void* __restrict__ obs, int64
 
 // Grid-stride: a few thousand long-lived blocks instead of one short block per 8 envs (CTA
 // launch rate, not HBM, bounded the one-shot version); two independent items per iteration.
-template <bool BF16>
+// SYM: the eight-view kernel K7a, 8n output rows (see bb_obs_plane).
+template <bool BF16, bool SYM = false>
 __global__ void __launch_bounds__(256)
 bb_unpack_obs_kernel(const uint64_t* __restrict__ board, const uint32_t* __restrict__ pieces,
                      void* __restrict__ obs, int64_t n, void* __restrict__ split, const int64_t* __restrict__ index) {
     __shared__ uint64_t cells[BB_NUM_PIECES + 3];
+    __shared__ uint8_t perm[SYM ? BB_SYM_N * BB_TABLE_N : 1];
     for (int k = threadIdx.x; k < BB_NUM_PIECES + 3; k += blockDim.x) cells[k] = c_piece_cells[k];
+    if (SYM)
+        for (int k = threadIdx.x; k < BB_SYM_N * BB_TABLE_N; k += blockDim.x) perm[k] = g_bb_sym.perm[k / BB_TABLE_N][k % BB_TABLE_N];
     __syncthreads();
-    const int64_t total = n * (BF16 ? 32 : 64);
+    if (SYM) split = nullptr;
+    const int64_t total = (SYM ? BB_SYM_N * n : n) * (BF16 ? 32 : 64);
     const int64_t stride = (int64_t)gridDim.x * blockDim.x;
     int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    for (; t + 3 * stride < total; t += 4 * stride) {
-        const uint64_t p0 = bb_obs_plane<BF16>(board, pieces, cells, t, index);
-        const uint64_t p1 = bb_obs_plane<BF16>(board, pieces, cells, t + stride, index);
-        const uint64_t p2 = bb_obs_plane<BF16>(board, pieces, cells, t + 2 * stride, index);
-        const uint64_t p3 = bb_obs_plane<BF16>(board, pieces, cells, t + 3 * stride, index);
+    // SYM: one item per iteration (the four-item body spills with the view transforms inlined four times)
+    for (; !SYM && t + 3 * stride < total; t += 4 * stride) {
+        const uint64_t p0 = bb_obs_plane<BF16, SYM>(board, pieces, cells, t, index, n, perm);
+        const uint64_t p1 = bb_obs_plane<BF16, SYM>(board, pieces, cells, t + stride, index, n, perm);
+        const uint64_t p2 = bb_obs_plane<BF16, SYM>(board, pieces, cells, t + 2 * stride, index, n, perm);
+        const uint64_t p3 = bb_obs_plane<BF16, SYM>(board, pieces, cells, t + 3 * stride, index, n, perm);
         bb_unpack_obs_item<BF16>(obs, t, p0, split);
         bb_unpack_obs_item<BF16>(obs, t + stride, p1, split);
         bb_unpack_obs_item<BF16>(obs, t + 2 * stride, p2, split);
         bb_unpack_obs_item<BF16>(obs, t + 3 * stride, p3, split);
     }
-    for (; t < total; t += stride) bb_unpack_obs_item<BF16>(obs, t, bb_obs_plane<BF16>(board, pieces, cells, t, index), split);
+    for (; t < total; t += stride)
+        bb_unpack_obs_item<BF16>(obs, t, bb_obs_plane<BF16, SYM>(board, pieces, cells, t, index, n, perm), split);
 }
 
 template <bool F32>
@@ -123,13 +142,25 @@ bb_unpack_mask_kernel(const uint64_t* __restrict__ mask, int64_t stride, void* _
 }
 
 static void bb_launch_obs_planes(const uint64_t* board, const uint32_t* pieces, void* obs, int obs_dtype, int64_t n,
-                                 void* split, const int64_t* index, cudaStream_t stream) {
-    const int64_t threads = n * (obs_dtype == 1 ? 32 : 64);
+                                 void* split, const int64_t* index, cudaStream_t stream, bool sym = false) {
+    const int64_t threads = (sym ? BB_SYM_N * n : n) * (obs_dtype == 1 ? 32 : 64);
     int64_t blocks = (threads + 255) / 256;
     if (blocks > 148 * 16) blocks = 148 * 16;        // grid-stride: 8 resident blocks per SM x 2 waves
     const unsigned grid = (unsigned)blocks;
+    if (sym) {
+        if (obs_dtype == 1) bb_unpack_obs_kernel<true, true><<<grid, 256, 0, stream>>>(board, pieces, obs, n, nullptr, index);
+        else bb_unpack_obs_kernel<false, true><<<grid, 256, 0, stream>>>(board, pieces, obs, n, nullptr, index);
+        return;
+    }
     if (obs_dtype == 1) bb_unpack_obs_kernel<true><<<grid, 256, 0, stream>>>(board, pieces, obs, n, nullptr, index);
     else bb_unpack_obs_kernel<false><<<grid, 256, 0, stream>>>(board, pieces, obs, n, split, index);
+}
+
+cudaError_t bb_launch_unpack_obs_sym(const uint64_t* board, const uint32_t* pieces, const int64_t* index, void* obs,
+                                     int obs_dtype, int64_t n, cudaStream_t stream) {
+    if (n <= 0) return cudaSuccess;
+    bb_launch_obs_planes(board, pieces, obs, obs_dtype, n, nullptr, index, stream, true);
+    return cudaGetLastError();
 }
 
 cudaError_t bb_launch_unpack_obs(const uint64_t* board, const uint32_t* pieces, const uint64_t* mask,
@@ -179,7 +210,7 @@ cudaError_t bb_launch_gather_minibatch(const int64_t* index, int64_t B, int64_t 
                                        void* obs, int obs_dtype, uint64_t* mask_out, int32_t* action_out, float* logp_out,
                                        float* adv_out, float* ret_out, cudaStream_t stream) {
     if (B <= 0) return cudaSuccess;
-    bb_launch_obs_planes(board, pieces, obs, obs_dtype, B, nullptr, index, stream);
+    if (obs) bb_launch_obs_planes(board, pieces, obs, obs_dtype, B, nullptr, index, stream);
     bb_gather_rows_kernel<<<(unsigned)((B + 255) / 256), 256, 0, stream>>>(index, B, N, mask, action, logp, adv, ret, mean_std,
                                                                           mask_out, action_out, logp_out, adv_out, ret_out);
     return cudaGetLastError();
@@ -648,5 +679,141 @@ cudaError_t bb_launch_ppo_loss(const void* logits, int dtype, const uint64_t* ma
         bb_masked_head_bwd_kernel<true, true><<<grid, 128, 0, stream>>>(logits, mask, mask_stride, action, nullptr, nullptr, dlogits, n, L);
     else
         bb_masked_head_bwd_kernel<false, true><<<grid, 128, 0, stream>>>(logits, mask, mask_stride, action, nullptr, nullptr, dlogits, n, L);
+    return cudaGetLastError();
+}
+
+// ------------------------------------------------------------------------------------ K7b
+// Group average of the policy logits over the eight views (K7a rows g*n + i):
+//   out[i, s*64 + a] = 0.125 * sum_{g = 0..7} L[g*n + i, s*64 + sigma_{g,p_s}(a)]      (f32, fixed g order)
+// for an in-bounds anchor a of the slot's piece p_s, 0 elsewhere and for an id >= 37 (positions that are always
+// masked).  The backward pass is the transposed map: every view position receives at most one term,
+// 0.125 * dout, and 0 elsewhere.  A block stages the 8 x BB_K7B_STATES view rows of its states in shared memory
+// with coalesced 16-byte accesses and does the permuted accesses there.  Per state: 8 x 768 B (f32) or
+// 8 x 384 B (bf16) of logits and 768 B of f32 averages.
+#define BB_K7B_STATES 4
+#define BB_K7B_THREADS 256
+
+__device__ __forceinline__ void k7b_load_tables(uint8_t* shift, uint64_t* inb) {
+    for (int k = threadIdx.x; k < BB_SYM_N * BB_TABLE_N; k += blockDim.x) shift[k] = g_bb_sym.shift[k / BB_TABLE_N][k % BB_TABLE_N];
+    for (int k = threadIdx.x; k < BB_TABLE_N; k += blockDim.x) inb[k] = k < BB_NUM_PIECES ? c_piece_inb[k] : 0ull;
+}
+
+// the piece id of output j (= s*64 + a) of a state with pieces word pw, or -1 where the output is always 0
+__device__ __forceinline__ int k7b_piece(const uint64_t* inb, uint32_t pw, int j) {
+    const uint32_t id = (pw >> (8 * (j >> 6))) & 0xFFu;
+    return id < BB_NUM_PIECES && ((inb[id] >> (j & 63)) & 1ull) ? (int)id : -1;
+}
+// position of output j in the row of view g: s*64 + sigma_{g,id}(a)
+__device__ __forceinline__ int k7b_pos(const uint8_t* shift, int id, int j, int g) {
+    return (j & ~63) + bb_sym_cell(g, j & 63) - (int)shift[g * BB_TABLE_N + id];
+}
+
+template <bool BF16>
+__global__ void __launch_bounds__(BB_K7B_THREADS)
+bb_sym_logits_mean_kernel(const void* __restrict__ logits, const uint32_t* __restrict__ pieces, float* __restrict__ out,
+                          int64_t n) {
+    __shared__ float4 tile[BB_SYM_N * BB_K7B_STATES * 48];            // [g][state][192] as f32
+    __shared__ uint8_t shift[BB_SYM_N * BB_TABLE_N];
+    __shared__ uint64_t inb[BB_TABLE_N];
+    k7b_load_tables(shift, inb);
+    const float* tf = reinterpret_cast<const float*>(tile);
+    for (int64_t i0 = (int64_t)blockIdx.x * BB_K7B_STATES; i0 < n; i0 += (int64_t)gridDim.x * BB_K7B_STATES) {
+        const int ns = (int)(n - i0 < BB_K7B_STATES ? n - i0 : BB_K7B_STATES);
+        // view g of the block's states is one contiguous run of rows g*n + i0 .. + ns
+        constexpr int PER_ROW = BF16 ? 24 : 48;                       // 16-byte units per row
+        for (int u = threadIdx.x; u < BB_SYM_N * BB_K7B_STATES * PER_ROW; u += blockDim.x) {
+            const int g = u / (BB_K7B_STATES * PER_ROW), rem = u - g * (BB_K7B_STATES * PER_ROW);
+            const int st = rem / PER_ROW, q = rem - st * PER_ROW;
+            if (st >= ns) continue;
+            const int64_t row = (int64_t)g * n + i0 + st;
+            float4* dst = tile + (g * BB_K7B_STATES + st) * 48;
+            if (BF16) {
+                const uint4 h = __ldcs(reinterpret_cast<const uint4*>(logits) + row * 24 + q);
+                dst[2 * q] = make_float4(__uint_as_float(h.x << 16), __uint_as_float(h.x & 0xFFFF0000u),
+                                         __uint_as_float(h.y << 16), __uint_as_float(h.y & 0xFFFF0000u));
+                dst[2 * q + 1] = make_float4(__uint_as_float(h.z << 16), __uint_as_float(h.z & 0xFFFF0000u),
+                                             __uint_as_float(h.w << 16), __uint_as_float(h.w & 0xFFFF0000u));
+            } else {
+                dst[q] = __ldcs(reinterpret_cast<const float4*>(logits) + row * 48 + q);
+            }
+        }
+        __syncthreads();
+        for (int v = threadIdx.x; v < ns * 192; v += blockDim.x) {
+            const int st = v / 192, j = v - st * 192;
+            const int id = k7b_piece(inb, __ldg(pieces + i0 + st), j);
+            float sum = 0.f;
+            if (id >= 0) {
+#pragma unroll
+                for (int g = 0; g < BB_SYM_N; ++g) sum += tf[(g * BB_K7B_STATES + st) * 192 + k7b_pos(shift, id, j, g)];
+            }
+            out[(i0 + st) * 192 + j] = 0.125f * sum;             // read by K3 / the loss tail next: keep in L2
+        }
+        __syncthreads();
+    }
+}
+
+template <bool BF16>
+__global__ void __launch_bounds__(BB_K7B_THREADS)
+bb_sym_logits_mean_bwd_kernel(const float* __restrict__ dout, const uint32_t* __restrict__ pieces, void* __restrict__ dlogits,
+                              int64_t n) {
+    __shared__ float4 tile[BB_SYM_N * BB_K7B_STATES * 48];
+    __shared__ uint8_t shift[BB_SYM_N * BB_TABLE_N];
+    __shared__ uint64_t inb[BB_TABLE_N];
+    k7b_load_tables(shift, inb);
+    float* tf = reinterpret_cast<float*>(tile);
+    for (int64_t i0 = (int64_t)blockIdx.x * BB_K7B_STATES; i0 < n; i0 += (int64_t)gridDim.x * BB_K7B_STATES) {
+        const int ns = (int)(n - i0 < BB_K7B_STATES ? n - i0 : BB_K7B_STATES);
+        for (int u = threadIdx.x; u < BB_SYM_N * BB_K7B_STATES * 48; u += blockDim.x) tile[u] = make_float4(0.f, 0.f, 0.f, 0.f);
+        __syncthreads();
+        for (int v = threadIdx.x; v < ns * 192; v += blockDim.x) {
+            const int st = v / 192, j = v - st * 192;
+            const int id = k7b_piece(inb, __ldg(pieces + i0 + st), j);
+            if (id < 0) continue;
+            const float d = 0.125f * __ldcs(dout + (i0 + st) * 192 + j);
+#pragma unroll
+            for (int g = 0; g < BB_SYM_N; ++g) tf[(g * BB_K7B_STATES + st) * 192 + k7b_pos(shift, id, j, g)] = d;
+        }
+        __syncthreads();
+        constexpr int PER_ROW = BF16 ? 24 : 48;
+        for (int u = threadIdx.x; u < BB_SYM_N * BB_K7B_STATES * PER_ROW; u += blockDim.x) {
+            const int g = u / (BB_K7B_STATES * PER_ROW), rem = u - g * (BB_K7B_STATES * PER_ROW);
+            const int st = rem / PER_ROW, q = rem - st * PER_ROW;
+            if (st >= ns) continue;
+            const int64_t row = (int64_t)g * n + i0 + st;
+            const float4* src = tile + (g * BB_K7B_STATES + st) * 48;
+            if (BF16) {
+                const float4 a = src[2 * q], b = src[2 * q + 1];
+                const __nv_bfloat162 h0 = __floats2bfloat162_rn(a.x, a.y), h1 = __floats2bfloat162_rn(a.z, a.w);
+                const __nv_bfloat162 h2 = __floats2bfloat162_rn(b.x, b.y), h3 = __floats2bfloat162_rn(b.z, b.w);
+                uint4 w;
+                w.x = *reinterpret_cast<const uint32_t*>(&h0); w.y = *reinterpret_cast<const uint32_t*>(&h1);
+                w.z = *reinterpret_cast<const uint32_t*>(&h2); w.w = *reinterpret_cast<const uint32_t*>(&h3);
+                __stcs(reinterpret_cast<uint4*>(dlogits) + row * 24 + q, w);
+            } else {
+                __stcs(reinterpret_cast<float4*>(dlogits) + row * 48 + q, src[q]);
+            }
+        }
+        __syncthreads();
+    }
+}
+
+static unsigned k7b_grid(int64_t n) {
+    const int64_t want = (n + BB_K7B_STATES - 1) / BB_K7B_STATES;
+    return (unsigned)(want < 148 * 8 ? want : 148 * 8);        // grid-stride: one wave of 8 blocks per SM
+}
+
+cudaError_t bb_launch_sym_logits_mean(const void* logits, int dtype, const uint32_t* pieces, float* out, int64_t n,
+                                      cudaStream_t stream) {
+    if (n <= 0) return cudaSuccess;
+    if (dtype == 1) bb_sym_logits_mean_kernel<true><<<k7b_grid(n), BB_K7B_THREADS, 0, stream>>>(logits, pieces, out, n);
+    else bb_sym_logits_mean_kernel<false><<<k7b_grid(n), BB_K7B_THREADS, 0, stream>>>(logits, pieces, out, n);
+    return cudaGetLastError();
+}
+
+cudaError_t bb_launch_sym_logits_mean_bwd(const float* dout, const uint32_t* pieces, void* dlogits, int dtype, int64_t n,
+                                          cudaStream_t stream) {
+    if (n <= 0) return cudaSuccess;
+    if (dtype == 1) bb_sym_logits_mean_bwd_kernel<true><<<k7b_grid(n), BB_K7B_THREADS, 0, stream>>>(dout, pieces, dlogits, n);
+    else bb_sym_logits_mean_bwd_kernel<false><<<k7b_grid(n), BB_K7B_THREADS, 0, stream>>>(dout, pieces, dlogits, n);
     return cudaGetLastError();
 }

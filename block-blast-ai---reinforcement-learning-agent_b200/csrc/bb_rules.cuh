@@ -27,6 +27,7 @@
 #endif
 
 #include "bb_piece_table.inc"
+#include "bb_sym_table.inc"
 
 // ---------------------------------------------------------------------------------------
 // tables
@@ -860,4 +861,96 @@ BB_HD int bb_expand_item(const BBState& s, const uint64_t m[3], int samples, int
     *k = 0;
     if (bb_expand_deals(s)) { a = j / samples; *k = j - a * samples; }
     return bb_kth_action(m, a);
+}
+
+// ---------------------------------------------------------------------------------------
+// The 8 symmetries of the square (group D4).  The rules are invariant under all of them: the piece
+// set is closed under each (BB_SYM_PERM), and placement, clears, score, holes, center openness and
+// trio solvability only see cell sets.  Ids, as maps of cell (r, c):
+//   0 identity (r, c)      1 R90 (c, 7-r)          2 R180 (7-r, 7-c)      3 R270 (7-c, r)
+//   4 mirror columns (r, 7-c)   5 mirror rows (7-r, c)   6 transpose (c, r)   7 anti-transpose (7-c, 7-r)
+// Each is "transpose, then mirror columns, then mirror rows", each step present or not: bit g of the
+// masks below says whether symmetry g has that step.
+// Pieces: the 8-bit ids of a pieces word map through BB_SYM_PERM (an id >= 37 stays as it is); slot
+// order and used bits are kept.  Actions: slot*64 + a -> slot*64 + sigma_{g,p}(a), with
+// sigma_{g,p}(a) = T_g(a) - BB_SYM_SHIFT[g][p]: the image of the top-left of the piece's bounding box
+// minus the offset of the image box's top-left from it.  A legal anchor maps to a legal anchor of the
+// image piece, so a mask plane maps as T_g(plane) >> shift (no wrap: every image anchor lies below
+// and right of the shift).  Tables: tools/gen_piece_tables.py --sym.
+// ---------------------------------------------------------------------------------------
+#define BB_SYM_N 8
+#define BB_SYM_HAS_TRANSPOSE 0xCAu     // g = 1, 3, 6, 7
+#define BB_SYM_HAS_MIRROR_COLS 0x96u   // g = 1, 2, 4, 7
+#define BB_SYM_HAS_MIRROR_ROWS 0xACu   // g = 2, 3, 5, 7
+
+struct BBSymTables { uint8_t perm[BB_SYM_N][BB_TABLE_N]; uint8_t shift[BB_SYM_N][BB_TABLE_N]; };
+
+static const uint8_t BB_HOST_SYM_PERM[BB_SYM_N][BB_TABLE_N] = BB_SYM_PERM;
+static const uint8_t BB_HOST_SYM_SHIFT[BB_SYM_N][BB_TABLE_N] = BB_SYM_SHIFT;
+
+inline void bb_fill_sym_tables(BBSymTables* t) {
+    for (int g = 0; g < BB_SYM_N; ++g)
+        for (int i = 0; i < BB_TABLE_N; ++i) { t->perm[g][i] = BB_HOST_SYM_PERM[g][i]; t->shift[g][i] = BB_HOST_SYM_SHIFT[g][i]; }
+}
+
+// (r, c) -> (c, r): three delta swaps
+BB_HD uint64_t bb_transpose(uint64_t x) {
+    uint64_t t = 0x0F0F0F0F00000000ull & (x ^ (x << 28)); x ^= t ^ (t >> 28);
+    t = 0x3333000033330000ull & (x ^ (x << 14)); x ^= t ^ (t >> 14);
+    t = 0x5500550055005500ull & (x ^ (x << 7)); x ^= t ^ (t >> 7);
+    return x;
+}
+// (r, c) -> (7-r, c): byte swap
+BB_HD uint64_t bb_mirror_rows(uint64_t x) {
+#if defined(__CUDA_ARCH__)
+    return (uint64_t)__byte_perm((uint32_t)(x >> 32), 0u, 0x0123u) | ((uint64_t)__byte_perm((uint32_t)x, 0u, 0x0123u) << 32);
+#else
+    return __builtin_bswap64(x);
+#endif
+}
+// (r, c) -> (r, 7-c): bit reversal within each byte
+BB_HD uint64_t bb_mirror_cols(uint64_t x) {
+#if defined(__CUDA_ARCH__)
+    // a 32-bit reversal takes (r, c) to (3-r, 7-c) within a half; a byte swap puts the rows back
+    return (uint64_t)__byte_perm(__brev((uint32_t)x), 0u, 0x0123u) |
+           ((uint64_t)__byte_perm(__brev((uint32_t)(x >> 32)), 0u, 0x0123u) << 32);
+#else
+    x = ((x >> 1) & 0x5555555555555555ull) | ((x & 0x5555555555555555ull) << 1);
+    x = ((x >> 2) & 0x3333333333333333ull) | ((x & 0x3333333333333333ull) << 2);
+    return ((x >> 4) & 0x0F0F0F0F0F0F0F0Full) | ((x & 0x0F0F0F0F0F0F0F0Full) << 4);
+#endif
+}
+
+// T_g(board), 0 <= g < 8
+BB_HD uint64_t bb_sym_board(int g, uint64_t b) {
+    if ((BB_SYM_HAS_TRANSPOSE >> g) & 1u) b = bb_transpose(b);
+    if ((BB_SYM_HAS_MIRROR_COLS >> g) & 1u) b = bb_mirror_cols(b);
+    if ((BB_SYM_HAS_MIRROR_ROWS >> g) & 1u) b = bb_mirror_rows(b);
+    return b;
+}
+// T_g of one cell index a = r*8 + c
+BB_HD int bb_sym_cell(int g, int a) {
+    int r = a >> 3, c = a & 7;
+    if ((BB_SYM_HAS_TRANSPOSE >> g) & 1u) { const int t = r; r = c; c = t; }
+    if ((BB_SYM_HAS_MIRROR_COLS >> g) & 1u) c = 7 - c;
+    if ((BB_SYM_HAS_MIRROR_ROWS >> g) & 1u) r = 7 - r;
+    return r * 8 + c;
+}
+// the pieces word of the transformed state: ids mapped, slot order and used bits kept
+BB_HD uint32_t bb_sym_pieces(const BBSymTables* S, int g, uint32_t pw) {
+    uint32_t out = pw & 0xFF000000u;
+#pragma unroll
+    for (int k = 0; k < 3; ++k) {
+        const uint32_t id = (pw >> (8 * k)) & 0xFFu;
+        out |= (uint32_t)(id < BB_NUM_PIECES ? S->perm[g][id] : id) << (8 * k);
+    }
+    return out;
+}
+// sigma_{g,p}(a) for an in-bounds anchor a of piece `id` (< 37)
+BB_HD int bb_sym_anchor(const BBSymTables* S, int g, uint32_t id, int a) {
+    return bb_sym_cell(g, a) - (int)S->shift[g][id];
+}
+// the mask plane of a slot holding piece `id` (< 37) in the transformed state
+BB_HD uint64_t bb_sym_mask_plane(const BBSymTables* S, int g, uint32_t id, uint64_t plane) {
+    return bb_sym_board(g, plane) >> S->shift[g][id];
 }

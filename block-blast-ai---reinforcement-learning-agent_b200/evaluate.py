@@ -11,6 +11,10 @@ like the reference's: scores, lengths, lines cleared, max combo.
 of every env is expanded on the GPU (``bb_env_expand``; a move that places the last piece is dealt K
 sampled trios from the look-ahead stream, never the env's own), the successors are scored by the value
 head, and each env plays the move with the highest mean ``reward + gamma * (1 - terminated) * V``.
+
+``--symmetrize`` evaluates the agent's policy and value as averages over the eight board symmetries
+(``PPOConfig.symmetrize``) even when the checkpoint was trained without them; by default the checkpoint's
+own setting applies.
 """
 import argparse
 import json
@@ -46,12 +50,14 @@ def lookahead_actions(agent, h, n, call_counter, samples, chunk=65536):
 
 @torch.no_grad()
 def evaluate(agent, num_episodes=100, seed=0, deterministic=True, max_steps=10000, reward_config=None,
-             return_actions=False, lookahead=0):
+             return_actions=False, lookahead=0, symmetrize=None):
     """``lookahead``: 0 = the agent's own policy (argmax when ``deterministic``); K >= 1 = one-ply value
     look-ahead with K sampled trios per dealing move (``lookahead_actions``, expansion call counter = the
     step number).  ``return_actions``: also return ``actions`` int32 [steps, n] (the action every env was given at every
     step; entries after an env's game over are ignored by the env) and ``rewards_per_episode`` — enough to
-    replay every episode through another implementation of the rules (tests do, through the oracle)."""
+    replay every episode through another implementation of the rules (tests do, through the oracle).
+    ``symmetrize``: None = the agent's own setting; True / False = with / without the eight-view average for
+    this evaluation (the successor values of ``lookahead`` included)."""
     dev = agent.device
     n = int(num_episodes)
     h = capi.EnvHandle(n, seed, 0, reward_config, capi.ENV_NO_AUTO_RESET)
@@ -62,26 +68,32 @@ def evaluate(agent, num_episodes=100, seed=0, deterministic=True, max_steps=1000
     term = torch.zeros(n, dtype=torch.uint8, device=dev)
     total_reward = torch.zeros(n, dtype=torch.float64, device=dev)
     done = torch.zeros(n, dtype=torch.bool, device=dev)
-    was_training = agent.training
+    was_training, was_sym = agent.training, agent.config.symmetrize
+    if symmetrize is not None:
+        agent.config.symmetrize = bool(symmetrize)
     agent.eval()                                       # scripts/evaluate.py evaluates in eval mode
     steps = 0
     log = []
-    while steps < max_steps and not bool(done.all()):
-        if lookahead:
-            act, _, _ = lookahead_actions(agent, h, n, steps, int(lookahead))
-        else:
-            h.observe(board, pieces, mask)
-            act, _, _ = agent.act({"board": board, "pieces": pieces, "mask": mask}, deterministic=deterministic)
-        if return_actions:
-            log.append(act.clone())
-        h.step(act, rewards, term, None, None, None, None)
-        total_reward += torch.where(done, torch.zeros_like(rewards), rewards).double()
-        done |= term.bool()
-        steps += 1
-    st = h.get_state()
-    h.close()
-    if was_training:
-        agent.train()
+    try:
+        while steps < max_steps and not bool(done.all()):
+            if lookahead:
+                act, _, _ = lookahead_actions(agent, h, n, steps, int(lookahead))
+            else:
+                h.observe(board, pieces, mask)
+                act, _, _ = agent.act({"board": board, "pieces": pieces, "mask": mask}, deterministic=deterministic)
+            if return_actions:
+                log.append(act.clone())
+            h.step(act, rewards, term, None, None, None, None)
+            total_reward += torch.where(done, torch.zeros_like(rewards), rewards).double()
+            done |= term.bool()
+            steps += 1
+        st = h.get_state()
+    finally:
+        # the caller's agent keeps its own policy form and mode whatever happens during the evaluation
+        h.close()
+        agent.config.symmetrize = was_sym
+        if was_training:
+            agent.train()
     scores, lengths = st["score"].astype(np.int64), st["moves"].astype(np.int64)
     extra = {}
     if return_actions:
@@ -103,10 +115,13 @@ def main():
     ap.add_argument("--stochastic", action="store_true")
     ap.add_argument("--lookahead", type=int, default=0,
                     help="K >= 1: one-ply value look-ahead with K sampled trios per dealing move (0 = policy argmax)")
+    ap.add_argument("--symmetrize", action="store_true", default=None,
+                    help="average the policy / value over the 8 board symmetries (default: the checkpoint's setting)")
     a = ap.parse_args()
     agent = PPOAgent()
     agent.load(a.checkpoint)
-    res = evaluate(agent, a.episodes, a.seed, deterministic=not a.stochastic, lookahead=a.lookahead)
+    res = evaluate(agent, a.episodes, a.seed, deterministic=not a.stochastic, lookahead=a.lookahead,
+                   symmetrize=a.symmetrize)
     print(json.dumps({k: v for k, v in res.items() if not isinstance(v, np.ndarray)}, indent=1))
 
 

@@ -171,6 +171,32 @@ class PPOLossTail(torch.autograd.Function):
                 None, None, None, None, None, None, None, None)
 
 
+class SymmetryMean(torch.autograd.Function):
+    """Group average of the policy logits over the eight board symmetries (K7b, bb_sym_logits_mean): raw
+    logits [8n,192] of the eight views (rows g*n + i, as bb_unpack_obs_sym writes the observations) and the
+    pieces words int32 [n] of the states -> f32 [n,192] logits of the states, 0 at positions that are always
+    masked.  The backward pass is the kernel's transposed map, in the logits' dtype."""
+
+    @staticmethod
+    def forward(ctx, logits, pieces):
+        lg = logits.detach()
+        if lg.dtype not in (torch.float32, torch.bfloat16):
+            lg = lg.float()
+        lg = lg.contiguous()
+        out = torch.empty((pieces.numel(), 192), dtype=torch.float32, device=lg.device)
+        capi.sym_logits_mean(lg, pieces, out)
+        ctx.save_for_backward(pieces)
+        ctx.dtype = lg.dtype
+        return out
+
+    @staticmethod
+    def backward(ctx, g):
+        pieces, = ctx.saved_tensors
+        grad = torch.empty((8 * pieces.numel(), 192), dtype=ctx.dtype, device=g.device)
+        capi.sym_logits_mean_backward(g.float().contiguous(), pieces, grad)
+        return grad, None
+
+
 class BlockBlastNetwork(nn.Module):
     def __init__(self, board_size=8, num_pieces=3, conv_channels=(64, 128, 128), fc_hidden=(512, 256),
                  action_space_size=192, use_residual=True, use_batch_norm=True):

@@ -2,8 +2,10 @@
 (src/agents/ppo.py:26-449) on the device-resident path.
 
 Collect: packed obs -> K2 (planes) -> CNN (PyTorch) -> K3 (masked sample + log-prob) -> K1
-(env step), nothing leaves HBM.  Update: K4 GAE, whole-buffer advantage normalisation,
-clipped surrogate + 0.5*MSE value loss + 0.01*entropy (ppo.py:372-392), grad-norm clip 0.5,
+(env step), nothing leaves HBM.  With ``PPOConfig.symmetrize`` the policy and value are the average
+of the network over the eight board symmetries: K7a (eight views) -> CNN on 8n rows -> K7b (logit
+average) and the mean of the eight values, in acting, evaluation and the update alike.
+Update: K4 GAE, whole-buffer advantage normalisation, clipped surrogate + 0.5*MSE value loss + 0.01*entropy (ppo.py:372-392), grad-norm clip 0.5,
 Adam(eps=1e-5).  With torch.distributed initialised every optimiser step all-reduces the
 gradients in one flat NCCL bucket (dist.py); BatchNorm statistics stay per GPU (the
 single-device reference has nothing to synchronise them with).
@@ -15,13 +17,14 @@ import numpy as np
 import torch
 
 from . import capi, dist
-from .network import BlockBlastNetwork, PPOLossTail, _pack_mask_planes
-from .rollout import RolloutBuffer  # noqa: F401  (re-export, as in the reference module)
+from .network import BlockBlastNetwork, PPOLossTail, SymmetryMean, _pack_mask_planes
+from .rollout import RolloutBuffer, pack_dense_obs  # noqa: F401  (RolloutBuffer: re-export, as in the reference module)
 
 
 @dataclass
 class PPOConfig:
-    """Field names and defaults of the reference (ppo.py:26-46); ``precision`` is ours."""
+    """Field names and defaults of the reference (ppo.py:26-46); ``precision``, ``fused_bn`` and
+    ``symmetrize`` are ours."""
     learning_rate: float = 3e-4
     gamma: float = 0.99
     gae_lambda: float = 0.95
@@ -35,6 +38,7 @@ class PPOConfig:
     fc_hidden: Tuple[int, ...] = (512, 256)
     precision: str = "fp32"          # "fp32" (reference numerics) | "bf16" (autocast, channels_last)
     fused_bn: bool = True            # bf16 only: BatchNorm + ReLU (+ residual add) as bb_bn_relu_* kernels around cuDNN's convs
+    symmetrize: bool = False         # policy / value = average of the network over the 8 board symmetries (K7)
 
     def to_dict(self):
         return {f.name: getattr(self, f.name) for f in fields(self)}
@@ -110,23 +114,50 @@ class PPOAgent:
             planes = _pack_mask_planes(m.to(dev))
         return x, planes
 
+    def _packed(self, obs):
+        """(board int64[N], pieces int32[N], mask planes int64[3,N] or None) of a packed observation, or of
+        the reference's dense arrays packed with rollout.pack_dense_obs."""
+        if isinstance(obs["board"], torch.Tensor) and obs["board"].dtype == torch.int64 and obs["board"].dim() == 1:
+            return obs["board"], obs["pieces"], obs.get("mask")
+        board, pieces = obs["board"], obs["pieces"]
+        n = len(board)
+        mask = obs.get("action_mask")
+        b, p, m = pack_dense_obs(board, pieces, mask if mask is not None else np.zeros((n, 192), np.int8), self.device)
+        return b, p, (m if mask is not None else None)
+
+    def _sym_trunk(self, board, pieces, x_buf=None):
+        """K7a -> CNN on the 8n view rows (one batch, so train-mode BatchNorm sees all views of every state)
+        -> K7b and the mean of the eight values: (f32 logits [n,192], values [n])."""
+        n = board.shape[0]
+        x = x_buf if x_buf is not None else torch.empty((8 * n, 4, 8, 8), dtype=torch.float32, device=self.device)
+        capi.unpack_obs_sym(board, pieces, x, n=n)
+        logits, value = self._trunk(x)
+        return SymmetryMean.apply(logits, pieces), value.view(8, n).mean(0)
+
+    def _policy(self, obs, chunk=None):
+        """(raw logits [N,192], values [N], mask planes int64 [3,N] or None) of an observation; ``chunk``
+        bounds the number of STATES per CNN batch."""
+        if self.config.symmetrize:
+            board, pieces, planes = self._packed(obs)
+            n = board.shape[0]
+            step = n if chunk is None or n <= chunk else chunk
+            parts = [self._sym_trunk(board[s0:s0 + step], pieces[s0:s0 + step]) for s0 in range(0, n, step)]
+        else:
+            x, planes = self._obs_to_nchw(obs)
+            n = x.shape[0]
+            step = n if chunk is None or n <= chunk else chunk
+            parts = [self._trunk(x[s0:s0 + step]) for s0 in range(0, n, step)]
+        if len(parts) == 1:
+            return parts[0][0], parts[0][1], planes
+        return torch.cat([l for l, _ in parts]), torch.cat([v for _, v in parts]), planes
+
     # ------------------------------------------------------------------ acting
     @torch.no_grad()
     def act(self, obs, deterministic=False, chunk=None):
         """Device fast path: returns (actions int32, log_probs, values) as CUDA tensors.
         ``chunk`` bounds the CNN batch (activation memory) for very large env counts; BatchNorm
         in train mode then uses per-chunk statistics."""
-        x, planes = self._obs_to_nchw(obs)
-        n = x.shape[0]
-        if chunk is None or n <= chunk:
-            logits, value = self._trunk(x)
-        else:
-            ls, vs = [], []
-            for s0 in range(0, n, chunk):
-                l, v = self._trunk(x[s0:s0 + chunk])
-                ls.append(l)
-                vs.append(v)
-            logits, value = torch.cat(ls), torch.cat(vs)
+        logits, value, planes = self._policy(obs, chunk)
         act, logp, _ = self.network.head_from_logits(logits, planes, None, deterministic, need_entropy=False)
         return act, logp, value
 
@@ -135,11 +166,14 @@ class PPOAgent:
         """``act`` on a packed observation with caller-owned outputs (rows of a RolloutBuffer):
         K2 -> CNN -> K3 writing ``actions`` int32[N] / ``log_probs`` f32[N] in place, ``values`` f32[N]
         copied.  No allocation of result tensors, no host work besides the launches — the body of a
-        captured rollout graph."""
+        captured rollout graph.  ``x_buf``: f32 [N,4,8,8], or [8N,4,8,8] with ``symmetrize``."""
         n = obs["board"].shape[0]
-        x = x_buf if x_buf is not None else torch.empty((n, 4, 8, 8), dtype=torch.float32, device=self.device)
-        capi.unpack_obs(obs["board"], obs["pieces"], obs["mask"], obs["mask"].stride(0), obs=x, n=n)
-        logits, value = self._trunk(x)
+        if self.config.symmetrize:
+            logits, value = self._sym_trunk(obs["board"], obs["pieces"], x_buf)
+        else:
+            x = x_buf if x_buf is not None else torch.empty((n, 4, 8, 8), dtype=torch.float32, device=self.device)
+            capi.unpack_obs(obs["board"], obs["pieces"], obs["mask"], obs["mask"].stride(0), obs=x, n=n)
+            logits, value = self._trunk(x)
         if logits.dtype not in (torch.float32, torch.bfloat16):
             logits = logits.float()
         net = self.network
@@ -158,31 +192,31 @@ class PPOAgent:
         """ppo.py:261-289 (single observation)."""
         obs = {k: (v.unsqueeze(0) if isinstance(v, torch.Tensor) else np.asarray(v)[None]) for k, v in observation.items()
                if k in ("board", "pieces", "action_mask")}
-        x, planes = self._obs_to_nchw(obs)
         with torch.no_grad():
-            logits, value = self._trunk(x)
+            logits, value, planes = self._policy(obs)
             act, logp, ent = self.network.head_from_logits(logits, planes, None, deterministic)
         return int(act.item()), {"log_prob": float(logp.item()), "entropy": float(ent.item()), "value": float(value.item())}
 
     @torch.no_grad()
     def values(self, obs, chunk=None):
-        x, _ = self._obs_to_nchw({k: v for k, v in obs.items() if k != "action_mask"})
-        if chunk is None or x.shape[0] <= chunk:
-            return self._trunk(x)[1]
-        return torch.cat([self._trunk(x[s0:s0 + chunk])[1] for s0 in range(0, x.shape[0], chunk)])
+        return self._policy({k: v for k, v in obs.items() if k != "action_mask"}, chunk)[1]
 
     def get_values(self, observations):
         """ppo.py:321-328."""
         return self.values(observations).cpu().numpy()
 
     # ------------------------------------------------------------------ update
-    def _fused_step(self, obs, mask, actions, old_logp, adv, ret, sums):
-        """One optimiser step on a gathered minibatch (fused loss tail); metric terms added to ``sums``."""
+    def _fused_step(self, obs, mask, actions, old_logp, adv, ret, sums, pieces=None):
+        """One optimiser step on a gathered minibatch (fused loss tail); metric terms added to ``sums``.
+        ``pieces`` (symmetrize): the minibatch's pieces words, ``obs`` then holds its eight views."""
         cfg = self.config
         if cfg.precision == "bf16":
             obs = obs.contiguous(memory_format=torch.channels_last)
         with self._autocast():
             logits, values = self.network.trunk(obs)
+        if pieces is not None:
+            logits = SymmetryMean.apply(logits, pieces)
+            values = values.float().view(8, -1).mean(0)
         loss, means = PPOLossTail.apply(logits, values.float(), mask, actions, old_logp, adv, ret,
                                         cfg.clip_epsilon, cfg.value_coef, cfg.entropy_coef)
         self.bucket.zero()
@@ -194,22 +228,22 @@ class PPOAgent:
 
     def _minibatch(self, buffer, idx, mean_std, out, sums):
         """gather (bb_gather_minibatch) of samples ``idx``, then one optimiser step on them."""
-        g = buffer.gather(idx, mean_std, out=out)
-        self._fused_step(g["obs"], g["mask"], g["actions"], g["logp"], g["adv"], g["ret"], sums)
+        g = buffer.gather(idx, mean_std, out=out, symmetrize=self.config.symmetrize)
+        self._fused_step(g["obs"], g["mask"], g["actions"], g["logp"], g["adv"], g["ret"], sums, g.get("pieces"))
 
     def _graph_step(self, buffer):
         """The minibatch step as a replayable CUDA graph: gather (bb_gather_minibatch) of the static
         index tensor, CNN forward / backward, loss tail, gradient all-reduce, clip, Adam — ~250
         launches collapse into one graph launch, which is what bounds the reference's own schedule
         (2,048-sample minibatches) on a B200.  Captured once per (buffer, batch size)."""
-        key = (id(buffer), self.config.batch_size)
+        key = (id(buffer), self.config.batch_size, self.config.symmetrize)
         if self._graph is not None and self._graph["key"] == key:
             return self._graph
         dev, b = self.device, self.config.batch_size
         st = {"key": key, "idx": torch.zeros(b, dtype=torch.int64, device=dev),
               "ms": torch.zeros(2, dtype=torch.float32, device=dev),
               "sums": torch.zeros(6, dtype=torch.float64, device=dev)}
-        st["out"] = buffer.gather(st["idx"], st["ms"])
+        st["out"] = buffer.gather(st["idx"], st["ms"], symmetrize=self.config.symmetrize)
         graph = torch.cuda.CUDAGraph()
         with torch.cuda.graph(graph):
             self._minibatch(buffer, st["idx"], st["ms"], st["out"], st["sums"])
@@ -258,16 +292,18 @@ class PPOAgent:
         default of the reference's torch.load call).  The optimizer state is written in the form a
         plain torch.optim.Adam on any device accepts: CPU scalar ``step`` counters, no
         fused / foreach / capturable flags of ours.  ``b200_state`` (ignored by the reference)
-        carries the sampling-noise position for --resume."""
+        carries the sampling-noise position for --resume and ``symmetrize`` (kept out of ``config``, which the
+        reference's PPOConfig(**config) must accept)."""
         cfgd = {k: (list(v) if isinstance(v, tuple) else v) for k, v in self.config.to_dict().items()
-                if k not in ("precision", "fused_bn")}
+                if k not in ("precision", "fused_bn", "symmetrize")}
         opt = self.optimizer.state_dict()
         opt = {"state": {k: {n: (v.detach().cpu().float().reshape(()) if n == "step" and torch.is_tensor(v) else v)
                              for n, v in st.items()} for k, st in opt["state"].items()},
                "param_groups": [{**g, "fused": None, "foreach": None, "capturable": False} for g in opt["param_groups"]]}
         torch.save({"network_state_dict": network_state if network_state is not None else self.network.state_dict(),
                     "optimizer_state_dict": opt, "config": cfgd,
-                    "b200_state": {"sample_calls": self.network.sample_calls, "sample_seed": self.network.sample_seed}},
+                    "b200_state": {"sample_calls": self.network.sample_calls, "sample_seed": self.network.sample_seed,
+                                   "symmetrize": bool(self.config.symmetrize)}},
                    path)
 
     def load(self, path):
@@ -284,6 +320,8 @@ class PPOAgent:
             cfg = {k: (tuple(v) if isinstance(v, list) else v) for k, v in ck["config"].items()}
             self.config = PPOConfig.from_dict({**cfg, "precision": self.config.precision,
                                                "fused_bn": self.config.fused_bn})
+        # the checkpoint's own policy form: symmetrized only when it was trained (or saved) so
+        self.config.symmetrize = bool(ck.get("b200_state", {}).get("symmetrize", False))
         if "b200_state" in ck:
             self.network.sample_calls = ck["b200_state"].get("sample_calls", 0)
         self.bucket.rebind()

@@ -129,22 +129,30 @@ class RolloutBuffer:
         return mean.float(), var.sqrt().float()
 
     # ------------------------------------------------------------------ minibatches
-    def gather(self, idx, mean_std, obs_dtype=torch.float32, out=None):
+    def gather(self, idx, mean_std, obs_dtype=torch.float32, out=None, symmetrize=False):
         """Minibatch ``idx`` (int64 flat sample indices) of the packed buffer in ONE library call
         (bb_gather_minibatch): obs planes (B,4,8,8), mask planes int64 [3,B], actions int32, old
         log-probs, advantages normalised with ``mean_std`` (float32 [2] device tensor), returns.
+        ``symmetrize``: obs holds the eight views (8B,4,8,8) of the samples (bb_unpack_obs_sym through the
+        same index) and ``pieces`` int32 [B] their pieces words.
         ``out``: a dict of preallocated outputs to fill (static buffers of a captured CUDA graph)."""
         b, dev = idx.numel(), self.device
         if out is None:
-            out = dict(obs=torch.empty((b, 4, 8, 8), dtype=obs_dtype, device=dev),
+            out = dict(obs=torch.empty((8 * b if symmetrize else b, 4, 8, 8), dtype=obs_dtype, device=dev),
                        mask=torch.empty((3, b), dtype=torch.int64, device=dev),
                        actions=torch.empty(b, dtype=torch.int32, device=dev),
                        logp=torch.empty(b, dtype=torch.float32, device=dev),
                        adv=torch.empty(b, dtype=torch.float32, device=dev),
                        ret=torch.empty(b, dtype=torch.float32, device=dev))
+            if symmetrize:
+                out["pieces"] = torch.empty(b, dtype=torch.int32, device=dev)
         capi.gather_minibatch(idx, self.num_envs, self.boards, self.pieces, self.action_masks, self.actions,
-                              self.log_probs, self.advantages, self.returns, mean_std, out["obs"], out["mask"],
-                              out["actions"], out["logp"], out["adv"], out["ret"])
+                              self.log_probs, self.advantages, self.returns, mean_std,
+                              None if symmetrize else out["obs"], out["mask"], out["actions"], out["logp"], out["adv"],
+                              out["ret"])
+        if symmetrize:
+            capi.unpack_obs_sym(self.boards, self.pieces, out["obs"], index=idx)
+            torch.index_select(self.pieces.view(-1), 0, idx, out=out["pieces"])
         return out
 
     def get_samples(self, batch_size):

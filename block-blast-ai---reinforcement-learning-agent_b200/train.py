@@ -8,7 +8,7 @@ and checkpoint files, run by one process per GPU.
 Config quirks of the reference are honoured (SURVEY.md §5): ``num_epochs`` is read from the
 ``ppo`` section (both shipped YAMLs put it under ``training``, so the default 10 applies),
 ``batch_size`` from ``training``, the ``network`` / ``environment`` sections are ignored.
-Keys of ours live under ``b200:`` (precision, reseed_on_reset, log_every_update).
+Keys of ours live under ``b200:`` (precision, reseed_on_reset, log_every_update, symmetrize).
 """
 import argparse
 import json
@@ -49,7 +49,8 @@ class RolloutRunner:
     def __init__(self, vec_env, agent, buffer, use_graph=True):
         self.vec_env, self.agent, self.buffer = vec_env, agent, buffer
         n, dev = buffer.num_envs, buffer.device
-        self.x_buf = torch.empty((n, 4, 8, 8), dtype=torch.float32, device=dev)
+        rows = 8 * n if agent.config.symmetrize else n            # symmetrize: the eight views of every env
+        self.x_buf = torch.empty((rows, 4, 8, 8), dtype=torch.float32, device=dev)
         self.last_values = torch.zeros(n, dtype=torch.float32, device=dev)
         self.use_graph, self.graph, self.calls = bool(use_graph), None, 0
 
@@ -120,12 +121,15 @@ def train(config, resume_path=None, seed=42, progress_callback=None, max_updates
         gae_lambda=ppo_c.get("gae_lambda", 0.95), clip_epsilon=ppo_c.get("clip_epsilon", 0.2),
         entropy_coef=ppo_c.get("entropy_coef", 0.01), value_coef=ppo_c.get("value_coef", 0.5),
         max_grad_norm=ppo_c.get("max_grad_norm", 0.5), num_epochs=ppo_c.get("num_epochs", 10),
-        batch_size=tr_c.get("batch_size", 2048), precision=ours.get("precision", "fp32")), device,
+        batch_size=tr_c.get("batch_size", 2048), precision=ours.get("precision", "fp32"),
+        symmetrize=bool(ours.get("symmetrize", False))), device,
         seed=seed, global_env_offset=offset)                  # sampling noise keyed by (seed, GLOBAL env id, call)
     agent.train()                                             # train mode during rollout too (scripts/train.py:122)
     start_step = 0
     if resume_path and os.path.exists(resume_path):
         agent.load(resume_path)
+        if "symmetrize" in ours:                              # the config's policy form wins over the checkpoint's
+            agent.config.symmetrize = bool(ours["symmetrize"])
         try:
             start_step = int(os.path.splitext(os.path.basename(resume_path))[0].split("_")[-1])
         except ValueError:

@@ -243,7 +243,8 @@ int bb_unpack_obs_reference_layout(const uint64_t* board, const uint32_t* pieces
  *   index device i64[batch]; board device u64[T*n_envs]; pieces device u32[T*n_envs];
  *   mask device u64[T][3][n_envs]; action i32, logp / adv / ret f32 [T*n_envs]
  *   adv_mean_std device f32[2] or NULL: adv_out = (adv - mean) / (std + 1e-8) (ppo.py:196)
- *   obs_nchw device [batch,4,8,8] of obs_dtype; mask_out device u64[3][batch];
+ *   obs_nchw device [batch,4,8,8] of obs_dtype, or NULL to gather everything but the observation
+ *            planes (obs_dtype is then ignored); mask_out device u64[3][batch];
  *   action_out i32, logp_out / adv_out / ret_out f32 [batch] */
 int bb_gather_minibatch(const int64_t* index, int64_t batch, int64_t n_envs, const uint64_t* board,
                         const uint32_t* pieces, const uint64_t* mask, const int32_t* action,
@@ -251,6 +252,26 @@ int bb_gather_minibatch(const int64_t* index, int64_t batch, int64_t n_envs, con
                         const float* adv_mean_std, void* obs_nchw, int obs_dtype, uint64_t* mask_out,
                         int32_t* action_out, float* logp_out, float* adv_out, float* ret_out,
                         void* stream);
+
+/* Board symmetries (group D4, ids and maps in csrc/bb_rules.cuh): the symmetric policy evaluates
+ * the network on the eight views of each state and averages over them.
+ * bb_unpack_obs_sym: the observation planes of bb_unpack_obs for all eight views, view-major:
+ *   row g*n + i of obs_nchw device [8n,4,8,8] of obs_dtype (BB_F32 / BB_BF16) is view g of input
+ *   row index[i] (index device i64[n], or NULL for row i) of board device u64[], pieces device u32[].
+ * bb_sym_logits_mean: out device f32[n,192],
+ *   out[i, s*64 + a] = 0.125 * sum_{g=0..7} logits[g*n + i, s*64 + sigma_{g,p_s}(a)]
+ *   (f32 sum in g order) where a is an in-bounds anchor of the piece p_s < 37 of slot s of
+ *   pieces[i] (device u32[n]), 0 elsewhere.  logits device [8n,192] of logits_dtype, raw, 16-byte
+ *   aligned (read as 16-byte vectors; an unaligned pointer is rejected with code -1).
+ * bb_sym_logits_mean_backward: the transposed map, grad_logits device [8n,192] of logits_dtype:
+ *   0.125 * grad_out[i, s*64 + a] at the view position of every such (s, a), 0 elsewhere;
+ *   grad_logits 16-byte aligned like logits. */
+int bb_unpack_obs_sym(const uint64_t* board, const uint32_t* pieces, const int64_t* index, void* obs_nchw,
+                      int obs_dtype, int64_t n, void* stream);
+int bb_sym_logits_mean(const void* logits, int logits_dtype, const uint32_t* pieces, float* out, int64_t n,
+                       void* stream);
+int bb_sym_logits_mean_backward(const float* grad_out, const uint32_t* pieces, void* grad_logits,
+                                int logits_dtype, int64_t n, void* stream);
 
 /* Masked categorical head (BlockBlastNetwork.forward masking + get_action_and_value +
  * _masked_entropy, src/models/network.py:172-262) fused in one kernel.
