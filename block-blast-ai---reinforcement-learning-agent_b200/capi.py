@@ -80,6 +80,9 @@ def lib():
     L.bb_unpack_obs_sym.argtypes = [vp, vp, vp, vp, C.c_int, i64, vp]
     L.bb_sym_logits_mean.argtypes = [vp, C.c_int, vp, vp, i64, vp]
     L.bb_sym_logits_mean_backward.argtypes = [vp, vp, vp, C.c_int, i64, vp]
+    L.bb_sym_canonical.argtypes = [vp, vp, vp, vp, vp, vp, i64, vp]
+    L.bb_sym_logits_canonical.argtypes = [vp, C.c_int, vp, vp, vp, i64, vp]
+    L.bb_sym_logits_canonical_backward.argtypes = [vp, vp, vp, vp, C.c_int, i64, vp]
     L.bb_masked_sample.argtypes = [vp, C.c_int, vp, i64, u64, u64, C.c_int, vp, vp, vp, i64, i64, vp, vp]
     L.bb_masked_head_backward.argtypes = [vp, C.c_int, vp, i64, vp, vp, vp, vp, i64, vp]
     L.bb_ppo_loss.argtypes = [vp, C.c_int, vp, i64, vp, vp, vp, vp, vp, C.c_double, C.c_double, C.c_double, vp, vp, vp, i64, vp]
@@ -340,6 +343,37 @@ def sym_logits_mean_backward(grad_out, pieces, grad_logits):
     assert grad_out.is_contiguous() and grad_out.dtype == torch.float32 and grad_logits.shape == (8 * n, 192)
     dt = BB_BF16 if grad_logits.dtype == torch.bfloat16 else BB_F32
     check(lib().bb_sym_logits_mean_backward(ptr(grad_out), ptr(pieces), ptr(grad_logits), dt, n, current_stream()))
+
+
+def sym_canonical(board, pieces, board_out, pieces_out, views_out, index=None, n=None):
+    """K7c (bb_sym_canonical): canonical view board_out int64 [n] / pieces_out int32 [n] and view set views_out
+    uint8 [n] of packed row i (or index[i])."""
+    n = int((index.numel() if index is not None else board.numel()) if n is None else n)
+    assert board_out.numel() >= n and pieces_out.numel() >= n and views_out.numel() >= n
+    check(lib().bb_sym_canonical(ptr(board), ptr(pieces), ptr(index), ptr(board_out), ptr(pieces_out), ptr(views_out), n,
+                                 current_stream()))
+
+
+def sym_logits_canonical(logits, pieces, views, out):
+    """K7c forward (bb_sym_logits_canonical): canonical-row logits [n,192] f32 / bf16, the states' own pieces int32
+    [n] and view sets uint8 [n] -> out f32 [n,192] in the states' frames."""
+    import torch
+    n = pieces.numel()
+    assert logits.is_contiguous() and logits.shape == (n, 192) and out.dtype == torch.float32 and out.is_contiguous()
+    assert views.numel() == n and views.dtype == torch.uint8
+    dt = BB_BF16 if logits.dtype == torch.bfloat16 else BB_F32
+    check(lib().bb_sym_logits_canonical(ptr(logits), dt, ptr(pieces), ptr(views), ptr(out), n, current_stream()))
+
+
+def sym_logits_canonical_backward(grad_out, pieces, views, grad_logits):
+    """K7c backward (bb_sym_logits_canonical_backward): grad_out f32 [n,192] -> grad_logits [n,192] f32 / bf16."""
+    import torch
+    n = pieces.numel()
+    assert grad_out.is_contiguous() and grad_out.dtype == torch.float32 and grad_logits.shape == (n, 192)
+    assert views.numel() == n and views.dtype == torch.uint8
+    dt = BB_BF16 if grad_logits.dtype == torch.bfloat16 else BB_F32
+    check(lib().bb_sym_logits_canonical_backward(ptr(grad_out), ptr(pieces), ptr(views), ptr(grad_logits), dt, n,
+                                                 current_stream()))
 
 
 def gather_minibatch(index, n_envs, board, pieces, mask, action, logp, adv, ret, adv_mean_std, obs, mask_out,

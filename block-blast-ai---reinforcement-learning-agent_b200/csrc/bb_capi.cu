@@ -514,6 +514,43 @@ int bb_sym_logits_mean_backward(const float* grad_out, const uint32_t* pieces, v
     return 0;
 }
 
+int bb_sym_canonical(const uint64_t* board, const uint32_t* pieces, const int64_t* index, uint64_t* board_out,
+                     uint32_t* pieces_out, uint8_t* views_out, int64_t n, void* stream) {
+    if (n < 0) return fail(-1, "bb_sym_canonical: negative n");
+    if (n == 0) return 0;
+    if (!board || !pieces || !board_out || !pieces_out || !views_out) return fail(-1, "bb_sym_canonical: NULL array");
+    BB_CUDA(bb_launch_sym_canonical(board, pieces, index, board_out, pieces_out, views_out, n, (cudaStream_t)stream),
+            "bb_sym_canonical launch");
+    return 0;
+}
+
+int bb_sym_logits_canonical(const void* logits, int logits_dtype, const uint32_t* pieces, const uint8_t* views, float* out,
+                            int64_t n, void* stream) {
+    if (n < 0) return fail(-1, "bb_sym_logits_canonical: negative n");
+    if (logits_dtype != BB_F32 && logits_dtype != BB_BF16)
+        return fail(-1, "bb_sym_logits_canonical: logits_dtype must be BB_F32 or BB_BF16");
+    if (n == 0) return 0;
+    if (!logits || !pieces || !views || !out) return fail(-1, "bb_sym_logits_canonical: NULL array");
+    if ((uintptr_t)logits & 15) return fail(-1, "bb_sym_logits_canonical: logits must be 16-byte aligned");
+    BB_CUDA(bb_launch_sym_logits_canonical(logits, logits_dtype, pieces, views, out, n, (cudaStream_t)stream),
+            "bb_sym_logits_canonical launch");
+    return 0;
+}
+
+int bb_sym_logits_canonical_backward(const float* grad_out, const uint32_t* pieces, const uint8_t* views, void* grad_logits,
+                                     int logits_dtype, int64_t n, void* stream) {
+    if (n < 0) return fail(-1, "bb_sym_logits_canonical_backward: negative n");
+    if (logits_dtype != BB_F32 && logits_dtype != BB_BF16)
+        return fail(-1, "bb_sym_logits_canonical_backward: logits_dtype must be BB_F32 or BB_BF16");
+    if (n == 0) return 0;
+    if (!grad_out || !pieces || !views || !grad_logits) return fail(-1, "bb_sym_logits_canonical_backward: NULL array");
+    if (((uintptr_t)grad_out | (uintptr_t)grad_logits) & 15)
+        return fail(-1, "bb_sym_logits_canonical_backward: grad_out and grad_logits must be 16-byte aligned");
+    BB_CUDA(bb_launch_sym_logits_canonical_bwd(grad_out, pieces, views, grad_logits, logits_dtype, n, (cudaStream_t)stream),
+            "bb_sym_logits_canonical_backward launch");
+    return 0;
+}
+
 int bb_masked_sample(const void* logits, int logits_dtype, const uint64_t* mask, int64_t mask_stride,
                      uint64_t seed, uint64_t call_counter, int mode, int32_t* action, float* logp,
                      float* entropy, int64_t n, int64_t row_offset, const uint64_t* call_counter_dev, void* stream) {

@@ -68,6 +68,14 @@ cudaError_t bb_launch_sym_logits_mean(const void* logits, int dtype, const uint3
                                       cudaStream_t stream);
 cudaError_t bb_launch_sym_logits_mean_bwd(const float* dout, const uint32_t* pieces, void* dlogits, int dtype, int64_t n,
                                           cudaStream_t stream);
+// K7c (canonical view of each row and its view set; index: optional row gather) and the map of the canonical
+// row's logits into the state's own frame, with its transpose
+cudaError_t bb_launch_sym_canonical(const uint64_t* board, const uint32_t* pieces, const int64_t* index, uint64_t* cboard,
+                                    uint32_t* cpieces, uint8_t* views, int64_t n, cudaStream_t stream);
+cudaError_t bb_launch_sym_logits_canonical(const void* logits, int dtype, const uint32_t* pieces, const uint8_t* views,
+                                           float* out, int64_t n, cudaStream_t stream);
+cudaError_t bb_launch_sym_logits_canonical_bwd(const float* dout, const uint32_t* pieces, const uint8_t* views, void* dlogits,
+                                               int dtype, int64_t n, cudaStream_t stream);
 cudaError_t bb_launch_masked_sample(const void* logits, int logits_dtype, const uint64_t* mask,
                                     int64_t mask_stride, uint64_t seed, uint64_t call_counter, int mode,
                                     int32_t* action, float* logp, float* entropy, int64_t n, cudaStream_t stream,

@@ -817,3 +817,179 @@ cudaError_t bb_launch_sym_logits_mean_bwd(const float* dout, const uint32_t* pie
     else bb_sym_logits_mean_bwd_kernel<false><<<k7b_grid(n), BB_K7B_THREADS, 0, stream>>>(dout, pieces, dlogits, n);
     return cudaGetLastError();
 }
+
+// ------------------------------------------------------------------------------------ K7c
+// Canonical frame: the network runs once per state, on the canonical view c(s) (bb_sym_canonical,
+// bb_rules.cuh), and its logits are mapped back into the state's own frame.  With M(s) the view set
+// (bit g set iff view g of s is c(s)):
+//   out[i, s*64 + a] = (1/|M|) * sum_{g in M, ascending} L[i, s*64 + sigma_{g,p_s}(a)]      (f32)
+// for an in-bounds anchor a of the slot's piece p_s (< 37) of the state's OWN pieces word, 0 elsewhere: the
+// positions and zeros of K7b, restricted to the views that equal c(s).  1/|M| is a power of two.
+// bb_sym_canonical_kernel: one thread per state, 12 B read (+ 8 B of index), 13 B written; the canonical
+// rows then go through the unchanged K2.
+__global__ void __launch_bounds__(256)
+bb_sym_canonical_kernel(const uint64_t* __restrict__ board, const uint32_t* __restrict__ pieces,
+                        const int64_t* __restrict__ index, uint64_t* __restrict__ cboard, uint32_t* __restrict__ cpieces,
+                        uint8_t* __restrict__ views, int64_t n) {
+    __shared__ BBSymTables S;                                   // only perm is read (bb_sym_pieces)
+    for (int k = threadIdx.x; k < BB_SYM_N * BB_TABLE_N; k += blockDim.x) S.perm[k / BB_TABLE_N][k % BB_TABLE_N] = g_bb_sym.perm[k / BB_TABLE_N][k % BB_TABLE_N];
+    __syncthreads();
+    for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x) {
+        const int64_t r = index ? __ldg(index + i) : i;
+        uint64_t cb;
+        uint32_t cp;
+        views[i] = (uint8_t)bb_sym_canonical(&S, __ldg(board + r), __ldg(pieces + r), &cb, &cp);
+        cboard[i] = cb;
+        cpieces[i] = cp;
+    }
+}
+
+// K7b's 16-byte staging of a logit row (f32 or bf16 in HBM <-> f32 in shared memory).  The K7b kernels keep
+// their inline copies, which compile to the same instructions as before this section was added.
+template <bool BF16>
+__device__ __forceinline__ void k7c_stage(const void* __restrict__ logits, int64_t row, int q, float4* dst) {
+    if (BF16) {
+        const uint4 h = __ldcs(reinterpret_cast<const uint4*>(logits) + row * 24 + q);
+        dst[2 * q] = make_float4(__uint_as_float(h.x << 16), __uint_as_float(h.x & 0xFFFF0000u),
+                                 __uint_as_float(h.y << 16), __uint_as_float(h.y & 0xFFFF0000u));
+        dst[2 * q + 1] = make_float4(__uint_as_float(h.z << 16), __uint_as_float(h.z & 0xFFFF0000u),
+                                     __uint_as_float(h.w << 16), __uint_as_float(h.w & 0xFFFF0000u));
+    } else {
+        dst[q] = __ldcs(reinterpret_cast<const float4*>(logits) + row * 48 + q);
+    }
+}
+template <bool BF16>
+__device__ __forceinline__ void k7c_unstage(void* __restrict__ dlogits, int64_t row, int q, const float4* src) {
+    if (BF16) {
+        const float4 a = src[2 * q], b = src[2 * q + 1];
+        const __nv_bfloat162 h0 = __floats2bfloat162_rn(a.x, a.y), h1 = __floats2bfloat162_rn(a.z, a.w);
+        const __nv_bfloat162 h2 = __floats2bfloat162_rn(b.x, b.y), h3 = __floats2bfloat162_rn(b.z, b.w);
+        uint4 w;
+        w.x = *reinterpret_cast<const uint32_t*>(&h0); w.y = *reinterpret_cast<const uint32_t*>(&h1);
+        w.z = *reinterpret_cast<const uint32_t*>(&h2); w.w = *reinterpret_cast<const uint32_t*>(&h3);
+        __stcs(reinterpret_cast<uint4*>(dlogits) + row * 24 + q, w);
+    } else {
+        __stcs(reinterpret_cast<float4*>(dlogits) + row * 48 + q, src[q]);
+    }
+}
+
+// 1/|M| (exact: |M| is 1, 2, 4 or 8); an empty view set gives 0
+__device__ __forceinline__ float k7c_scale(uint32_t views) {
+    const int c = __popc(views);
+    return c ? 1.f / (float)c : 0.f;
+}
+
+#define BB_K7C_STATES 16
+
+// Forward: a block stages the logit rows of BB_K7C_STATES states (one row each, contiguous) and gathers
+// from them.  Per state: 768 B (f32) or 384 B (bf16) of logits, 4 B pieces, 1 B views, 768 B of f32 out.
+template <bool BF16>
+__global__ void __launch_bounds__(BB_K7B_THREADS)
+bb_sym_logits_canonical_kernel(const void* __restrict__ logits, const uint32_t* __restrict__ pieces,
+                               const uint8_t* __restrict__ views, float* __restrict__ out, int64_t n) {
+    __shared__ float4 tile[BB_K7C_STATES * 48];
+    __shared__ uint8_t shift[BB_SYM_N * BB_TABLE_N];
+    __shared__ uint64_t inb[BB_TABLE_N];
+    k7b_load_tables(shift, inb);
+    const float* tf = reinterpret_cast<const float*>(tile);
+    constexpr int PER_ROW = BF16 ? 24 : 48;
+    for (int64_t i0 = (int64_t)blockIdx.x * BB_K7C_STATES; i0 < n; i0 += (int64_t)gridDim.x * BB_K7C_STATES) {
+        const int ns = (int)(n - i0 < BB_K7C_STATES ? n - i0 : BB_K7C_STATES);
+        for (int u = threadIdx.x; u < ns * PER_ROW; u += blockDim.x) {
+            const int st = u / PER_ROW;
+            k7c_stage<BF16>(logits, i0 + st, u - st * PER_ROW, tile + st * 48);
+        }
+        __syncthreads();
+        for (int v = threadIdx.x; v < ns * 192; v += blockDim.x) {
+            const int st = v / 192, j = v - st * 192;
+            const int id = k7b_piece(inb, __ldg(pieces + i0 + st), j);
+            const uint32_t vm = __ldg(views + i0 + st);
+            float sum = 0.f;
+            if (id >= 0) {
+#pragma unroll
+                for (int g = 0; g < BB_SYM_N; ++g)
+                    if ((vm >> g) & 1u) sum += tf[st * 192 + k7b_pos(shift, id, j, g)];
+            }
+            out[(i0 + st) * 192 + j] = k7c_scale(vm) * sum;    // read by K3 / the loss tail next: keep in L2
+        }
+        __syncthreads();
+    }
+}
+
+// Backward: the transposed map as a gather, so that a canonical position that several (g, j) pairs reach
+// (|M| > 1: a stabiliser element maps the state onto itself) sums its terms in ascending g, the same order
+// in every run.  Position k = s*64 + b of the canonical row is reached from view g in M exactly when b is an
+// in-bounds anchor of the canonical slot's piece q = PERM[g][p_s] (the same for every g in M), from
+// a = T_{g^-1}(b + SHIFT[g][p_s]) (sigma_{g,p} is a bijection of in-bounds anchors); elsewhere it is 0.
+template <bool BF16>
+__global__ void __launch_bounds__(BB_K7B_THREADS)
+bb_sym_logits_canonical_bwd_kernel(const float* __restrict__ dout, const uint32_t* __restrict__ pieces,
+                                   const uint8_t* __restrict__ views, void* __restrict__ dlogits, int64_t n) {
+    __shared__ float4 din[BB_K7C_STATES * 48];                  // grad_out rows
+    __shared__ float4 dst[BB_K7C_STATES * 48];                  // grad_logits rows
+    __shared__ uint8_t shift[BB_SYM_N * BB_TABLE_N];
+    __shared__ uint8_t perm[BB_SYM_N * BB_TABLE_N];
+    __shared__ uint64_t inb[BB_TABLE_N];
+    k7b_load_tables(shift, inb);
+    for (int k = threadIdx.x; k < BB_SYM_N * BB_TABLE_N; k += blockDim.x) perm[k] = g_bb_sym.perm[k / BB_TABLE_N][k % BB_TABLE_N];
+    const float* fin = reinterpret_cast<const float*>(din);
+    float* fdst = reinterpret_cast<float*>(dst);
+    constexpr int PER_ROW = BF16 ? 24 : 48;
+    for (int64_t i0 = (int64_t)blockIdx.x * BB_K7C_STATES; i0 < n; i0 += (int64_t)gridDim.x * BB_K7C_STATES) {
+        const int ns = (int)(n - i0 < BB_K7C_STATES ? n - i0 : BB_K7C_STATES);
+        for (int u = threadIdx.x; u < ns * 48; u += blockDim.x) din[u] = __ldcs(reinterpret_cast<const float4*>(dout) + i0 * 48 + u);
+        __syncthreads();
+        for (int v = threadIdx.x; v < ns * 192; v += blockDim.x) {
+            const int st = v / 192, k = v - st * 192;
+            const uint32_t pw = __ldg(pieces + i0 + st), vm = __ldg(views + i0 + st);
+            const uint32_t p = (pw >> (8 * (k >> 6))) & 0xFFu;
+            const int b = k & 63;
+            float sum = 0.f;
+            if (p < BB_NUM_PIECES && vm && ((inb[perm[(__ffs(vm) - 1) * BB_TABLE_N + p]] >> b) & 1ull)) {
+#pragma unroll
+                for (int g = 0; g < BB_SYM_N; ++g)
+                    if ((vm >> g) & 1u)
+                        sum += fin[st * 192 + (k & ~63) + bb_sym_cell(bb_sym_inverse(g), b + (int)shift[g * BB_TABLE_N + p])];
+            }
+            fdst[v] = k7c_scale(vm) * sum;
+        }
+        __syncthreads();
+        for (int u = threadIdx.x; u < ns * PER_ROW; u += blockDim.x) {
+            const int st = u / PER_ROW;
+            k7c_unstage<BF16>(dlogits, i0 + st, u - st * PER_ROW, dst + st * 48);
+        }
+        __syncthreads();
+    }
+}
+
+static unsigned k7c_grid(int64_t n, int per_block) {
+    const int64_t want = (n + per_block - 1) / per_block;
+    return (unsigned)(want < 148 * 8 ? want : 148 * 8);        // grid-stride: one wave of 8 blocks per SM
+}
+
+cudaError_t bb_launch_sym_canonical(const uint64_t* board, const uint32_t* pieces, const int64_t* index, uint64_t* cboard,
+                                    uint32_t* cpieces, uint8_t* views, int64_t n, cudaStream_t stream) {
+    if (n <= 0) return cudaSuccess;
+    const int64_t blocks = (n + 255) / 256;
+    bb_sym_canonical_kernel<<<(unsigned)(blocks < 148 * 16 ? blocks : 148 * 16), 256, 0, stream>>>(board, pieces, index, cboard,
+                                                                                                  cpieces, views, n);
+    return cudaGetLastError();
+}
+
+cudaError_t bb_launch_sym_logits_canonical(const void* logits, int dtype, const uint32_t* pieces, const uint8_t* views,
+                                           float* out, int64_t n, cudaStream_t stream) {
+    if (n <= 0) return cudaSuccess;
+    const unsigned grid = k7c_grid(n, BB_K7C_STATES);
+    if (dtype == 1) bb_sym_logits_canonical_kernel<true><<<grid, BB_K7B_THREADS, 0, stream>>>(logits, pieces, views, out, n);
+    else bb_sym_logits_canonical_kernel<false><<<grid, BB_K7B_THREADS, 0, stream>>>(logits, pieces, views, out, n);
+    return cudaGetLastError();
+}
+
+cudaError_t bb_launch_sym_logits_canonical_bwd(const float* dout, const uint32_t* pieces, const uint8_t* views, void* dlogits,
+                                               int dtype, int64_t n, cudaStream_t stream) {
+    if (n <= 0) return cudaSuccess;
+    const unsigned grid = k7c_grid(n, BB_K7C_STATES);
+    if (dtype == 1) bb_sym_logits_canonical_bwd_kernel<true><<<grid, BB_K7B_THREADS, 0, stream>>>(dout, pieces, views, dlogits, n);
+    else bb_sym_logits_canonical_bwd_kernel<false><<<grid, BB_K7B_THREADS, 0, stream>>>(dout, pieces, views, dlogits, n);
+    return cudaGetLastError();
+}

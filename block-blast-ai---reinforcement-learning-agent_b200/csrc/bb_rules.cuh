@@ -954,3 +954,23 @@ BB_HD int bb_sym_anchor(const BBSymTables* S, int g, uint32_t id, int a) {
 BB_HD uint64_t bb_sym_mask_plane(const BBSymTables* S, int g, uint32_t id, uint64_t plane) {
     return bb_sym_board(g, plane) >> S->shift[g][id];
 }
+// the inverse of symmetry g (the two quarter turns swap, every other element is an involution)
+BB_HD int bb_sym_inverse(int g) { return g == 1 ? 3 : g == 3 ? 1 : g; }
+// Canonical representative of the orbit of (board b, pieces word pw): the view g with the smallest key
+// (bb_sym_board(g, b) as u64, then bb_sym_pieces(g, pw) as u32; the full word, used bits and ids of used
+// slots included).  Writes the view to *cb / *cp and returns the view set: bit g set iff view g equals it
+// (never 0; its size is the order of the state's stabiliser).
+BB_HD uint32_t bb_sym_canonical(const BBSymTables* S, uint64_t b, uint32_t pw, uint64_t* cb, uint32_t* cp) {
+    uint64_t kb = b;
+    uint32_t kp = pw, views = 1u;
+#pragma unroll
+    for (int g = 1; g < BB_SYM_N; ++g) {
+        const uint64_t tb = bb_sym_board(g, b);
+        const uint32_t tp = bb_sym_pieces(S, g, pw);
+        if (tb < kb || (tb == kb && tp < kp)) { kb = tb; kp = tp; views = 1u << g; }
+        else if (tb == kb && tp == kp) views |= 1u << g;
+    }
+    *cb = kb;
+    *cp = kp;
+    return views;
+}

@@ -13,8 +13,9 @@ sampled trios from the look-ahead stream, never the env's own), the successors a
 head, and each env plays the move with the highest mean ``reward + gamma * (1 - terminated) * V``.
 
 ``--symmetrize`` evaluates the agent's policy and value as averages over the eight board symmetries
-(``PPOConfig.symmetrize``) even when the checkpoint was trained without them; by default the checkpoint's
-own setting applies.
+(``PPOConfig.symmetrize``) even when the checkpoint was trained without them; ``--canonical-frame`` evaluates
+them on the canonical view of each state instead (``PPOConfig.canonical_frame``, one network row per state).
+By default the checkpoint's own setting applies.
 """
 import argparse
 import json
@@ -50,14 +51,18 @@ def lookahead_actions(agent, h, n, call_counter, samples, chunk=65536):
 
 @torch.no_grad()
 def evaluate(agent, num_episodes=100, seed=0, deterministic=True, max_steps=10000, reward_config=None,
-             return_actions=False, lookahead=0, symmetrize=None):
+             return_actions=False, lookahead=0, symmetrize=None, canonical_frame=None):
     """``lookahead``: 0 = the agent's own policy (argmax when ``deterministic``); K >= 1 = one-ply value
     look-ahead with K sampled trios per dealing move (``lookahead_actions``, expansion call counter = the
     step number).  ``return_actions``: also return ``actions`` int32 [steps, n] (the action every env was given at every
     step; entries after an env's game over are ignored by the env) and ``rewards_per_episode`` — enough to
     replay every episode through another implementation of the rules (tests do, through the oracle).
     ``symmetrize``: None = the agent's own setting; True / False = with / without the eight-view average for
-    this evaluation (the successor values of ``lookahead`` included)."""
+    this evaluation (the successor values of ``lookahead`` included).  ``canonical_frame``: the same for the
+    canonical-frame policy.  Turning one of the two on turns the other off for this evaluation; the agent's
+    own settings are restored afterwards."""
+    if symmetrize and canonical_frame:
+        raise ValueError("evaluate: symmetrize and canonical_frame are mutually exclusive")
     dev = agent.device
     n = int(num_episodes)
     h = capi.EnvHandle(n, seed, 0, reward_config, capi.ENV_NO_AUTO_RESET)
@@ -68,9 +73,15 @@ def evaluate(agent, num_episodes=100, seed=0, deterministic=True, max_steps=1000
     term = torch.zeros(n, dtype=torch.uint8, device=dev)
     total_reward = torch.zeros(n, dtype=torch.float64, device=dev)
     done = torch.zeros(n, dtype=torch.bool, device=dev)
-    was_training, was_sym = agent.training, agent.config.symmetrize
+    was_training, was_sym, was_canon = agent.training, agent.config.symmetrize, agent.config.canonical_frame
     if symmetrize is not None:
         agent.config.symmetrize = bool(symmetrize)
+        if symmetrize:
+            agent.config.canonical_frame = False
+    if canonical_frame is not None:
+        agent.config.canonical_frame = bool(canonical_frame)
+        if canonical_frame:
+            agent.config.symmetrize = False
     agent.eval()                                       # scripts/evaluate.py evaluates in eval mode
     steps = 0
     log = []
@@ -91,7 +102,7 @@ def evaluate(agent, num_episodes=100, seed=0, deterministic=True, max_steps=1000
     finally:
         # the caller's agent keeps its own policy form and mode whatever happens during the evaluation
         h.close()
-        agent.config.symmetrize = was_sym
+        agent.config.symmetrize, agent.config.canonical_frame = was_sym, was_canon
         if was_training:
             agent.train()
     scores, lengths = st["score"].astype(np.int64), st["moves"].astype(np.int64)
@@ -117,11 +128,14 @@ def main():
                     help="K >= 1: one-ply value look-ahead with K sampled trios per dealing move (0 = policy argmax)")
     ap.add_argument("--symmetrize", action="store_true", default=None,
                     help="average the policy / value over the 8 board symmetries (default: the checkpoint's setting)")
+    ap.add_argument("--canonical-frame", action="store_true", default=None,
+                    help="evaluate the network on the canonical view of each state, mapped back (default: the "
+                         "checkpoint's setting)")
     a = ap.parse_args()
     agent = PPOAgent()
     agent.load(a.checkpoint)
     res = evaluate(agent, a.episodes, a.seed, deterministic=not a.stochastic, lookahead=a.lookahead,
-                   symmetrize=a.symmetrize)
+                   symmetrize=a.symmetrize, canonical_frame=a.canonical_frame)
     print(json.dumps({k: v for k, v in res.items() if not isinstance(v, np.ndarray)}, indent=1))
 
 

@@ -197,6 +197,32 @@ class SymmetryMean(torch.autograd.Function):
         return grad, None
 
 
+class CanonicalFrame(torch.autograd.Function):
+    """The canonical-frame policy's logit map (K7c, bb_sym_logits_canonical): raw logits [n,192] of the
+    canonical views (bb_sym_canonical), the states' own pieces words int32 [n] and view sets uint8 [n] -> f32
+    [n,192] logits in the states' own frames, 0 at positions that are always masked.  The backward pass is
+    the kernel's transposed map, in the logits' dtype."""
+
+    @staticmethod
+    def forward(ctx, logits, pieces, views):
+        lg = logits.detach()
+        if lg.dtype not in (torch.float32, torch.bfloat16):
+            lg = lg.float()
+        lg = lg.contiguous()
+        out = torch.empty((pieces.numel(), 192), dtype=torch.float32, device=lg.device)
+        capi.sym_logits_canonical(lg, pieces, views, out)
+        ctx.save_for_backward(pieces, views)
+        ctx.dtype = lg.dtype
+        return out
+
+    @staticmethod
+    def backward(ctx, g):
+        pieces, views = ctx.saved_tensors
+        grad = torch.empty((pieces.numel(), 192), dtype=ctx.dtype, device=g.device)
+        capi.sym_logits_canonical_backward(g.float().contiguous(), pieces, views, grad)
+        return grad, None, None
+
+
 class BlockBlastNetwork(nn.Module):
     def __init__(self, board_size=8, num_pieces=3, conv_channels=(64, 128, 128), fc_hidden=(512, 256),
                  action_space_size=192, use_residual=True, use_batch_norm=True):

@@ -5,6 +5,8 @@ Collect: packed obs -> K2 (planes) -> CNN (PyTorch) -> K3 (masked sample + log-p
 (env step), nothing leaves HBM.  With ``PPOConfig.symmetrize`` the policy and value are the average
 of the network over the eight board symmetries: K7a (eight views) -> CNN on 8n rows -> K7b (logit
 average) and the mean of the eight values, in acting, evaluation and the update alike.
+``PPOConfig.canonical_frame`` gives the same exact symmetry at the price of one network row per state:
+K7c (canonical view of each state) -> K2 -> CNN on n rows -> K7c logit map back into each state's frame.
 Update: K4 GAE, whole-buffer advantage normalisation, clipped surrogate + 0.5*MSE value loss + 0.01*entropy (ppo.py:372-392), grad-norm clip 0.5,
 Adam(eps=1e-5).  With torch.distributed initialised every optimiser step all-reduces the
 gradients in one flat NCCL bucket (dist.py); BatchNorm statistics stay per GPU (the
@@ -17,14 +19,14 @@ import numpy as np
 import torch
 
 from . import capi, dist
-from .network import BlockBlastNetwork, PPOLossTail, SymmetryMean, _pack_mask_planes
+from .network import BlockBlastNetwork, CanonicalFrame, PPOLossTail, SymmetryMean, _pack_mask_planes
 from .rollout import RolloutBuffer, pack_dense_obs  # noqa: F401  (RolloutBuffer: re-export, as in the reference module)
 
 
 @dataclass
 class PPOConfig:
-    """Field names and defaults of the reference (ppo.py:26-46); ``precision``, ``fused_bn`` and
-    ``symmetrize`` are ours."""
+    """Field names and defaults of the reference (ppo.py:26-46); ``precision``, ``fused_bn``, ``symmetrize``
+    and ``canonical_frame`` are ours."""
     learning_rate: float = 3e-4
     gamma: float = 0.99
     gae_lambda: float = 0.95
@@ -39,6 +41,10 @@ class PPOConfig:
     precision: str = "fp32"          # "fp32" (reference numerics) | "bf16" (autocast, channels_last)
     fused_bn: bool = True            # bf16 only: BatchNorm + ReLU (+ residual add) as bb_bn_relu_* kernels around cuDNN's convs
     symmetrize: bool = False         # policy / value = average of the network over the 8 board symmetries (K7)
+    canonical_frame: bool = False    # policy / value = the network on the canonical view, mapped back (K7c)
+
+    def __post_init__(self):
+        check_policy_form(self)
 
     def to_dict(self):
         return {f.name: getattr(self, f.name) for f in fields(self)}
@@ -47,6 +53,12 @@ class PPOConfig:
     def from_dict(cls, data):
         names = {f.name for f in fields(cls)}
         return cls(**{k: v for k, v in data.items() if k in names})
+
+
+def check_policy_form(cfg):
+    """``symmetrize`` and ``canonical_frame`` are two different symmetric policies; a config selects one."""
+    if cfg.symmetrize and cfg.canonical_frame:
+        raise ValueError("PPOConfig: symmetrize and canonical_frame are mutually exclusive")
 
 
 class PPOAgent:
@@ -134,14 +146,30 @@ class PPOAgent:
         logits, value = self._trunk(x)
         return SymmetryMean.apply(logits, pieces), value.view(8, n).mean(0)
 
+    def _canon_trunk(self, board, pieces, x_buf=None, canon=None):
+        """K7c canonical views -> K2 -> CNN on n rows -> K7c logit map: (f32 logits [n,192] in the states' own
+        frames, values [n]).  ``canon``: (board int64 [n], pieces int32 [n], views uint8 [n]) scratch."""
+        n, dev = board.shape[0], self.device
+        if canon is None:
+            canon = (torch.empty(n, dtype=torch.int64, device=dev), torch.empty(n, dtype=torch.int32, device=dev),
+                     torch.empty(n, dtype=torch.uint8, device=dev))
+        cb, cp, views = canon
+        capi.sym_canonical(board, pieces, cb, cp, views, n=n)
+        x = x_buf if x_buf is not None else torch.empty((n, 4, 8, 8), dtype=torch.float32, device=dev)
+        capi.unpack_obs(cb, cp, None, n, obs=x, n=n)
+        logits, value = self._trunk(x)
+        return CanonicalFrame.apply(logits, pieces, views), value
+
     def _policy(self, obs, chunk=None):
         """(raw logits [N,192], values [N], mask planes int64 [3,N] or None) of an observation; ``chunk``
         bounds the number of STATES per CNN batch."""
-        if self.config.symmetrize:
+        check_policy_form(self.config)
+        if self.config.symmetrize or self.config.canonical_frame:
             board, pieces, planes = self._packed(obs)
             n = board.shape[0]
             step = n if chunk is None or n <= chunk else chunk
-            parts = [self._sym_trunk(board[s0:s0 + step], pieces[s0:s0 + step]) for s0 in range(0, n, step)]
+            trunk = self._sym_trunk if self.config.symmetrize else self._canon_trunk
+            parts = [trunk(board[s0:s0 + step], pieces[s0:s0 + step]) for s0 in range(0, n, step)]
         else:
             x, planes = self._obs_to_nchw(obs)
             n = x.shape[0]
@@ -162,14 +190,18 @@ class PPOAgent:
         return act, logp, value
 
     @torch.no_grad()
-    def act_into(self, obs, actions, log_probs, values, x_buf=None):
+    def act_into(self, obs, actions, log_probs, values, x_buf=None, canon=None):
         """``act`` on a packed observation with caller-owned outputs (rows of a RolloutBuffer):
         K2 -> CNN -> K3 writing ``actions`` int32[N] / ``log_probs`` f32[N] in place, ``values`` f32[N]
         copied.  No allocation of result tensors, no host work besides the launches — the body of a
-        captured rollout graph.  ``x_buf``: f32 [N,4,8,8], or [8N,4,8,8] with ``symmetrize``."""
+        captured rollout graph.  ``x_buf``: f32 [N,4,8,8], or [8N,4,8,8] with ``symmetrize``; ``canon``: the
+        canonical rows' scratch of ``_canon_trunk`` (``canonical_frame``)."""
         n = obs["board"].shape[0]
+        check_policy_form(self.config)
         if self.config.symmetrize:
             logits, value = self._sym_trunk(obs["board"], obs["pieces"], x_buf)
+        elif self.config.canonical_frame:
+            logits, value = self._canon_trunk(obs["board"], obs["pieces"], x_buf, canon)
         else:
             x = x_buf if x_buf is not None else torch.empty((n, 4, 8, 8), dtype=torch.float32, device=self.device)
             capi.unpack_obs(obs["board"], obs["pieces"], obs["mask"], obs["mask"].stride(0), obs=x, n=n)
@@ -206,15 +238,19 @@ class PPOAgent:
         return self.values(observations).cpu().numpy()
 
     # ------------------------------------------------------------------ update
-    def _fused_step(self, obs, mask, actions, old_logp, adv, ret, sums, pieces=None):
+    def _fused_step(self, obs, mask, actions, old_logp, adv, ret, sums, pieces=None, views=None):
         """One optimiser step on a gathered minibatch (fused loss tail); metric terms added to ``sums``.
-        ``pieces`` (symmetrize): the minibatch's pieces words, ``obs`` then holds its eight views."""
+        ``pieces`` (symmetrize): the minibatch's pieces words, ``obs`` then holds its eight views.
+        ``views`` (canonical_frame): the samples' view sets, ``obs`` holds their canonical views and the
+        logits are mapped back into the samples' frames (``pieces``: their own words)."""
         cfg = self.config
         if cfg.precision == "bf16":
             obs = obs.contiguous(memory_format=torch.channels_last)
         with self._autocast():
             logits, values = self.network.trunk(obs)
-        if pieces is not None:
+        if views is not None:
+            logits = CanonicalFrame.apply(logits, pieces, views)
+        elif pieces is not None:
             logits = SymmetryMean.apply(logits, pieces)
             values = values.float().view(8, -1).mean(0)
         loss, means = PPOLossTail.apply(logits, values.float(), mask, actions, old_logp, adv, ret,
@@ -228,22 +264,25 @@ class PPOAgent:
 
     def _minibatch(self, buffer, idx, mean_std, out, sums):
         """gather (bb_gather_minibatch) of samples ``idx``, then one optimiser step on them."""
-        g = buffer.gather(idx, mean_std, out=out, symmetrize=self.config.symmetrize)
-        self._fused_step(g["obs"], g["mask"], g["actions"], g["logp"], g["adv"], g["ret"], sums, g.get("pieces"))
+        cfg = self.config
+        g = buffer.gather(idx, mean_std, out=out, symmetrize=cfg.symmetrize, canonical=cfg.canonical_frame)
+        self._fused_step(g["obs"], g["mask"], g["actions"], g["logp"], g["adv"], g["ret"], sums, g.get("pieces"),
+                         g.get("views"))
 
     def _graph_step(self, buffer):
         """The minibatch step as a replayable CUDA graph: gather (bb_gather_minibatch) of the static
         index tensor, CNN forward / backward, loss tail, gradient all-reduce, clip, Adam — ~250
         launches collapse into one graph launch, which is what bounds the reference's own schedule
         (2,048-sample minibatches) on a B200.  Captured once per (buffer, batch size)."""
-        key = (id(buffer), self.config.batch_size, self.config.symmetrize)
+        key = (id(buffer), self.config.batch_size, self.config.symmetrize, self.config.canonical_frame)
         if self._graph is not None and self._graph["key"] == key:
             return self._graph
         dev, b = self.device, self.config.batch_size
         st = {"key": key, "idx": torch.zeros(b, dtype=torch.int64, device=dev),
               "ms": torch.zeros(2, dtype=torch.float32, device=dev),
               "sums": torch.zeros(6, dtype=torch.float64, device=dev)}
-        st["out"] = buffer.gather(st["idx"], st["ms"], symmetrize=self.config.symmetrize)
+        st["out"] = buffer.gather(st["idx"], st["ms"], symmetrize=self.config.symmetrize,
+                                  canonical=self.config.canonical_frame)
         graph = torch.cuda.CUDAGraph()
         with torch.cuda.graph(graph):
             self._minibatch(buffer, st["idx"], st["ms"], st["out"], st["sums"])
@@ -292,10 +331,10 @@ class PPOAgent:
         default of the reference's torch.load call).  The optimizer state is written in the form a
         plain torch.optim.Adam on any device accepts: CPU scalar ``step`` counters, no
         fused / foreach / capturable flags of ours.  ``b200_state`` (ignored by the reference)
-        carries the sampling-noise position for --resume and ``symmetrize`` (kept out of ``config``, which the
-        reference's PPOConfig(**config) must accept)."""
+        carries the sampling-noise position for --resume, ``symmetrize`` and ``canonical_frame`` (kept out of
+        ``config``, which the reference's PPOConfig(**config) must accept)."""
         cfgd = {k: (list(v) if isinstance(v, tuple) else v) for k, v in self.config.to_dict().items()
-                if k not in ("precision", "fused_bn", "symmetrize")}
+                if k not in ("precision", "fused_bn", "symmetrize", "canonical_frame")}
         opt = self.optimizer.state_dict()
         opt = {"state": {k: {n: (v.detach().cpu().float().reshape(()) if n == "step" and torch.is_tensor(v) else v)
                              for n, v in st.items()} for k, st in opt["state"].items()},
@@ -303,7 +342,8 @@ class PPOAgent:
         torch.save({"network_state_dict": network_state if network_state is not None else self.network.state_dict(),
                     "optimizer_state_dict": opt, "config": cfgd,
                     "b200_state": {"sample_calls": self.network.sample_calls, "sample_seed": self.network.sample_seed,
-                                   "symmetrize": bool(self.config.symmetrize)}},
+                                   "symmetrize": bool(self.config.symmetrize),
+                                   "canonical_frame": bool(self.config.canonical_frame)}},
                    path)
 
     def load(self, path):
@@ -322,6 +362,8 @@ class PPOAgent:
                                                "fused_bn": self.config.fused_bn})
         # the checkpoint's own policy form: symmetrized only when it was trained (or saved) so
         self.config.symmetrize = bool(ck.get("b200_state", {}).get("symmetrize", False))
+        self.config.canonical_frame = bool(ck.get("b200_state", {}).get("canonical_frame", False))
+        check_policy_form(self.config)
         if "b200_state" in ck:
             self.network.sample_calls = ck["b200_state"].get("sample_calls", 0)
         self.bucket.rebind()

@@ -129,12 +129,15 @@ class RolloutBuffer:
         return mean.float(), var.sqrt().float()
 
     # ------------------------------------------------------------------ minibatches
-    def gather(self, idx, mean_std, obs_dtype=torch.float32, out=None, symmetrize=False):
+    def gather(self, idx, mean_std, obs_dtype=torch.float32, out=None, symmetrize=False, canonical=False):
         """Minibatch ``idx`` (int64 flat sample indices) of the packed buffer in ONE library call
         (bb_gather_minibatch): obs planes (B,4,8,8), mask planes int64 [3,B], actions int32, old
         log-probs, advantages normalised with ``mean_std`` (float32 [2] device tensor), returns.
         ``symmetrize``: obs holds the eight views (8B,4,8,8) of the samples (bb_unpack_obs_sym through the
         same index) and ``pieces`` int32 [B] their pieces words.
+        ``canonical``: obs holds the canonical view (B,4,8,8) of each sample (bb_sym_canonical through the same
+        index, then K2), ``pieces`` int32 [B] the samples' own pieces words and ``views`` uint8 [B] their view
+        sets; ``canon_board`` / ``canon_pieces`` hold the canonical packed rows.
         ``out``: a dict of preallocated outputs to fill (static buffers of a captured CUDA graph)."""
         b, dev = idx.numel(), self.device
         if out is None:
@@ -144,14 +147,22 @@ class RolloutBuffer:
                        logp=torch.empty(b, dtype=torch.float32, device=dev),
                        adv=torch.empty(b, dtype=torch.float32, device=dev),
                        ret=torch.empty(b, dtype=torch.float32, device=dev))
-            if symmetrize:
+            if symmetrize or canonical:
                 out["pieces"] = torch.empty(b, dtype=torch.int32, device=dev)
+            if canonical:
+                out.update(views=torch.empty(b, dtype=torch.uint8, device=dev),
+                           canon_board=torch.empty(b, dtype=torch.int64, device=dev),
+                           canon_pieces=torch.empty(b, dtype=torch.int32, device=dev))
         capi.gather_minibatch(idx, self.num_envs, self.boards, self.pieces, self.action_masks, self.actions,
                               self.log_probs, self.advantages, self.returns, mean_std,
-                              None if symmetrize else out["obs"], out["mask"], out["actions"], out["logp"], out["adv"],
-                              out["ret"])
+                              None if symmetrize or canonical else out["obs"], out["mask"], out["actions"], out["logp"],
+                              out["adv"], out["ret"])
         if symmetrize:
             capi.unpack_obs_sym(self.boards, self.pieces, out["obs"], index=idx)
+        if canonical:
+            capi.sym_canonical(self.boards, self.pieces, out["canon_board"], out["canon_pieces"], out["views"], index=idx)
+            capi.unpack_obs(out["canon_board"], out["canon_pieces"], None, b, obs=out["obs"], n=b)
+        if symmetrize or canonical:
             torch.index_select(self.pieces.view(-1), 0, idx, out=out["pieces"])
         return out
 

@@ -8,7 +8,7 @@ and checkpoint files, run by one process per GPU.
 Config quirks of the reference are honoured (SURVEY.md §5): ``num_epochs`` is read from the
 ``ppo`` section (both shipped YAMLs put it under ``training``, so the default 10 applies),
 ``batch_size`` from ``training``, the ``network`` / ``environment`` sections are ignored.
-Keys of ours live under ``b200:`` (precision, reseed_on_reset, log_every_update, symmetrize).
+Keys of ours live under ``b200:`` (precision, reseed_on_reset, log_every_update, symmetrize, canonical_frame).
 """
 import argparse
 import json
@@ -51,6 +51,9 @@ class RolloutRunner:
         n, dev = buffer.num_envs, buffer.device
         rows = 8 * n if agent.config.symmetrize else n            # symmetrize: the eight views of every env
         self.x_buf = torch.empty((rows, 4, 8, 8), dtype=torch.float32, device=dev)
+        # canonical_frame: static canonical rows and view sets of the n envs, so that the rollout graph captures them
+        self.canon = ((torch.empty(n, dtype=torch.int64, device=dev), torch.empty(n, dtype=torch.int32, device=dev),
+                       torch.empty(n, dtype=torch.uint8, device=dev)) if agent.config.canonical_frame else None)
         self.last_values = torch.zeros(n, dtype=torch.float32, device=dev)
         self.use_graph, self.graph, self.calls = bool(use_graph), None, 0
 
@@ -58,7 +61,7 @@ class RolloutRunner:
         buf, T = self.buffer, self.buffer.buffer_size
         buf.set_first_obs(buf.obs_row(T))                      # continue from the last observation
         for t in range(T):
-            self.agent.act_into(buf.obs_row(t), buf.actions[t], buf.log_probs[t], buf.values[t], self.x_buf)
+            self.agent.act_into(buf.obs_row(t), buf.actions[t], buf.log_probs[t], buf.values[t], self.x_buf, self.canon)
             self.vec_env.step_into(buf.actions[t], buf.rewards[t], buf.terminated[t], buf.obs_row(t + 1))
         self.last_values.copy_(self.agent.values(buf.obs_row(T)))
         buf.finish_direct()
@@ -122,14 +125,17 @@ def train(config, resume_path=None, seed=42, progress_callback=None, max_updates
         entropy_coef=ppo_c.get("entropy_coef", 0.01), value_coef=ppo_c.get("value_coef", 0.5),
         max_grad_norm=ppo_c.get("max_grad_norm", 0.5), num_epochs=ppo_c.get("num_epochs", 10),
         batch_size=tr_c.get("batch_size", 2048), precision=ours.get("precision", "fp32"),
-        symmetrize=bool(ours.get("symmetrize", False))), device,
+        symmetrize=bool(ours.get("symmetrize", False)), canonical_frame=bool(ours.get("canonical_frame", False))), device,
         seed=seed, global_env_offset=offset)                  # sampling noise keyed by (seed, GLOBAL env id, call)
     agent.train()                                             # train mode during rollout too (scripts/train.py:122)
     start_step = 0
     if resume_path and os.path.exists(resume_path):
         agent.load(resume_path)
-        if "symmetrize" in ours:                              # the config's policy form wins over the checkpoint's
-            agent.config.symmetrize = bool(ours["symmetrize"])
+        for k in ("symmetrize", "canonical_frame"):           # the config's policy form wins over the checkpoint's
+            if k in ours:
+                setattr(agent.config, k, bool(ours[k]))
+        if agent.config.symmetrize and agent.config.canonical_frame:   # one from the checkpoint, one from the config
+            setattr(agent.config, "canonical_frame" if "symmetrize" in ours else "symmetrize", False)
         try:
             start_step = int(os.path.splitext(os.path.basename(resume_path))[0].split("_")[-1])
         except ValueError:

@@ -273,6 +273,29 @@ int bb_sym_logits_mean(const void* logits, int logits_dtype, const uint32_t* pie
 int bb_sym_logits_mean_backward(const float* grad_out, const uint32_t* pieces, void* grad_logits,
                                 int logits_dtype, int64_t n, void* stream);
 
+/* Canonical frame (group D4 as above): the network runs once per state, on the canonical view of its orbit,
+ * and its logits are mapped back into the state's own frame; policy and value are then exactly invariant /
+ * equivariant under the eight symmetries at the cost of one network row per state.
+ * bb_sym_canonical: for row r = index[i] (index device i64[n], or NULL for r = i) of board device u64[],
+ *   pieces device u32[]: board_out / pieces_out device u64[n] / u32[n] = the view g (bb_sym_board(g, b),
+ *   bb_sym_pieces(g, pw)) with the smallest key (board as u64, then the full pieces word as u32), and
+ *   views_out device u8[n] = the view set M: bit g set iff view g equals that view (never 0).
+ * bb_sym_logits_canonical: out device f32[n,192],
+ *   out[i, s*64 + a] = (1/|M_i|) * sum_{g in M_i, ascending} logits[i, s*64 + sigma_{g,p_s}(a)]
+ *   (f32) where a is an in-bounds anchor of the piece p_s < 37 of slot s of the state's own pieces[i]
+ *   (device u32[n]), 0 elsewhere.  logits device [n,192] of logits_dtype: the network's raw logits of
+ *   the canonical rows, 16-byte aligned (an unaligned pointer is rejected with code -1); views device
+ *   u8[n] from bb_sym_canonical.
+ * bb_sym_logits_canonical_backward: the transposed map, grad_logits device [n,192] of logits_dtype:
+ *   each canonical position sums (1/|M|) * grad_out over the (g, s*64 + a) that reach it, in ascending g
+ *   (several when |M| > 1), 0 where none does; grad_out device f32[n,192]; both 16-byte aligned. */
+int bb_sym_canonical(const uint64_t* board, const uint32_t* pieces, const int64_t* index, uint64_t* board_out,
+                     uint32_t* pieces_out, uint8_t* views_out, int64_t n, void* stream);
+int bb_sym_logits_canonical(const void* logits, int logits_dtype, const uint32_t* pieces, const uint8_t* views,
+                            float* out, int64_t n, void* stream);
+int bb_sym_logits_canonical_backward(const float* grad_out, const uint32_t* pieces, const uint8_t* views,
+                                     void* grad_logits, int logits_dtype, int64_t n, void* stream);
+
 /* Masked categorical head (BlockBlastNetwork.forward masking + get_action_and_value +
  * _masked_entropy, src/models/network.py:172-262) fused in one kernel.
  *   logits  device [n,192] of logits_dtype (BB_F32 / BB_BF16), raw (unmasked)

@@ -1,13 +1,16 @@
 #!/usr/bin/env python3
-"""Measure the board-symmetric policy (K7, PPOConfig.symmetrize) on one GPU, in one run with the card's name,
-power limit and maximum SM clock.
+"""Measure the board-symmetric policies on one GPU, in one run with the card's name, power limit and maximum SM
+clock: the eight-view average (K7, PPOConfig.symmetrize) and the canonical frame (K7c, PPOConfig.canonical_frame)
+against the plain policy.
 
 Kernels (CUDA events over many launches, outputs larger than L2 at the two large sizes; at 64 states the
 numbers are launch overhead): K7a (bb_unpack_obs_sym, n states -> 8n rows) against K2 (bb_unpack_obs) at the
 same 8n output rows, and K7b forward / backward (bb_sym_logits_mean[_backward]), f32 and bf16, at 64, 131,072
-and 262,144 states, each with its algorithmic HBM bytes and their fraction of the 7.7 TB/s data-sheet figure.
+and 262,144 states, each with its algorithmic HBM bytes and their fraction of the 7.7 TB/s data-sheet figure;
+K7c: bb_sym_canonical followed by K2 on the n canonical rows against K2 alone on n rows, and the logit map
+forward / backward (bb_sym_logits_canonical[_backward]), f32 and bf16, at the same sizes.
 
-Training shapes (bf16, CUDA graphs, with and without symmetrize): rollout time per env step (RolloutRunner:
+Training shapes (bf16, CUDA graphs; plain, symmetrize and canonical_frame, alternating): rollout time per env step (RolloutRunner:
 K7a / K2, CNN, K7b, K3, K1) and PPO update time per minibatch (gather, CNN forward and backward, loss tail, clip,
 Adam; GAE and the per-epoch permutation included), each with the peak allocated memory of that phase:
   ref: the reference's schedule, 64 envs x 128 steps, minibatch 2,048, 10 epochs
@@ -89,16 +92,50 @@ def kernels(emit):
             emit({"kernel": "K7b_backward", "dtype": name, "states": n, "us": us_b, "bytes": b_b,
                   "hbm_fraction": b_b / (us_b * 1e-6) / HBM_BYTES_PER_S})
             del logits, out, grad
+            # K7c: canonical views + K2 on n rows against K2 alone on n rows; the logit map on n rows
+            obs = torch.empty((n, 4, 8, 8), dtype=dt, device="cuda")
+            cb, cp = torch.empty_like(board), torch.empty_like(pieces)
+            views = torch.empty(n, dtype=torch.uint8, device="cuda")
+
+            def canon_k2():
+                capi.sym_canonical(board, pieces, cb, cp, views, n=n)
+                capi.unpack_obs(cb, cp, None, n, obs=obs, n=n)
+            us_k2n = event_time_us(lambda: capi.unpack_obs(board, pieces, None, n, obs=obs, n=n), reps)
+            us_c = event_time_us(lambda: capi.sym_canonical(board, pieces, cb, cp, views, n=n), reps)
+            us_ck2 = event_time_us(canon_k2, reps)
+            b_k2n = n * (12 + 256 * es)
+            b_c = n * (12 + 13)
+            b_ck2 = b_c + b_k2n
+            emit({"kernel": "K2_at_n_rows", "dtype": name, "states": n, "us": us_k2n, "bytes": b_k2n,
+                  "hbm_fraction": b_k2n / (us_k2n * 1e-6) / HBM_BYTES_PER_S})
+            emit({"kernel": "K7c_sym_canonical", "dtype": name, "states": n, "us": us_c, "bytes": b_c,
+                  "hbm_fraction": b_c / (us_c * 1e-6) / HBM_BYTES_PER_S})
+            emit({"kernel": "K7c_sym_canonical_plus_K2", "dtype": name, "states": n, "us": us_ck2, "bytes": b_ck2,
+                  "hbm_fraction": b_ck2 / (us_ck2 * 1e-6) / HBM_BYTES_PER_S})
+            del obs
+            logits = torch.randn((n, 192), device="cuda", generator=g).to(dt)
+            out = torch.empty((n, 192), dtype=torch.float32, device="cuda")
+            grad = torch.empty_like(logits)
+            us_f = event_time_us(lambda: capi.sym_logits_canonical(logits, pieces, views, out), reps)
+            us_b = event_time_us(lambda: capi.sym_logits_canonical_backward(out, pieces, views, grad), reps)
+            b_f = n * 192 * es + 5 * n + n * 768
+            b_b = n * 768 + 5 * n + n * 192 * es
+            emit({"kernel": "K7c_map_forward", "dtype": name, "states": n, "us": us_f, "bytes": b_f,
+                  "hbm_fraction": b_f / (us_f * 1e-6) / HBM_BYTES_PER_S})
+            emit({"kernel": "K7c_map_backward", "dtype": name, "states": n, "us": us_b, "bytes": b_b,
+                  "hbm_fraction": b_b / (us_b * 1e-6) / HBM_BYTES_PER_S})
+            del logits, out, grad
         torch.cuda.empty_cache()
 
 
-def train_shape(emit, label, n_envs, T, minibatch, epochs, sym, rollouts, updates):
+def train_shape(emit, label, n_envs, T, minibatch, epochs, policy, rollouts, updates):
     from bbgpu.ppo import PPOAgent, PPOConfig
     from bbgpu.rollout import RolloutBuffer
     from bbgpu.train import RolloutRunner
     from bbgpu.vec_env import VectorizedBlockBlastEnv
     dev = torch.device("cuda", 0)
-    agent = PPOAgent(PPOConfig(batch_size=minibatch, num_epochs=epochs, precision="bf16", symmetrize=sym), dev, seed=1)
+    agent = PPOAgent(PPOConfig(batch_size=minibatch, num_epochs=epochs, precision="bf16", symmetrize=policy == "symmetrize",
+                               canonical_frame=policy == "canonical_frame"), dev, seed=1)
     agent.train()
     venv = VectorizedBlockBlastEnv(n_envs, seed=1, output="packed")
     buf = RolloutBuffer(T, n_envs)
@@ -122,7 +159,7 @@ def train_shape(emit, label, n_envs, T, minibatch, epochs, sym, rollouts, update
     n_mb = updates * epochs * (T * n_envs // minibatch)
     t_mb = (time.perf_counter() - t0) / n_mb
     peak_upd = torch.cuda.max_memory_allocated()
-    emit({"shape": label, "symmetrize": sym, "envs": n_envs, "rollout_steps": T, "minibatch": minibatch, "epochs": epochs,
+    emit({"shape": label, "policy": policy, "envs": n_envs, "rollout_steps": T, "minibatch": minibatch, "epochs": epochs,
           "rollout_step_ms": t_roll * 1e3, "rollout_peak_gb": peak_roll / 1e9, "minibatch_step_ms": t_mb * 1e3,
           "update_peak_gb": peak_upd / 1e9, "rollouts_timed": rollouts, "minibatches_timed": n_mb})
     venv.close()
@@ -150,10 +187,12 @@ def main():
 
     kernels(emit)
     if not a.skip_train:
-        for sym in (False, True):
-            train_shape(emit, "ref", 64, 128, 2048, 10, sym, rollouts=5, updates=3)
-        for sym in (False, True):
-            train_shape(emit, "cfg4", 131072, 8, 32768, 1, sym, rollouts=2, updates=2)
+        policies = ("plain", "symmetrize", "canonical_frame")
+        for rep in range(2):                                 # alternating arms, twice: the spread is part of the result
+            for policy in policies:
+                train_shape(emit, "ref", 64, 128, 2048, 10, policy, rollouts=5, updates=3)
+            for policy in policies:
+                train_shape(emit, "cfg4", 131072, 8, 32768, 1, policy, rollouts=2, updates=2)
     if f:
         f.close()
 
