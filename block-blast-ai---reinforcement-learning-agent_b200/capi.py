@@ -65,6 +65,7 @@ def lib():
     L.bb_env_step_random.argtypes = [vp, i32, vp, vp, vp, vp, vp, vp, vp]
     L.bb_env_rollout_random.argtypes = [vp, i32, vp, vp, vp, vp, vp, vp]
     L.bb_env_observe.argtypes = [vp, vp, vp, vp, vp]
+    L.bb_env_observe_live.argtypes = [vp, vp, vp, vp, i64, vp, vp, vp]
     L.bb_env_sample_valid_actions.argtypes = [vp, u64, vp, vp, vp]
     L.bb_env_expand.argtypes = [vp, u64, i32, i64, vp, vp, vp, vp, vp, vp, vp, vp, vp]
     L.bb_env_get_state.argtypes = [vp, vp, vp]
@@ -198,6 +199,15 @@ class EnvHandle:
 
     def observe(self, board_out=None, pieces_out=None, mask_out=None):
         check(lib().bb_env_observe(self.h, ptr(board_out), ptr(pieces_out), ptr(mask_out), current_stream()))
+
+    def observe_live(self, board_out, pieces_out, mask_out, ids_out, count_out):
+        """Packed observation of the envs that are not game over, in rows 0..count-1 in ascending env order
+        (bb_env_observe_live): board int64 [n], pieces int32 [n], mask int64 [3, >= n] (its row stride is the
+        plane stride), ids int32 [n] (env index of each row), count int32 [1] — all CUDA tensors, written on the
+        device without a host synchronisation."""
+        check(lib().bb_env_observe_live(self.h, ptr(board_out), ptr(pieces_out), ptr(mask_out),
+                                        int(mask_out.stride(0)) if mask_out is not None else 0, ptr(ids_out),
+                                        ptr(count_out), current_stream()))
 
     def expand(self, call_counter, samples=1):
         """One-ply successors of every env's current state (bb_env_expand; no state changes).

@@ -196,6 +196,18 @@ int bb_env_observe(bb_env* e, uint64_t* board_out, uint32_t* pieces_out, uint64_
     return 0;
 }
 
+int bb_env_observe_live(bb_env* e, uint64_t* board_out, uint32_t* pieces_out, uint64_t* mask_out, int64_t mask_stride,
+                        int32_t* ids_out, int32_t* count_out, void* stream) {
+    if (!e) return fail(-1, "bb_env_observe_live: env is NULL");
+    if (!board_out || !pieces_out || !mask_out || !ids_out || !count_out)
+        return fail(-1, "bb_env_observe_live: NULL output (board/pieces/mask/ids/count are all required)");
+    if (mask_stride < e->arr.n) return fail(-1, "bb_env_observe_live: mask_stride must be >= n_envs");
+    BB_DEVICE(e, "bb_env_observe_live");
+    BB_CUDA(bb_launch_observe_live(e->arr, e->d_expand_scratch, board_out, pieces_out, mask_out, mask_stride, ids_out,
+                                   count_out, (cudaStream_t)stream), "bb_env_observe_live launch");
+    return 0;
+}
+
 int bb_env_sample_valid_actions(bb_env* e, uint64_t call_counter, int32_t* actions_out, int32_t* h_actions_out, void* stream) {
     if (!e) return fail(-1, "bb_env_sample_valid_actions: env is NULL");
     if (!actions_out && !h_actions_out) return fail(-1, "bb_env_sample_valid_actions: no output given");

@@ -554,11 +554,69 @@ bb_expand_kernel(BBEnvArrays E, BBRewardCfg cfg, uint32_t call_counter, int samp
 }
 
 // ---------------------------------------------------------------------------------------
+// bb_env_observe_live: the observation of every env that is not game over, compacted into rows
+// 0..count-1 in ascending env order.  Count per block -> bb_expand_scan_blocks_kernel (exclusive
+// block offsets, grand total) -> write; no atomics, so the row order is fixed.
+// ---------------------------------------------------------------------------------------
+__global__ void __launch_bounds__(BB_STEP_THREADS)
+bb_live_count_kernel(BBEnvArrays E, int64_t* __restrict__ block_sums) {
+    const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    const bool live = i < E.n && !((E.s0[i].w >> 16) & 1u);       // aux byte 2: game over (BB_OVER)
+    const int c = __syncthreads_count(live);
+    if (threadIdx.x == 0) block_sums[blockIdx.x] = c;
+}
+
+// row of env i = its block's offset + live envs before it in the block (warp ballots)
+__global__ void __launch_bounds__(BB_STEP_THREADS)
+bb_observe_live_kernel(BBEnvArrays E, const int64_t* __restrict__ block_offsets, const int64_t* __restrict__ total,
+                       uint64_t* __restrict__ board_out, uint32_t* __restrict__ pieces_out, uint64_t* __restrict__ mask_out,
+                       int64_t mask_stride, int32_t* __restrict__ ids_out, int32_t* __restrict__ count_out) {
+    __shared__ int warp_live[BB_STEP_THREADS / 32];
+    const BBTables& T = g_bb_tables;
+    const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
+    BBState s;
+    bool live = false;
+    if (i < E.n) {
+        bb_load_state(E, i, s);
+        live = !BB_OVER(s);
+    }
+    const unsigned ballot = __ballot_sync(0xffffffffu, live);
+    if (lane == 0) warp_live[w] = __popc(ballot);
+    __syncthreads();
+    int before = __popc(ballot & ((1u << lane) - 1u));
+    for (int k = 0; k < w; ++k) before += warp_live[k];
+    if (i == 0) *count_out = (int32_t)*total;
+    if (!live) return;
+    const int64_t row = block_offsets[blockIdx.x] + before;
+    board_out[row] = s.board;
+    pieces_out[row] = s.pieces;
+    uint64_t m[3];
+    bb_action_mask(s, &T, m);
+    mask_out[row] = m[0];
+    mask_out[mask_stride + row] = m[1];
+    mask_out[2 * mask_stride + row] = m[2];
+    ids_out[row] = (int32_t)i;
+}
+
+// ---------------------------------------------------------------------------------------
 // launchers
 // ---------------------------------------------------------------------------------------
 static inline unsigned bb_grid(int64_t n) { return (unsigned)((n + BB_STEP_THREADS - 1) / BB_STEP_THREADS); }
 
-int64_t bb_expand_scratch_count(int64_t n) { return (int64_t)bb_grid(n); }
+// one int64 per block of the offset scan, plus the grand total of bb_launch_observe_live's scan
+int64_t bb_expand_scratch_count(int64_t n) { return (int64_t)bb_grid(n) + 1; }
+
+cudaError_t bb_launch_observe_live(const BBEnvArrays& E, int64_t* scratch, uint64_t* board_out, uint32_t* pieces_out,
+                                   uint64_t* mask_out, int64_t mask_stride, int32_t* ids_out, int32_t* count_out,
+                                   cudaStream_t stream) {
+    const unsigned nb = bb_grid(E.n);
+    bb_live_count_kernel<<<nb, BB_STEP_THREADS, 0, stream>>>(E, scratch);
+    bb_expand_scan_blocks_kernel<<<1, BB_STEP_THREADS, 0, stream>>>(scratch, (int64_t)nb, scratch + nb);
+    bb_observe_live_kernel<<<nb, BB_STEP_THREADS, 0, stream>>>(E, scratch, scratch + nb, board_out, pieces_out, mask_out,
+                                                               mask_stride, ids_out, count_out);
+    return cudaGetLastError();
+}
 
 cudaError_t bb_launch_expand(const BBEnvArrays& E, const BBRewardCfg& cfg, uint32_t call_counter, int samples,
                              int64_t capacity, int64_t* offsets, int64_t* scratch, int32_t* action_out, float* reward_out,

@@ -44,8 +44,12 @@ cudaError_t bb_launch_step_random(const BBEnvArrays& E, const BBRewardCfg& cfg, 
 cudaError_t bb_launch_zero_draw_ctr(const BBEnvArrays& E, cudaStream_t stream);
 cudaError_t bb_launch_reset(const BBEnvArrays& E, const uint8_t* reset_mask, uint64_t* mask_out, cudaStream_t stream);
 cudaError_t bb_launch_sample_valid(const BBEnvArrays& E, uint64_t call_counter, int32_t* actions_out, cudaStream_t stream);
-// bb_env_expand (phase 1 + phase 2); scratch: bb_expand_scratch_count(n) int64 block totals
+// bb_env_expand (phase 1 + phase 2); scratch: bb_expand_scratch_count(n) int64 block totals (+ one grand total)
 int64_t bb_expand_scratch_count(int64_t n);
+// bb_env_observe_live; scratch: the same bb_expand_scratch_count(n) int64
+cudaError_t bb_launch_observe_live(const BBEnvArrays& E, int64_t* scratch, uint64_t* board_out, uint32_t* pieces_out,
+                                   uint64_t* mask_out, int64_t mask_stride, int32_t* ids_out, int32_t* count_out,
+                                   cudaStream_t stream);
 cudaError_t bb_launch_expand(const BBEnvArrays& E, const BBRewardCfg& cfg, uint32_t call_counter, int samples,
                              int64_t capacity, int64_t* offsets, int64_t* scratch, int32_t* action_out, float* reward_out,
                              uint8_t* terminated_out, uint32_t* info_out, uint64_t* board_out, uint32_t* pieces_out,

@@ -3,7 +3,8 @@
 
 Each of ``num_episodes`` envs plays exactly one episode (``BB_ENV_NO_AUTO_RESET``: a finished env
 stays GAME_OVER and its further steps are no-ops), so the returned statistics are per-episode
-like the reference's: scores, lengths, lines cleared, max combo.
+like the reference's: scores, lengths, lines cleared, max combo.  The argmax policy runs the network only
+on the episodes that are still going (``bb_env_observe_live`` compacts their observations each step).
 
     python -m bbgpu.evaluate --checkpoint checkpoints/best.pt --episodes 1000
 
@@ -49,9 +50,17 @@ def lookahead_actions(agent, h, n, call_counter, samples, chunk=65536):
     return q.argmax(dim=1).to(torch.int32), ex, q
 
 
+def live_rows(m, n):
+    """Network rows for ``m`` live envs of ``n``: ``m`` rounded up to one of four sizes per octave (at most n).
+    It bounds the number of distinct batch shapes cuDNN plans for (and, with ``cudnn.benchmark``, times) to
+    about four per octave, at most a quarter more rows than ``m``."""
+    q = 1 << max(m.bit_length() - 3, 0)
+    return min(n, -(-m // q) * q)
+
+
 @torch.no_grad()
 def evaluate(agent, num_episodes=100, seed=0, deterministic=True, max_steps=10000, reward_config=None,
-             return_actions=False, lookahead=0, symmetrize=None, canonical_frame=None):
+             return_actions=False, lookahead=0, symmetrize=None, canonical_frame=None, global_env_offset=0):
     """``lookahead``: 0 = the agent's own policy (argmax when ``deterministic``); K >= 1 = one-ply value
     look-ahead with K sampled trios per dealing move (``lookahead_actions``, expansion call counter = the
     step number).  ``return_actions``: also return ``actions`` int32 [steps, n] (the action every env was given at every
@@ -60,12 +69,16 @@ def evaluate(agent, num_episodes=100, seed=0, deterministic=True, max_steps=1000
     ``symmetrize``: None = the agent's own setting; True / False = with / without the eight-view average for
     this evaluation (the successor values of ``lookahead`` included).  ``canonical_frame``: the same for the
     canonical-frame policy.  Turning one of the two on turns the other off for this evaluation; the agent's
-    own settings are restored afterwards."""
+    own settings are restored afterwards.  ``global_env_offset``: global id of episode 0, so that each rank's shard
+    plays the games that episodes ``global_env_offset ...`` of one single-process evaluation would play.
+
+    The deterministic policy (``lookahead`` 0) runs the network on the unfinished episodes only
+    (``bb_env_observe_live``); the other paths run it on every episode at every step."""
     if symmetrize and canonical_frame:
         raise ValueError("evaluate: symmetrize and canonical_frame are mutually exclusive")
     dev = agent.device
     n = int(num_episodes)
-    h = capi.EnvHandle(n, seed, 0, reward_config, capi.ENV_NO_AUTO_RESET)
+    h = capi.EnvHandle(n, seed, global_env_offset, reward_config, capi.ENV_NO_AUTO_RESET)
     board = torch.zeros(n, dtype=torch.int64, device=dev)
     pieces = torch.zeros(n, dtype=torch.int32, device=dev)
     mask = torch.zeros((3, n), dtype=torch.int64, device=dev)
@@ -85,13 +98,34 @@ def evaluate(agent, num_episodes=100, seed=0, deterministic=True, max_steps=1000
     agent.eval()                                       # scripts/evaluate.py evaluates in eval mode
     steps = 0
     log = []
+    # K3 keys its sampling noise by row index: compacting the rows would change which draws a seeded
+    # stochastic evaluation makes, so only the deterministic policy runs on the live rows
+    compact = deterministic and not lookahead
+    if compact:
+        ids = torch.zeros(n, dtype=torch.int32, device=dev)
+        count = torch.zeros(1, dtype=torch.int32, device=dev)
+        act = torch.zeros(n, dtype=torch.int32, device=dev)
     try:
-        while steps < max_steps and not bool(done.all()):
-            if lookahead:
-                act, _, _ = lookahead_actions(agent, h, n, steps, int(lookahead))
+        while steps < max_steps:
+            if compact:
+                # the live rows, then one 4-byte read: the host synchronisation of the step
+                h.observe_live(board, pieces, mask, ids, count)
+                m = int(count.item())
+                if m == 0:
+                    break
+                rows = live_rows(m, n)          # rows m..rows-1 hold observations of earlier steps; dropped below
+                a, _, _ = agent.act({"board": board[:rows], "pieces": pieces[:rows], "mask": mask[:, :rows]},
+                                    deterministic=True)
+                # a finished env keeps its last action, which BB_ENV_NO_AUTO_RESET ignores
+                act.index_copy_(0, ids[:m].long(), a[:m])
             else:
-                h.observe(board, pieces, mask)
-                act, _, _ = agent.act({"board": board, "pieces": pieces, "mask": mask}, deterministic=deterministic)
+                if bool(done.all()):
+                    break
+                if lookahead:
+                    act, _, _ = lookahead_actions(agent, h, n, steps, int(lookahead))
+                else:
+                    h.observe(board, pieces, mask)
+                    act, _, _ = agent.act({"board": board, "pieces": pieces, "mask": mask}, deterministic=deterministic)
             if return_actions:
                 log.append(act.clone())
             h.step(act, rewards, term, None, None, None, None)

@@ -2,7 +2,8 @@
 summary), ``TensorBoardLogger`` and ``MetricsTracker`` interfaces (src/utils/logger.py:28-302),
 so dashboards and scripts that read the reference's logs read ours: one JSON object per line with
 ``step``/``time``/``timestamp`` plus the metrics, ``<name>_summary.json`` with mean/std/min/max/last
-per metric, and the TensorBoard tags of scripts/train.py:247-258 (``performance/*``, ``training/*``).
+per metric, and the TensorBoard tags of scripts/train.py:247-258 (``performance/*``, ``training/*``), plus
+``evaluation/*`` for the held-out evaluations of ``b200.eval_interval``.
 
 The values are produced by on-device episode reductions (train.py), not by a per-episode Python
 loop; only the writer side lives here.
@@ -188,7 +189,11 @@ class MetricsTracker:
         self.metrics.clear()
 
 
-# TensorBoard tags of scripts/train.py:247-258, from one JSONL row of train.py
+EVAL_KEYS = ("eval_mean_score", "eval_std_score", "eval_max_score", "eval_min_score", "eval_mean_length",
+             "eval_finished", "eval_wall_s")
+
+
+# TensorBoard tags of scripts/train.py:247-258, from one JSONL row of train.py; evaluation/* for held-out evaluations
 def tensorboard_tags(row):
     tags = {"performance/avg_score": row["avg_score"], "performance/max_score": row["max_score"],
             "performance/best_score": row["best_score"], "performance/avg_length": row["avg_length"],
@@ -196,4 +201,7 @@ def tensorboard_tags(row):
     for k in ("policy_loss", "value_loss", "entropy", "approx_kl", "clip_fraction"):
         if k in row and not (isinstance(row[k], float) and math.isnan(row[k])):
             tags["training/" + k] = row[k]
+    for k in EVAL_KEYS:                       # rows of updates with a held-out evaluation (train.py)
+        if k in row:
+            tags["evaluation/" + k[len("eval_"):]] = row[k]
     return tags

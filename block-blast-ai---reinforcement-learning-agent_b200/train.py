@@ -8,7 +8,19 @@ and checkpoint files, run by one process per GPU.
 Config quirks of the reference are honoured (SURVEY.md §5): ``num_epochs`` is read from the
 ``ppo`` section (both shipped YAMLs put it under ``training``, so the default 10 applies),
 ``batch_size`` from ``training``, the ``network`` / ``environment`` sections are ignored.
-Keys of ours live under ``b200:`` (precision, reseed_on_reset, log_every_update, symmetrize, canonical_frame).
+Keys of ours live under ``b200:`` (precision, reseed_on_reset, log_every_update, symmetrize, canonical_frame,
+and the held-out evaluation below).
+
+Held-out evaluation (``b200:``; the reference's own ``eval_interval`` / ``eval_episodes`` stay ignored, SURVEY §5):
+  eval_interval   evaluate every this many updates and once more when training stops; 0 or absent = off
+  eval_episodes   episodes per evaluation for the whole job (default 1,000), divisible by the number of GPUs
+  eval_seed       Philox seed of the evaluation games (default seed + 1: disjoint from the training streams);
+                  every evaluation plays the same games, so two checkpoints' evaluations are paired
+  eval_lookahead  ``evaluate``'s ``lookahead`` (default 0: the argmax policy)
+  eval_max_steps  default 10,000
+Each rank plays its shard of the games with rank 0's network, the results are reduced, and rows of evaluation
+updates gain ``eval_*`` keys (TensorBoard ``evaluation/*``); rank 0 writes ``best_eval.pt`` at each new best
+``eval_mean_score``.  An evaluation changes nothing of the training run.
 """
 import argparse
 import json
@@ -19,6 +31,7 @@ import numpy as np
 import torch
 
 from . import dist
+from .evaluate import evaluate
 from .logger import Logger, TensorBoardLogger, tensorboard_tags
 from .ppo import PPOAgent, PPOConfig
 from .rollout import RolloutBuffer
@@ -35,6 +48,72 @@ def set_seed(seed):
     np.random.seed(seed)
     torch.manual_seed(seed)
     torch.cuda.manual_seed_all(seed)
+
+
+def eval_settings(ours, world, seed):
+    """The held-out evaluation of a config's ``b200`` section: None when ``eval_interval`` is 0 or absent,
+    else {interval, episodes, seed, lookahead, max_steps}.  Raises ValueError for settings a job of ``world``
+    GPUs cannot run."""
+    interval = int(ours.get("eval_interval", 0) or 0)
+    if interval < 0:
+        raise ValueError("b200.eval_interval (%d) must be >= 0" % interval)
+    if not interval:
+        return None
+    episodes = int(ours.get("eval_episodes", 1000))
+    if episodes <= 0 or episodes % world:
+        # every rank plays an equal shard, so that the ranks reach the reduction together
+        raise ValueError("b200.eval_episodes (%d) must be positive and divisible by the number of GPUs (%d)"
+                         % (episodes, world))
+    return {"interval": interval, "episodes": episodes, "seed": int(ours.get("eval_seed", seed + 1)),
+            "lookahead": int(ours.get("eval_lookahead", 0)), "max_steps": int(ours.get("eval_max_steps", 10000))}
+
+
+def eval_sums(res):
+    """The parts of one shard's ``evaluate`` result that the ranks reduce: ([episodes, sum of scores, sum of
+    squared scores, sum of lengths, finished], [max score, -min score]) — the first list is summed, the second
+    maximised."""
+    s = res["scores"].astype(np.float64)
+    return ([float(s.size), float(s.sum()), float((s * s).sum()), float(res["lengths"].sum()), float(res["finished"])],
+            [float(s.max()), -float(s.min())])
+
+
+def eval_stats(sums, maxes, wall_s):
+    """The ``eval_*`` row keys from reduced ``eval_sums`` and the evaluation's wall time."""
+    cnt, ssum, ssq, lsum, fin = sums
+    mean = ssum / cnt
+    return {"eval_mean_score": mean, "eval_std_score": float(np.sqrt(max(ssq / cnt - mean * mean, 0.0))),
+            "eval_max_score": int(maxes[0]), "eval_min_score": int(-maxes[1]), "eval_mean_length": lsum / cnt,
+            "eval_finished": int(fin), "eval_wall_s": wall_s}
+
+
+@torch.no_grad()
+def evaluate_held_out(agent, ev, reward_config, device):
+    """One held-out evaluation inside training (``eval_settings`` ``ev``): this rank plays its shard of the games
+    with the argmax policy (or ``lookahead``) and the shards' results are reduced.  Returns the ``eval_*`` keys.
+    Nothing of the training run changes: ``evaluate`` restores the agent's mode and policy form, the deterministic
+    policy draws no sampling noise, and the rank's own BatchNorm statistics are put back."""
+    offset, n_local = dist.shard(ev["episodes"])
+    calls = agent.network.sample_calls
+    own = None
+    if dist.world_size() > 1:
+        # BatchNorm running statistics are per GPU: every rank evaluates rank 0's network, the one checkpoints hold
+        own = [b.detach().clone() for b in agent.network.buffers()]
+        for b in agent.network.buffers():
+            torch.distributed.broadcast(b.data, 0)
+    t0 = time.time()
+    try:
+        res = evaluate(agent, n_local, seed=ev["seed"], deterministic=True, max_steps=ev["max_steps"],
+                       reward_config=reward_config, lookahead=ev["lookahead"], global_env_offset=offset)
+    finally:
+        if own is not None:
+            for b, v in zip(agent.network.buffers(), own):
+                b.data.copy_(v)
+    wall = time.time() - t0
+    assert agent.network.sample_calls == calls, "a deterministic evaluation must not advance the sampling counter"
+    sums, maxes = eval_sums(res)
+    sums = dist.all_reduce_scalars(sums, device=device)
+    *maxes, wall = dist.all_reduce_scalars(maxes + [wall], op="max", device=device)
+    return eval_stats(sums, maxes, wall)
 
 
 class RolloutRunner:
@@ -109,6 +188,7 @@ def train(config, resume_path=None, seed=42, progress_callback=None, max_updates
         # unequal shards would give the ranks different minibatch counts, i.e. different numbers of
         # gradient all-reduces per epoch (a hang), and unequal weights in the gradient mean
         raise ValueError("training.num_envs (%d) must be divisible by the number of GPUs (%d)" % (num_envs, world))
+    ev = eval_settings(ours, world, seed)
     offset, n_local = dist.shard(num_envs)
     # b200.stream_period = P: env g draws its pieces from stream g mod P, i.e. the job plays num_envs / P copies of
     # the same P piece streams (with reseed_on_reset: the reference's 64 fixed games, several trajectories of each
@@ -154,6 +234,7 @@ def train(config, resume_path=None, seed=42, progress_callback=None, max_updates
     best_every_s = float(ours.get("best_save_min_interval_s", 10.0))
     global_step, num_updates, best_score, recent = start_step, 0, 0.0, []
     best_state, best_saved_at = None, 0.0
+    best_eval = float("-inf")
     history = []
     # same files / keys / TensorBoard tags as scripts/train.py:136-137, 231-258 (rank 0 only)
     logger = Logger(log_dir, name="ppo_b200") if rank == 0 else None
@@ -180,6 +261,9 @@ def train(config, resume_path=None, seed=42, progress_callback=None, max_updates
             history.append(row)
             stop = bool((max_updates and num_updates >= max_updates) or (max_wall_s and elapsed >= max_wall_s) or
                         (target_score and len(recent) == 10 and avg10 >= target_score) or global_step >= total_timesteps)
+            if ev and (num_updates % ev["interval"] == 0 or stop):
+                row.update(evaluate_held_out(agent, ev, rew_c or None, device))
+            evaluated = "eval_mean_score" in row
             if rank == 0:
                 if avg_score > best_score:
                     # snapshot the weights on the device now (cheap), write best.pt at most every few seconds:
@@ -189,13 +273,22 @@ def train(config, resume_path=None, seed=42, progress_callback=None, max_updates
                 if best_state is not None and time.time() - best_saved_at > best_every_s:
                     agent.save(os.path.join(ckpt_dir, "best.pt"), network_state=best_state)
                     best_state, best_saved_at = None, time.time()
-                if num_updates % log_interval == 0 or num_updates <= 10 or ours.get("log_every_update") or stop:
+                if evaluated and row["eval_mean_score"] > best_eval:
+                    best_eval = row["eval_mean_score"]
+                    agent.save(os.path.join(ckpt_dir, "best_eval.pt"))
+                if (num_updates % log_interval == 0 or num_updates <= 10 or ours.get("log_every_update") or stop
+                        or evaluated):
                     logger.log(row, global_step)
                     if tb_logger is not None:
                         tb_logger.log_metrics(tensorboard_tags(row), global_step)
                     print("update %d step=%d fps=%.0f avg_score=%.1f max=%d len=%.1f entropy=%.3f kl=%.4f clip=%.3f"
                           % (num_updates, global_step, row["fps"], avg_score, smax, row["avg_length"], metrics["entropy"],
                              metrics["approx_kl"], metrics["clip_fraction"]), flush=True)
+                    if evaluated:
+                        print("  eval: %d episodes mean=%.1f std=%.1f max=%d min=%d len=%.1f finished=%d (%.2f s)"
+                              % (ev["episodes"], row["eval_mean_score"], row["eval_std_score"], row["eval_max_score"],
+                                 row["eval_min_score"], row["eval_mean_length"], row["eval_finished"], row["eval_wall_s"]),
+                              flush=True)
                 if num_updates % save_interval == 0:
                     agent.save(os.path.join(ckpt_dir, "checkpoint_%d.pt" % global_step))
                     agent.save(os.path.join(ckpt_dir, "latest.pt"))

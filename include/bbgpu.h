@@ -180,6 +180,19 @@ int bb_env_expand(bb_env* env, uint64_t call_counter, int32_t samples, int64_t c
 int bb_env_observe(bb_env* env, uint64_t* board_out, uint32_t* pieces_out, uint64_t* mask_out,
                    void* stream);
 
+/* Packed observation of the envs that are NOT game over, compacted: row r = the r-th such env in
+ * ascending env order, with exactly the bytes bb_env_observe writes for that env.  count_out[0] =
+ * number of rows, written on the device (no host synchronisation); the rows are ordered without
+ * atomics (per-block counts, a scan, the write), so a repeated call writes the same bytes.  Uses the
+ * handle's create-time scratch, so two calls on one handle must not run concurrently.  No env state
+ * changes.  Rows >= count_out[0] are left untouched.
+ *   board_out  device u64[n]   pieces_out device u32[n]   ids_out device i32[n] (env index 0..n-1)
+ *   mask_out   device u64[3*mask_stride], plane-major with plane stride mask_stride >= n
+ *   count_out  device i32[1]
+ * Every output is required. */
+int bb_env_observe_live(bb_env* env, uint64_t* board_out, uint32_t* pieces_out, uint64_t* mask_out,
+                        int64_t mask_stride, int32_t* ids_out, int32_t* count_out, void* stream);
+
 /* Full state export / import for checkpoints and parity tests (GameEngine.get_state /
  * set_state, engine.py:456-476, plus counters).  HOST arrays of n_envs records, 48 bytes each:
  * {u64 board; u32 pieces; u32 aux(prev_holes | prev_center_filled<<8 | game_over<<16);
